@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the motion-compensation hot path (BASELINE.json).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--frames F]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--frames F] [--dump-outputs DIR]
 
 One "step" = one pass of the soft-mode (softmax) forward splat over one batch of F synthetic
 1080p fp32 frames (BASELINE.json north_star: "fp32 softmax-splat forward on 1080p frames"; the
@@ -490,6 +490,21 @@ def _uvg_sweep(torch, d, dev, rank, world, peak, gops_per_chunk=16):
             "deterministic_hash_first_8_gops": det_hash, "output_gather": out_gather}
 
 
+DUMP_SAMPLE = 1 << 22          # elements of the output drawn at fixed positions: 16 MiB in fp32
+
+
+def _dump_outputs(torch, out, directory):
+    """What the last timed step returned, for comparing two builds output for output (the inputs are seeded, so the
+    same arguments give the same inputs): frame 0 in full, and the values at DUMP_SAMPLE fixed positions drawn over
+    the whole output with a fixed seed, so that every frame of the step is checked. About 42 MB at the bench's sizes."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    flat = out.reshape(-1)
+    idx = np.sort(np.random.default_rng(0).integers(0, flat.numel(), size=min(DUMP_SAMPLE, flat.numel())))
+    np.save(os.path.join(directory, "softsplat_out_frame0.npy"), out[0].float().cpu().numpy())
+    np.save(os.path.join(directory, "softsplat_out_sample.npy"), flat[torch.from_numpy(idx).to(out.device)].float().cpu().numpy())
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -545,6 +560,8 @@ def run_ours(args):
     launches = d.launch_count() - launches0
     ms_step = max_over_ranks(a.elapsed_time(b)) / args.steps
     value = world * px_per_step / ms_step / 1e3                            # Mpixel/s, whole job
+    if args.dump_outputs and rank == 0:
+        _dump_outputs(torch, out, args.dump_outputs)
     out0 = out[:1].clone()                                                 # for the output check below
 
     # ---- forward + backward (the other half of BASELINE's metric): all three gradients, 16 frames per GPU per step ----
@@ -675,7 +692,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-extra", action="store_true")
     ap.add_argument("--no-c5", action="store_true", help="skip the UVG-shaped sweep (C5)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write a fixed sample of the last step's output (rank 0) as DIR/*.npy, float32")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:
