@@ -15,7 +15,7 @@ from .control_utils import compute_mask, FeatureWarperSoftsplat, resize_and_norm
 from .warp import WarpingLayerBWFlow, backwarp, backwarp_residual
 from .extractors import (bidir_fuse, bidirectional_warp_fuse, bidirectional_block, bidirectional_pyramid, pyramid_conditioning, resample_batch,
                          Bi_Dir_FeatureExtractor, Bi_Dir_ResidueExtractor, WarpExtractor, ConvBlock)
-from .residual_utils import residual_conditioning, ResidueDataset, WarpingDatasetWrapper
+from .residual_utils import residual_conditioning, residual_conditioning_bidir, ResidueDataset, WarpingDatasetWrapper
 from .sharding import UVG_SEQUENCES, GopUnit, enumerate_gops, shard_units, gather_checksums, gather_outputs, checksum
 from .host import softsplat_host, bind_to_gpu_numa
 from .patch_utils import merge_latent_tiles_from_pixel_coords, crop_into_tiles

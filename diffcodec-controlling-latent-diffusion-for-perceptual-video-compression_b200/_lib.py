@@ -86,6 +86,7 @@ SYMBOLS = {
     "dcb_resample_batch": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int32, ctypes.c_void_p]),
     "dcb_convert": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int32, ctypes.c_void_p, ctypes.c_int32, ctypes.c_int64, ctypes.c_float, ctypes.c_void_p]),
     "dcb_residual_fused": (ctypes.c_int, [_P] * 8 + [ctypes.c_void_p, ctypes.c_int64, ctypes.c_int32, ctypes.c_int32, ctypes.c_void_p]),
+    "dcb_residual_bidir": (ctypes.c_int, [_P] * 9 + [ctypes.c_void_p, ctypes.c_int64, ctypes.c_int32, ctypes.c_void_p]),
 }
 
 

@@ -50,6 +50,8 @@ long long recipe_workspace(long long N, long long C, long long H, long long W);
 int occlusion_mask_impl(const DcbTensor*, const DcbTensor*, const DcbTensor*, void*, long long, int, cudaStream_t);
 int residual_fused_impl(const DcbTensor*, const DcbTensor*, const DcbTensor*, const DcbTensor*, const DcbTensor*,
                         const DcbTensor*, const DcbTensor*, const DcbTensor*, void*, long long, int, int, cudaStream_t);
+int residual_bidir_impl(const DcbTensor*, const DcbTensor*, const DcbTensor*, const DcbTensor*, const DcbTensor*, const DcbTensor*,
+                        const DcbTensor*, const DcbTensor*, const DcbTensor*, void*, long long, int, cudaStream_t);
 int bidir_fuse_fwd_impl(const DcbTensor*, const DcbTensor*, const DcbTensor*, const DcbTensor*, const DcbTensor*,
                         const DcbTensor*, const DcbTensor*, cudaStream_t);
 int bidir_fuse_bwd_impl(const DcbTensor*, const DcbTensor*, const DcbTensor*, const DcbTensor*, const DcbTensor*,
@@ -382,6 +384,42 @@ int dcb_residual_fused(const DcbTensor* image1, const DcbTensor* flow1, const Dc
     TRY(check_out(fn, "occ_fwd", occ_fwd, dt, elem_size(dt)));
     TRY(check_out(fn, "occ_bwd", occ_bwd, dt, elem_size(dt)));
     return residual_fused_impl(image1, flow1, flow2, gt, fused, residual, occ_fwd, occ_bwd, ws, ws_bytes, variant, flags,
+                               (cudaStream_t)stream);
+}
+
+int dcb_residual_bidir(const DcbTensor* image1, const DcbTensor* image2, const DcbTensor* flow1, const DcbTensor* flow2,
+                       const DcbTensor* gt, const DcbTensor* fused, const DcbTensor* residual, const DcbTensor* occ_fwd,
+                       const DcbTensor* occ_bwd, void* ws, int64_t ws_bytes, int32_t flags, void* stream) {
+    const char* fn = "dcb_residual_bidir";
+    TRY(check_tensor(fn, "image1", image1, true));
+    TRY(check_tensor(fn, "image2", image2, true));
+    TRY(check_tensor(fn, "flow1", flow1, true));
+    TRY(check_tensor(fn, "flow2", flow2, true));
+    TRY(check_tensor(fn, "gt", gt, true));
+    TRY(check_tensor(fn, "fused", fused, true));
+    TRY(check_tensor(fn, "residual", residual, true));
+    TRY(check_tensor(fn, "occ_fwd", occ_fwd, false));
+    TRY(check_tensor(fn, "occ_bwd", occ_bwd, false));
+    if (flags & ~DCB_FLAG_WS_CLEAN) return set_error(DCB_E_MODE, "%s: unknown flags 0x%x", fn, flags);
+    const long long N = image1->size[0], C = image1->size[1], H = image1->size[2], W = image1->size[3];
+    TRY(check_limits(fn, image1));
+    if (C < 1 || C > 3) return set_error(DCB_E_LIMIT, "%s: fused recipe handles 1..3 image channels, got %lld", fn, C);
+    TRY(check_shape(fn, "image2", image2, N, C, H, W));
+    TRY(check_shape(fn, "flow1", flow1, N, 2, H, W));
+    TRY(check_shape(fn, "flow2", flow2, N, 2, H, W));
+    TRY(check_shape(fn, "gt", gt, N, C, H, W));
+    TRY(check_shape(fn, "fused", fused, N, C, H, W));
+    TRY(check_shape(fn, "residual", residual, N, C, H, W));
+    TRY(check_shape(fn, "occ_fwd", occ_fwd, N, 1, H, W));
+    TRY(check_shape(fn, "occ_bwd", occ_bwd, N, 1, H, W));
+    const int dt = image1->dtype;
+    if (image2->dtype != dt || flow1->dtype != dt || flow2->dtype != dt || gt->dtype != dt)
+        return set_error(DCB_E_DTYPE, "%s: all tensors must share one dtype", fn);
+    TRY(check_out(fn, "fused", fused, dt, elem_size(dt)));
+    TRY(check_out(fn, "residual", residual, dt, elem_size(dt)));
+    TRY(check_out(fn, "occ_fwd", occ_fwd, dt, elem_size(dt)));
+    TRY(check_out(fn, "occ_bwd", occ_bwd, dt, elem_size(dt)));
+    return residual_bidir_impl(image1, image2, flow1, flow2, gt, fused, residual, occ_fwd, occ_bwd, ws, ws_bytes, flags,
                                (cudaStream_t)stream);
 }
 

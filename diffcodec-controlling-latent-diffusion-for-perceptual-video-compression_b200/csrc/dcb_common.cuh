@@ -192,6 +192,18 @@ __device__ __forceinline__ float occlusion(float wx, float wy, float d, float mx
     return add_rn(mul_rn(ex, ex), mul_rn(ey, ey)) > __uint_as_float(0x3DB851EDu) ? 1.f : 0.f;
 }
 
+// soft_fuse (improv_experiments.ipynb cell 3) of two warps on the VALID masks 1 - occ_fwd, 1 - occ_bwd of two binary occlusion
+// masks: clamp(M) / (M.sum() + 1e-6) takes one of three values, 0, 1 / (1 + 1e-6) or 1 / (2 + 1e-6) (IEEE divisions of
+// constants, folded at compile time: exactly what the per-pixel division gives); where both references are occluded
+// (M_fwd + M_bwd < 0.5) the result is 0.5 * (warped1 + warped2). Equal to bidir_fuse(w1, w2, 1 - of, 1 - ob, of, ob).
+__device__ __forceinline__ float bidir_soft_fuse(float w1, float w2, float of, float ob) {
+    const float one_of_one = 1.f / (1.f + 0.000001f), one_of_two = 1.f / (2.f + 0.000001f);
+    const bool v1 = of == 0.f, v2 = ob == 0.f;
+    if (!v1 && !v2) return mul_rn(0.5f, add_rn(w1, w2));
+    const float k1 = v1 ? (v2 ? one_of_two : one_of_one) : 0.f, k2 = v2 ? (v1 ? one_of_two : one_of_one) : 0.f;
+    return add_rn(mul_rn(k1, w1), mul_rn(k2, w2));
+}
+
 // Bilinear footprint of one source pixel: softsplat.py:298-318 (and :386-404, :457-470).
 template <class A> struct Foot {
     A fx, fy;        // landing position

@@ -27,7 +27,8 @@
 //     and the post-op (eps rule, divide, (1 - mask), cast, saved normaliser) never touch memory;
 //  5. epilogues besides the normalise: the occlusion test of compute_mask, and the conditioning recipe's second pass
 //     (KIND = 1: a 2-channel rider scattered with the same footprints into float2 cells, one epilogue that normalises,
-//     tests occlusion, fuses and subtracts) -- two pixels per lane with 256-bit cell loads where the layout allows.
+//     tests occlusion, fuses and subtracts) -- two pixels per lane with 256-bit cell loads where the layout allows; the
+//     two-reference recipe runs the same rider scatter twice (KIND = 2, 3: bidir_chunk epilogues).
 //  What bounds it (DESIGN.md section 4.1): the scatter launch's time is its reduction sector-ops x ~2.4 L2 slice clocks.
 //
 // Replaces controlnet/softsplat.py:240-270 (pre/post ops) + :281-345 (zero-init + softsplat_out).
@@ -746,6 +747,141 @@ __device__ __forceinline__ void recipe_chunk_v2(const PipeArgs& a, int frame, in
 }
 
 // ---------------------------------------------------------------------------------------------
+// two-reference recipe (dcb_residual_bidir): the rider scatter above, run twice with the roles of the frames swapped.
+//   pass A (KIND 2): image2 splatted by flow2, flow1 riding. Epilogue: warped2 = S / (D + 1e-7), parked (rounded to T) in the
+//                    caller's `fused` buffer; occ_fwd = compute_mask(flow1, flow2), tested against flow2 at the target
+//   pass B (KIND 3): image1 splatted by flow1, flow2 riding. Epilogue: warped1; occ_bwd = compute_mask(flow2, flow1), tested
+//                    against flow1; soft_fuse(warped1, warped2, 1 - occ_fwd, 1 - occ_bwd); fused and gt - fused stored once
+// Pass B reads what pass A's epilogues wrote (warped2 in `fused`, the occ_fwd plane), as the one-reference recipe reads its
+// mask plane: every launch of the chain waits (griddepcontrol.wait) until its predecessor has completed and its writes are
+// visible, and that predecessor did the same, so all of pass A is visible to every launch of pass B.
+// ---------------------------------------------------------------------------------------------
+template <class T, int C>
+__device__ __forceinline__ void bidir_pixel(const float (&sv)[4], float qx, float qy, float mx, float my, float& occ, float* warped) {
+    const float d = sv[C];
+    occ = occlusion(qx, qy, d, mx, my);                                  // control_utils.py:15-16
+    const float scale = __frcp_rn(add_rn(d, 0.0000001f));                // softsplat.py:256-258, :270
+#pragma unroll
+    for (int c = 0; c < C; ++c) warped[c] = round_as<T>(mul_rn(sv[c], scale));
+}
+
+template <class T, int CA, bool PASS_B>
+__device__ __forceinline__ void bidir_chunk(const PipeArgs& a, int frame, int chunk, float* acc, float* acc2, int lane) {
+    constexpr int C = CA - 1;
+    T* fo = (T*)a.out + (long long)frame * C * a.HW;                    // pass A: warped2 out; pass B: warped2 in, fused out
+    T* ro = (T*)a.residual + (long long)frame * C * a.HW;
+    const T* oo = (const T*)a.occ_other + (long long)frame * a.HW;
+    T* mo = a.mask_out ? (T*)a.mask_out + (long long)frame * a.HW : nullptr;
+    const T* fbase = (const T*)a.epi_flow.p + frame * a.epi_flow.sN;
+    const T* gbase = (const T*)a.gt.p + frame * a.gt.sN;
+#pragma unroll 1
+    for (int b = 0; b < kChunk / (32 * kRPer); ++b) {
+        const unsigned base = (unsigned)chunk * kChunk + b * (32 * kRPer) + lane;
+        if (base - lane >= a.HW) break;
+        float4 s[kRPer]; float2 q[kRPer]; float mx[kRPer], my[kRPer];
+#pragma unroll
+        for (int i = 0; i < kRPer; ++i) {                                // every load of the batch in flight first
+            const unsigned r = base + i * 32;
+            s[i] = make_float4(0.f, 0.f, 0.f, 0.f); q[i] = make_float2(0.f, 0.f);
+            mx[i] = my[i] = 0.f;
+            if (r < a.HW) {
+                s[i] = __ldcg((const float4*)acc + r);
+                q[i] = __ldcg((const float2*)acc2 + r);
+                const int y = (int)(r / (unsigned)a.W), x = (int)(r - (unsigned)y * (unsigned)a.W);
+                const T* fp = fbase + (long long)y * a.epi_flow.sH + (long long)x * a.epi_flow.sW;
+                mx[i] = ld<float>(fp); my[i] = ld<float>(fp + a.epi_flow.sC);
+            }
+        }
+#pragma unroll
+        for (int i = 0; i < kRPer; ++i) {
+            const unsigned r = base + i * 32;
+            if (r < a.HW) {
+                __stcg((float4*)acc + r, make_float4(0.f, 0.f, 0.f, 0.f));   // accumulators leave the kernel all-zero
+                __stcg((float2*)acc2 + r, make_float2(0.f, 0.f));
+                const float sv[4] = {s[i].x, s[i].y, s[i].z, s[i].w};
+                float occ, wv[C > 0 ? C : 1];
+                bidir_pixel<T, C>(sv, q[i].x, q[i].y, mx[i], my[i], occ, wv);
+                if (mo) st<T, float>(mo + r, occ);
+                if (!PASS_B) {
+#pragma unroll
+                    for (int c = 0; c < C; ++c) st_stream(fo + (size_t)c * a.HW + r, wv[c]);
+                    continue;
+                }
+                const float of = ld_stream(oo + r);
+                const int y = (int)(r / (unsigned)a.W), x = (int)(r - (unsigned)y * (unsigned)a.W);
+                const T* gp = gbase + (long long)y * a.gt.sH + (long long)x * a.gt.sW;
+#pragma unroll
+                for (int c = 0; c < C; ++c) {
+                    const float f = bidir_soft_fuse(wv[c], ld_stream(fo + (size_t)c * a.HW + r), of, occ);
+                    st_stream(fo + (size_t)c * a.HW + r, f);
+                    st_stream(ro + (size_t)c * a.HW + r, sub_rn(ld_stream(gp + (long long)c * a.gt.sC), round_as<T>(f)));   // residual of the stored value
+                }
+            }
+        }
+    }
+}
+
+// two consecutive pixels per lane (a.flat2: every plane the epilogue touches is a plain, pair-aligned [H,W] plane)
+template <class T, int CA, bool PASS_B>
+__device__ __forceinline__ void bidir_chunk_v2(const PipeArgs& a, int frame, int chunk, float* acc, float* acc2, int lane) {
+    constexpr int C = CA - 1;
+    constexpr int kGroups = kRPer / 2;
+    T* fo = (T*)a.out + (long long)frame * C * a.HW;                    // pass A: warped2 out; pass B: warped2 in, fused out
+    T* ro = (T*)a.residual + (long long)frame * C * a.HW;
+    const T* oo = (const T*)a.occ_other + (long long)frame * a.HW;
+    T* mo = a.mask_out ? (T*)a.mask_out + (long long)frame * a.HW : nullptr;
+    const T* fbase = (const T*)a.epi_flow.p + frame * a.epi_flow.sN;
+    const T* gbase = (const T*)a.gt.p + frame * a.gt.sN;
+#pragma unroll 1
+    for (int b = 0; b < kChunk / (32 * kRPer); ++b) {
+        const unsigned base = (unsigned)chunk * kChunk + b * (32 * kRPer);
+        if (base >= a.HW) break;
+        float4 s[kGroups][2], q[kGroups]; float2 mx[kGroups], my[kGroups];
+#pragma unroll
+        for (int g = 0; g < kGroups; ++g) {                               // accumulator and flow loads of the batch in flight first
+            const unsigned r = base + g * 64 + lane * 2;
+            s[g][0] = s[g][1] = q[g] = make_float4(0.f, 0.f, 0.f, 0.f);
+            mx[g] = my[g] = make_float2(0.f, 0.f);
+            if (r < a.HW) {
+                ld_cells2(acc + (size_t)r * 4, s[g][0], s[g][1]);
+                q[g] = __ldcg((const float4*)(acc2 + (size_t)r * 2));
+                mx[g] = ld2_stream(fbase + r); my[g] = ld2_stream(fbase + a.epi_flow.sC + r);
+            }
+        }
+#pragma unroll
+        for (int g = 0; g < kGroups; ++g) {
+            const unsigned r = base + g * 64 + lane * 2;
+            if (r < a.HW) {
+                // pass B: the streamed operands of this pair, issued before the accumulator cells are re-zeroed
+                float2 of = make_float2(0.f, 0.f), gv[C > 0 ? C : 1], w2[C > 0 ? C : 1];
+                if (PASS_B) {
+                    of = ld2_stream(oo + r);
+#pragma unroll
+                    for (int c = 0; c < C; ++c) { gv[c] = ld2_stream(gbase + (long long)c * a.gt.sC + r); w2[c] = ld2_stream(fo + (size_t)c * a.HW + r); }
+                }
+                zero_cells2(acc + (size_t)r * 4);                         // accumulators leave the kernel all-zero
+                __stcg((float4*)(acc2 + (size_t)r * 2), make_float4(0.f, 0.f, 0.f, 0.f));
+                const float s0[4] = {s[g][0].x, s[g][0].y, s[g][0].z, s[g][0].w}, s1[4] = {s[g][1].x, s[g][1].y, s[g][1].z, s[g][1].w};
+                float w0v[C > 0 ? C : 1], w1v[C > 0 ? C : 1], ob0, ob1;
+                bidir_pixel<T, C>(s0, q[g].x, q[g].y, mx[g].x, my[g].x, ob0, w0v);
+                bidir_pixel<T, C>(s1, q[g].z, q[g].w, mx[g].y, my[g].y, ob1, w1v);
+                if (mo) st_stream2(mo + r, ob0, ob1);
+#pragma unroll
+                for (int c = 0; c < C; ++c) {
+                    if (!PASS_B) {
+                        st_stream2(fo + (size_t)c * a.HW + r, w0v[c], w1v[c]);
+                    } else {
+                        const float f0 = bidir_soft_fuse(w0v[c], w2[c].x, of.x, ob0), f1 = bidir_soft_fuse(w1v[c], w2[c].y, of.y, ob1);
+                        st_stream2(fo + (size_t)c * a.HW + r, f0, f1);
+                        st_stream2(ro + (size_t)c * a.HW + r, sub_rn(gv[c].x, round_as<T>(f0)), sub_rn(gv[c].y, round_as<T>(f1)));   // residual of the stored values
+                    }
+                }
+            }
+        }
+    }
+}
+
+// ---------------------------------------------------------------------------------------------
 // the step kernel: warp w of CTA b owns item 4b + w; normalise items first, then scatter items
 // ---------------------------------------------------------------------------------------------
 // one epilogue item: chunk `chunk` of frame `z` of the group being normalised
@@ -756,6 +892,11 @@ __device__ __forceinline__ void epilogue_item(const PipeArgs& a, unsigned z, uns
     if (KIND == 1) {
         if (a.flat2) recipe_chunk_v2<T, CA>(a, f, (int)chunk, acc, a.acc2_n + z * ((size_t)a.HW * 2), lane);
         else recipe_chunk<T, CA>(a, f, (int)chunk, acc, a.acc2_n + z * ((size_t)a.HW * 2), lane);
+        return;
+    }
+    if (KIND == 2 || KIND == 3) {
+        if (a.flat2) bidir_chunk_v2<T, CA, KIND == 3>(a, f, (int)chunk, acc, a.acc2_n + z * ((size_t)a.HW * 2), lane);
+        else bidir_chunk<T, CA, KIND == 3>(a, f, (int)chunk, acc, a.acc2_n + z * ((size_t)a.HW * 2), lane);
         return;
     }
     if (a.epi == 1) { if (a.flat2) mask_chunk_v2<T>(a, f, (int)chunk, acc, lane); else mask_chunk<T>(a, f, (int)chunk, acc, lane); }
@@ -785,7 +926,8 @@ __global__ void __launch_bounds__(32 * kEpiWarps, KIND ? kMinCtasRecipe / kEpiWa
     epilogue_item<T, MODE, CA, KIND>(a, blockIdx.y, chunk, threadIdx.x & 31);
 }
 
-// KIND 0: softsplat / occlusion mask; KIND 1: the conditioning recipe's second pass (rider scatter + recipe epilogue)
+// KIND 0: softsplat / occlusion mask; KIND 1: the conditioning recipe's second pass (rider scatter + recipe epilogue);
+// KIND 2, 3: the two passes of the two-reference recipe (rider scatter + bidir_chunk epilogues)
 template <class T, class TF, int MODE, int CA, int KIND>
 __global__ void __launch_bounds__(kPipeThreads, KIND ? kMinCtasRecipe : kMinCtas) k_splat_step(const __grid_constant__ PipeArgs a) {
     // Programmatic dependent launch: let the next step's grid start being scheduled while this one
@@ -808,8 +950,8 @@ __global__ void __launch_bounds__(kPipeThreads, KIND ? kMinCtasRecipe : kMinCtas
         // the bottom rows of a frame (dispatched last) are cut into single-pass strips: the grid's tail drains in finer steps
         const int by = (int)blockIdx.y;
         const int y_first = by < a.ny_big ? by * kStripH : a.ny_big * kStripH + (by - a.ny_big) * kRows;
-        scatter_strip<T, TF, MODE, CA, KIND == 1>(a, a.s_frame0 + (int)zs, (int)blockIdx.x, y_first, by < a.ny_big ? kPasses : 1, a.acc_s + zs * frame_floats,
-                                                  KIND == 1 ? a.acc2_s + zs * ((size_t)a.HW * 2) : nullptr, lane);
+        scatter_strip<T, TF, MODE, CA, KIND != 0>(a, a.s_frame0 + (int)zs, (int)blockIdx.x, y_first, by < a.ny_big ? kPasses : 1, a.acc_s + zs * frame_floats,
+                                                  KIND != 0 ? a.acc2_s + zs * ((size_t)a.HW * 2) : nullptr, lane);
     }
 }
 
@@ -853,7 +995,7 @@ template <class T, class TF, int MODE, int CA, int KIND = 0> static int launch_s
     const unsigned gx = (unsigned)a.tiles_x;
     const unsigned rows_n = (unsigned)((a.tn + a.tiles_x - 1) / a.tiles_x);
     const unsigned gy = rows_n > (unsigned)a.tiles_y ? rows_n : (unsigned)a.tiles_y;
-    const bool one_slot = g_pipe_ring_slots == 1 || KIND == 1;
+    const bool one_slot = g_pipe_ring_slots == 1 || KIND != 0;
     for (int k = 0; k <= (one_slot ? 2 * groups - 1 : groups); ++k) {
         // two slots: launch k = normalise(group k-1) + scatter(group k); one slot: launch 2g = scatter(g), launch 2g+1 = normalise(g)
         const int gs = one_slot ? ((k & 1) ? -1 : k / 2) : (k < groups ? k : -1);
@@ -967,26 +1109,24 @@ long long recipe_pipe_workspace(long long N, long long H, long long W) {
     return align_up(G * H * W * 16, 256) + align_up(G * H * W * 8, 256);
 }
 
-template <class T> static int launch_recipe(PipeArgs& a, cudaStream_t st) {
+template <class T, int KIND> static int launch_recipe(PipeArgs& a, cudaStream_t st) {
     switch (a.C) {
-        case 1: return launch_steps<T, T, DCB_MODE_SOFT, 2, 1>(a, st);
-        case 2: return launch_steps<T, T, DCB_MODE_SOFT, 3, 1>(a, st);
-        case 3: return launch_steps<T, T, DCB_MODE_SOFT, 4, 1>(a, st);
+        case 1: return launch_steps<T, T, DCB_MODE_SOFT, 2, KIND>(a, st);
+        case 2: return launch_steps<T, T, DCB_MODE_SOFT, 3, KIND>(a, st);
+        case 3: return launch_steps<T, T, DCB_MODE_SOFT, 4, KIND>(a, st);
     }
     return set_error(DCB_E_LIMIT, "recipe_pipe: %d image channels", a.C);
 }
 
-// Preconditions (checked by the caller): 1 <= C <= 3, one dtype (F32/BF16) for every tensor, contiguous outputs,
-// pipe_supported() for every strided input, workspace >= recipe_pipe_workspace() and all-zero.
-int recipe_pipe_impl(const DcbTensor* image1, const DcbTensor* flow1, const DcbTensor* flow2, const DcbTensor* gt,
-                     const DcbTensor* fused, const DcbTensor* residual, const DcbTensor* occ_fwd, const DcbTensor* occ_bwd,
-                     void* ws, int variant, cudaStream_t st) {
+// the arguments of one rider pass: `in` (C channels) and `rider` (2 channels) splatted together by `flow` with the all-ones
+// metric, the occlusion epilogue comparing with `flow` at the target; accumulators [G frames of float4][G frames of float2] in ws
+static PipeArgs rider_args(const DcbTensor* in, const DcbTensor* flow, const DcbTensor* rider, const DcbTensor* gt, void* ws) {
     PipeArgs a = {};
     a.ones = 1; a.epi = 3;
-    a.in = make_view(image1); a.flow = make_view(flow1); a.metric = make_view(nullptr); a.mask = make_view(nullptr);
-    a.in2 = make_view(flow2); a.epi_flow = make_view(flow1); a.gt = make_view(gt);
-    a.N = (int)image1->size[0]; a.C = (int)image1->size[1]; a.H = (int)image1->size[2]; a.W = (int)image1->size[3];
-    a.HW = (unsigned)(image1->size[2] * image1->size[3]);
+    a.in = make_view(in); a.flow = make_view(flow); a.metric = make_view(nullptr); a.mask = make_view(nullptr);
+    a.in2 = make_view(rider); a.epi_flow = make_view(flow); a.gt = make_view(gt);
+    a.N = (int)in->size[0]; a.C = (int)in->size[1]; a.H = (int)in->size[2]; a.W = (int)in->size[3];
+    a.HW = (unsigned)(in->size[2] * in->size[3]);
     a.eps = DCB_EPS_ADD;
     a.G = (int)group_frames(a.N, a.H, a.W, 24);
     a.tiles_x = (a.W + 31) / 32;
@@ -994,19 +1134,58 @@ int recipe_pipe_impl(const DcbTensor* image1, const DcbTensor* flow1, const DcbT
     a.tiles_y = a.ny_big + (a.H - a.ny_big * kStripH + kRows - 1) / kRows;
     a.ts = a.tiles_x * a.tiles_y;
     a.tn = (int)((a.HW + kChunk - 1) / kChunk);
-    a.out = fused->ptr; a.residual = residual->ptr; a.norm = nullptr;
+    a.norm = nullptr;
+    a.vec4 = 0;
+    a.acc = (float*)ws;
+    a.acc2_s = a.acc2_n = (float*)((char*)ws + align_up((long long)a.G * a.HW * 16, 256));
+    return a;
+}
+
+// Preconditions (checked by the caller): 1 <= C <= 3, one dtype (F32/BF16) for every tensor, contiguous outputs,
+// pipe_supported() for every strided input, workspace >= recipe_pipe_workspace() and all-zero.
+int recipe_pipe_impl(const DcbTensor* image1, const DcbTensor* flow1, const DcbTensor* flow2, const DcbTensor* gt,
+                     const DcbTensor* fused, const DcbTensor* residual, const DcbTensor* occ_fwd, const DcbTensor* occ_bwd,
+                     void* ws, int variant, cudaStream_t st) {
+    PipeArgs a = rider_args(image1, flow1, flow2, gt, ws);
+    a.out = fused->ptr; a.residual = residual->ptr;
     a.occ_other = occ_fwd->ptr;
     a.mask_out = occ_bwd ? occ_bwd->ptr : nullptr;
     a.variant = variant;
-    a.vec4 = 0;
     a.flat2 = (a.HW % 2 == 0 && planes_pair_aligned(flow1, a.W) && planes_pair_aligned(gt, a.W) && planes_pair_aligned(fused, a.W) &&
                planes_pair_aligned(residual, a.W) && planes_pair_aligned(occ_fwd, a.W) && planes_pair_aligned(occ_bwd, a.W) &&
                (((uintptr_t)ws + align_up((long long)a.G * a.HW * 16, 256)) & 15) == 0) ? 1 : 0;
-    a.acc = (float*)ws;
-    a.acc2_s = a.acc2_n = (float*)((char*)ws + align_up((long long)a.G * a.HW * 16, 256));
-    if (image1->dtype == DCB_F32) return launch_recipe<float>(a, st);
-    if (image1->dtype == DCB_BF16) return launch_recipe<__nv_bfloat16>(a, st);
+    if (image1->dtype == DCB_F32) return launch_recipe<float, 1>(a, st);
+    if (image1->dtype == DCB_BF16) return launch_recipe<__nv_bfloat16, 1>(a, st);
     return set_error(DCB_E_DTYPE, "recipe_pipe: unsupported dtype %d", image1->dtype);
+}
+
+// ---------------------------------------------------------------------------------------------
+// two-reference recipe: pass A (image2 + rider flow1 by flow2, KIND 2) then pass B (image1 + rider flow2 by flow1, KIND 3),
+// four launches per frame group as the one-reference recipe. occ_fwd is required (the caller's plane or a workspace plane:
+// pass B reads it); occ_bwd is optional. Preconditions as recipe_pipe_impl.
+// ---------------------------------------------------------------------------------------------
+int bidir_pipe_impl(const DcbTensor* image1, const DcbTensor* image2, const DcbTensor* flow1, const DcbTensor* flow2,
+                    const DcbTensor* gt, const DcbTensor* fused, const DcbTensor* residual, const DcbTensor* occ_fwd,
+                    const DcbTensor* occ_bwd, void* ws, cudaStream_t st) {
+    PipeArgs a = rider_args(image2, flow2, flow1, gt, ws);
+    a.out = fused->ptr; a.residual = residual->ptr;
+    a.occ_other = nullptr;
+    a.mask_out = occ_fwd->ptr;
+    // one layout decision for both passes: every plane either epilogue touches
+    a.flat2 = (a.HW % 2 == 0 && planes_pair_aligned(flow1, a.W) && planes_pair_aligned(flow2, a.W) && planes_pair_aligned(gt, a.W) &&
+               planes_pair_aligned(fused, a.W) && planes_pair_aligned(residual, a.W) && planes_pair_aligned(occ_fwd, a.W) &&
+               planes_pair_aligned(occ_bwd, a.W) && (((uintptr_t)ws + align_up((long long)a.G * a.HW * 16, 256)) & 15) == 0) ? 1 : 0;
+    const int dt = image1->dtype;
+    if (dt != DCB_F32 && dt != DCB_BF16) return set_error(DCB_E_DTYPE, "bidir_pipe: unsupported dtype %d", dt);
+    int rc = dt == DCB_F32 ? launch_recipe<float, 2>(a, st) : launch_recipe<__nv_bfloat16, 2>(a, st);
+    if (rc != DCB_OK) return rc;
+    const int flat2 = a.flat2;
+    a = rider_args(image1, flow1, flow2, gt, ws);
+    a.out = fused->ptr; a.residual = residual->ptr;
+    a.occ_other = occ_fwd->ptr;
+    a.mask_out = occ_bwd ? occ_bwd->ptr : nullptr;
+    a.flat2 = flat2;
+    return dt == DCB_F32 ? launch_recipe<float, 3>(a, st) : launch_recipe<__nv_bfloat16, 3>(a, st);
 }
 
 }  // namespace dcb

@@ -6,6 +6,9 @@ Per sample the reference issues 4 ``softsplat`` calls (two of them identical, SU
 two norms / compares, a cat / clamp / sum / div fusion and a subtraction: ~45 launches for a
 batch of ONE frame. ``residual_conditioning`` does the same arithmetic for N frames in two
 pipeline passes (dcb_residual_fused: four launches per frame group).
+
+``residual_conditioning_bidir`` builds the residual the datasets intended (SURVEY.md App. B-6): BOTH decoded
+I-frames warped by their own flows, fused by occlusion, subtracted -- also two pipeline passes (dcb_residual_bidir).
 """
 from __future__ import annotations
 
@@ -14,9 +17,10 @@ from torch.utils.data import Dataset
 
 from . import _lib
 from .control_utils import compute_mask
+from .extractors import bidir_fuse
 from .softsplat import softsplat, is_deterministic
 
-__all__ = ["residual_conditioning", "ResidueDataset", "WarpingDatasetWrapper"]
+__all__ = ["residual_conditioning", "residual_conditioning_bidir", "ResidueDataset", "WarpingDatasetWrapper"]
 
 _VARIANTS = {"dataset": _lib.RECIPE_DATASET, "wrapper": _lib.RECIPE_WRAPPER}
 
@@ -77,6 +81,71 @@ def residual_conditioning(image1, flow1, flow2, gt, variant: str = "dataset", re
         if rc != 0:
             _lib.invalidate_acc(dev)
         _lib.check(rc, "dcb_residual_fused")
+    if return_masks:
+        return fused, residual, occ_fwd, occ_bwd
+    return fused, residual
+
+
+def _composed_bidir(image1, image2, flow1, flow2, gt):
+    """General path of the two-reference builder (any channel count / fp64 / deterministic): the single-op kernels."""
+    ones = torch.ones_like(flow1[:, :1])
+    warped1 = softsplat(tenIn=image1, tenFlow=flow1, tenMetric=ones, strMode="soft")
+    warped2 = softsplat(tenIn=image2, tenFlow=flow2, tenMetric=ones, strMode="soft")
+    occ_fwd = compute_mask(flow1, flow2).to(image1.dtype)
+    occ_bwd = compute_mask(flow2, flow1).to(image1.dtype)
+    if image1.dtype == torch.float64:
+        # the fusion kernel is F32/BF16 only: the fp64 composition fuses as _composed does (soft_fuse, improv_experiments.ipynb
+        # cell 3, on the valid masks; no .any() host sync)
+        conf = torch.cat([1 - occ_fwd, 1 - occ_bwd], dim=1)
+        w = conf / (conf.sum(dim=1, keepdim=True) + 1e-6)
+        fused = w[:, :1] * warped1 + w[:, 1:] * warped2
+        holes = (occ_fwd + occ_bwd) > 1.5
+        fused = torch.where(holes.expand_as(fused), 0.5 * (warped1 + warped2), fused)
+    else:
+        # soft_fuse on the valid masks 1 - occ == bidir_fuse with the occlusion masks as the hole test (binary masks)
+        fused = bidir_fuse(warped1, warped2, 1 - occ_fwd, 1 - occ_bwd, occ_fwd, occ_bwd)
+    return fused, gt - fused, occ_fwd, occ_bwd
+
+
+@torch.no_grad()
+def residual_conditioning_bidir(image1, image2, flow1, flow2, gt, return_masks: bool = False):
+    """Two-reference fused frame + residual for a batch of inter frames.
+
+    image1, image2, gt: [N,C,H,W]; flow1 moves image1, flow2 moves image2: [N,2,H,W]. The caller states the pairing (the
+    reference's dataset and extractor pair the frames of ``local_conditions`` with the flows in opposite ways). Computes
+    ``soft_fuse(softsplat(image1, flow1), softsplat(image2, flow2), 1 - compute_mask(flow1, flow2),
+    1 - compute_mask(flow2, flow1))`` (improv_experiments.ipynb cell 3, mask pairing of ``extractors.py:290-295``) and
+    ``gt - fused``. Inputs may be strided views; an I-frame shared by several inter frames can be an ``expand``ed batch.
+    Returns (fused, residual) or (fused, residual, occ_fwd, occ_bwd).
+    """
+    assert image1.dim() == 4 and image1.shape == image2.shape == gt.shape and flow1.shape == flow2.shape
+    assert flow1.shape[0] == image1.shape[0] and flow1.shape[1] == 2 and flow1.shape[2:] == image1.shape[2:]
+    assert image1.is_cuda, "residual_conditioning_bidir has no CPU path"
+    n, c, h, w = image1.shape
+    dt_ = image1.dtype
+    fusable = (c <= 3 and dt_ in (torch.float32, torch.bfloat16) and all(t.dtype == dt_ for t in (image2, flow1, flow2, gt))
+               and not is_deterministic())
+    if not fusable:
+        fused, residual, occ_fwd, occ_bwd = _composed_bidir(image1, image2.to(dt_), flow1.to(dt_), flow2.to(dt_), gt.to(dt_))
+    else:
+        lib = _lib.lib()
+        dev = image1.device
+        fused = torch.empty((n, c, h, w), dtype=dt_, device=dev)
+        residual = torch.empty_like(fused)
+        # the masks get their own storage, as in residual_conditioning: the in-workspace planes would dirty the kept-zero buffer
+        occ_fwd = torch.empty((n, 1, h, w), dtype=dt_, device=dev)
+        occ_bwd = torch.empty_like(occ_fwd)
+        need = lib.dcb_residual_workspace_bytes(n, c, h, w)        # the same requirement as dcb_residual_fused
+        dt = _lib._DTYPES[dt_]
+        scratch = _lib.fwd_is_scratch(n, c, h, w, dt, _lib.MODE_SOFT) and _lib.fwd_is_scratch(n, 2, h, w, dt, _lib.MODE_SOFT)
+        ws = _lib.workspace(dev, need, "scratch" if scratch else "acc")
+        with _lib.on_device(dev):
+            rc = lib.dcb_residual_bidir(_lib.desc(image1), _lib.desc(image2), _lib.desc(flow1), _lib.desc(flow2), _lib.desc(gt),
+                                        _lib.desc(fused), _lib.desc(residual), _lib.desc(occ_fwd), _lib.desc(occ_bwd),
+                                        ws.data_ptr(), ws.numel(), 0 if scratch else _lib.FLAG_WS_CLEAN, _lib.stream_ptr(dev))
+        if rc != 0:
+            _lib.invalidate_acc(dev)
+        _lib.check(rc, "dcb_residual_bidir")
     if return_masks:
         return fused, residual, occ_fwd, occ_bwd
     return fused, residual

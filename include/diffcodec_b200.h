@@ -223,6 +223,31 @@ int dcb_residual_fused(const DcbTensor* image1, const DcbTensor* flow1, const Dc
                        int32_t variant, int32_t flags, void* stream);
 
 /*
+ * Two-reference conditioning builder: the bidirectional blend the reference's datasets intended (SURVEY.md App. B-6) with the
+ * mask <-> warp pairing of Bi_Dir_FeatureExtractor (controlnet/extractors.py:290-295), built from reference functions only:
+ *   ones = all-ones metric
+ *   warped1 = softsplat(image1, flow1, ones, 'soft');  warped2 = softsplat(image2, flow2, ones, 'soft')   (softsplat.py:232-274)
+ *   occ_fwd = compute_mask(flow1, flow2);  occ_bwd = compute_mask(flow2, flow1)                          (control_utils.py:11-17)
+ *   fused = soft_fuse(warped1, warped2, 1 - occ_fwd, 1 - occ_bwd)     (improv_experiments.ipynb cell 3: where both references
+ *                                                                      are occluded, 0.5 * (warped1 + warped2))
+ *   residual = gt - fused
+ * image_k is moved by flow_k: the caller states the pairing (the reference's dataset and extractor pair the channels of
+ * local_conditions with the flows in opposite ways). Rounding follows the composition: warps rounded to the tensor dtype,
+ * fused stored, residual of the stored value. Two pipeline passes, four launches per frame group (image2 + flow1 splatted by
+ * flow2 with the warp / occ_fwd epilogue; image1 + flow2 splatted by flow1 with the fuse / residual epilogue).
+ *
+ *   image1, image2, gt [N,C,H,W] (1 <= C <= 3; one dtype, F32 or BF16, for every tensor); flow1, flow2 [N,2,H,W];
+ *   inputs may have any strides, a stride-0 batch included (one I-frame serving several inter frames)
+ *   fused, residual [N,C,H,W] contiguous; occ_fwd / occ_bwd [N,1,H,W] optional outputs
+ *   workspace: dcb_residual_workspace_bytes(N, C, H, W) -- the requirement is the same as dcb_residual_fused's;
+ *   DCB_FLAG_WS_CLEAN protocol as dcb_residual_fused
+ */
+int dcb_residual_bidir(const DcbTensor* image1, const DcbTensor* image2, const DcbTensor* flow1, const DcbTensor* flow2,
+                       const DcbTensor* gt, const DcbTensor* fused, const DcbTensor* residual,
+                       const DcbTensor* occ_fwd, const DcbTensor* occ_bwd,
+                       void* workspace, int64_t workspace_bytes, int32_t flags, void* stream);
+
+/*
  * Confidence fusion of the two warped maps of a bi-directional block, without the host sync.
  * Replaces controlnet/extractors.py:298-310 (also :193-205 and controlnet/residual_utils.py:181-193):
  *   conf = clamp(cat(conf_a, conf_b), min=0); w = conf / (conf.sum(1) + 1e-6);
