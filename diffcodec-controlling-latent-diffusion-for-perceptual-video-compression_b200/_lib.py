@@ -24,7 +24,7 @@ EPS_ADD, EPS_ZERO, EPS_CLIP = 0, 1, 2
 FLAG_DETERMINISTIC, FLAG_WS_CLEAN = 1, 2
 RECIPE_DATASET, RECIPE_WRAPPER = 0, 1
 FLOW_BILINEAR_RESCALE, FLOW_ADAPTIVE_AVG, FLOW_BILINEAR_NORMALIZE = 0, 1, 2
-PYRAMID_NO_MASKS = 4
+PYRAMID_NO_MASKS, PYRAMID_NO_HOLES = 4, 8
 RESAMPLE_NONE, RESAMPLE_MUL, RESAMPLE_DIV = 0, 1, 2
 
 E_NULL, E_SHAPE, E_DTYPE, E_MODE, E_WORKSPACE, E_LIMIT, E_ALIGN = -1, -2, -3, -4, -5, -6, -7
@@ -83,6 +83,8 @@ SYMBOLS = {
     "dcb_flow_resize": (ctypes.c_int, [_P, _P, ctypes.c_int32, ctypes.c_void_p]),
     "dcb_bidir_pyramid_workspace_bytes": (ctypes.c_int64, [ctypes.c_void_p, ctypes.c_int32]),
     "dcb_bidir_pyramid_fwd": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int32, ctypes.c_void_p, ctypes.c_int64, ctypes.c_int32, ctypes.c_void_p]),
+    "dcb_bidir_pyramid_bwd_workspace_bytes": (ctypes.c_int64, [ctypes.c_void_p, ctypes.c_int32]),
+    "dcb_bidir_pyramid_bwd": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int32, ctypes.c_void_p, ctypes.c_int64, ctypes.c_int32, ctypes.c_void_p]),
     "dcb_resample_batch": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int32, ctypes.c_void_p]),
     "dcb_convert": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int32, ctypes.c_void_p, ctypes.c_int32, ctypes.c_int64, ctypes.c_float, ctypes.c_void_p]),
     "dcb_residual_fused": (ctypes.c_int, [_P] * 8 + [ctypes.c_void_p, ctypes.c_int64, ctypes.c_int32, ctypes.c_int32, ctypes.c_void_p]),
@@ -193,6 +195,7 @@ def desc(t: torch.Tensor | None):
 _tls = threading.local()
 _DESC_BYTES = _DESC_STRUCT.size            # 80
 _LEVEL_STRUCT = struct.Struct("13P")       # DcbPyramidLevel: 6 descriptor pointers + 7 raw output pointers
+_BWD_LEVEL_STRUCT = struct.Struct("19P")   # DcbPyramidBwdLevel: 7 descriptor pointers + 6 saved + 6 gradient raw pointers
 _JOB_STRUCT = struct.Struct("PPiiff")      # DcbResampleJob
 _ARENA_BYTES = 1 << 14
 
@@ -234,6 +237,29 @@ def pack_pyramid(levels, outputs):
                 off += _DESC_BYTES
         ptrs += [0 if o is None else o.data_ptr() for o in outs]
         _LEVEL_STRUCT.pack_into(buf, l * _LEVEL_STRUCT.size, *ptrs)
+    return base
+
+
+def pack_pyramid_bwd(levels, saved, grads):
+    """levels: per scale (grad_fused, first, last, flow_f, flow_b, metric_f | None, metric_b | None); saved: per scale the six
+    forward outputs (warped_f, warped_b, norm_f, norm_b, occ_f, occ_b); grads: per scale six tensors or None (grad_first,
+    grad_last, grad_flow_f, grad_flow_b, grad_metric_f, grad_metric_b). Returns the address of a DcbPyramidBwdLevel[len(levels)]
+    that stays valid until the next pack_* call of this thread."""
+    buf, base = _arena()
+    n = len(levels)
+    off = n * _BWD_LEVEL_STRUCT.size
+    assert off + n * 7 * _DESC_BYTES <= _ARENA_BYTES
+    for l, (ins, sv, gr) in enumerate(zip(levels, saved, grads)):
+        ptrs = []
+        for t in ins:
+            if t is None:
+                ptrs.append(0)
+            else:
+                _pack_desc_into(buf, off, *_tensor_fields(t))
+                ptrs.append(base + off)
+                off += _DESC_BYTES
+        ptrs += [0 if o is None else o.data_ptr() for o in tuple(sv) + tuple(gr)]
+        _BWD_LEVEL_STRUCT.pack_into(buf, l * _BWD_LEVEL_STRUCT.size, *ptrs)
     return base
 
 

@@ -71,6 +71,8 @@ int bidir_block_bwd_impl(const DcbTensor*, const DcbTensor*, const DcbTensor*, c
 int flow_ingest_impl(const DcbTensor* flow, const DcbTensor* out, int mode, cudaStream_t st);
 long long pyramid_workspace(const DcbPyramidLevel* lv, int n);
 int bidir_pyramid_fwd_impl(const DcbPyramidLevel* lv, int n, void* ws, int flags, cudaStream_t st);
+long long pyramid_bwd_workspace(const DcbPyramidBwdLevel* lv, int n);
+int bidir_pyramid_bwd_impl(const DcbPyramidBwdLevel* lv, int n, void* ws, bool holes, cudaStream_t st);
 int resample_batch_impl(const DcbResampleJob* jobs, int n_jobs, cudaStream_t st);
 int convert_impl(const void* src, int src_dtype, void* dst, int dst_dtype, long long n, float scale, cudaStream_t st);
 extern int g_fwd_path;
@@ -587,36 +589,46 @@ int dcb_bidir_block_bwd(const DcbTensor* grad_fused, const DcbTensor* first, con
                                 grad_first, grad_last, grad_metric_f, grad_metric_b, ws, ws_bytes, (cudaStream_t)stream);
 }
 
+// the inputs of one pyramid level (forward and backward): dtype of every level = dtype of `first0`
+struct PyramidInputs { const DcbTensor *first, *last, *flow_f, *flow_b, *metric_f, *metric_b; };
+static int check_pyramid_inputs(const char* fn, const PyramidInputs& d, int l, const DcbTensor* first0) {
+    TRY(check_tensor(fn, "first", d.first, true));
+    TRY(check_tensor(fn, "last", d.last, true));
+    TRY(check_tensor(fn, "flow_f", d.flow_f, true));
+    TRY(check_tensor(fn, "flow_b", d.flow_b, true));
+    TRY(check_tensor(fn, "metric_f", d.metric_f, false));
+    TRY(check_tensor(fn, "metric_b", d.metric_b, false));
+    const long long N = d.first->size[0], C = d.first->size[1], H = d.first->size[2], W = d.first->size[3];
+    TRY(check_limits(fn, d.first));
+    TRY(check_shape(fn, "last", d.last, N, C, H, W));
+    TRY(check_shape(fn, "flow_f", d.flow_f, N, 2, H, W));
+    TRY(check_shape(fn, "flow_b", d.flow_b, N, 2, H, W));
+    TRY(check_shape(fn, "metric_f", d.metric_f, N, 1, H, W));
+    TRY(check_shape(fn, "metric_b", d.metric_b, N, 1, H, W));
+    const int dt = d.first->dtype;
+    if (dt != DCB_F32 && dt != DCB_BF16) return set_error(DCB_E_DTYPE, "%s: F32 or BF16 only, got %d", fn, dt);
+    if (dt != first0->dtype || d.last->dtype != dt || d.flow_f->dtype != dt || d.flow_b->dtype != dt ||
+        (d.metric_f && d.metric_f->dtype != dt) || (d.metric_b && d.metric_b->dtype != dt))
+        return set_error(DCB_E_DTYPE, "%s: all tensors of all levels must share one dtype", fn);
+    const DcbTensor* in32[6] = {d.first, d.last, d.flow_f, d.flow_b, d.metric_f, d.metric_b};
+    for (int i = 0; i < 6; ++i) {
+        if (!in32[i]) continue;
+        long long span = 0;
+        for (int k = 0; k < 4; ++k) span += (in32[i]->size[k] - 1) * (in32[i]->stride[k] < 0 ? -in32[i]->stride[k] : in32[i]->stride[k]);
+        if (span >= (1ll << 31)) return set_error(DCB_E_LIMIT, "%s: level %d: a tensor spans 2^31 elements or more", fn, l);
+    }
+    return DCB_OK;
+}
+
 static int check_pyramid(const char* fn, const DcbPyramidLevel* lv, int32_t n) {
     if (n < 0 || n > 4) return set_error(DCB_E_LIMIT, "%s: %d levels (at most 4 per call)", fn, n);
     if (n > 0 && !lv) return set_error(DCB_E_NULL, "%s: levels is required", fn);
+    if (n > 0) TRY(check_tensor(fn, "first", lv[0].first, true));
     for (int l = 0; l < n; ++l) {
         const DcbPyramidLevel& d = lv[l];
-        TRY(check_tensor(fn, "first", d.first, true));
-        TRY(check_tensor(fn, "last", d.last, true));
-        TRY(check_tensor(fn, "flow_f", d.flow_f, true));
-        TRY(check_tensor(fn, "flow_b", d.flow_b, true));
-        TRY(check_tensor(fn, "metric_f", d.metric_f, false));
-        TRY(check_tensor(fn, "metric_b", d.metric_b, false));
+        TRY(check_pyramid_inputs(fn, {d.first, d.last, d.flow_f, d.flow_b, d.metric_f, d.metric_b}, l, lv[0].first));
         const long long N = d.first->size[0], C = d.first->size[1], H = d.first->size[2], W = d.first->size[3];
-        TRY(check_limits(fn, d.first));
-        TRY(check_shape(fn, "last", d.last, N, C, H, W));
-        TRY(check_shape(fn, "flow_f", d.flow_f, N, 2, H, W));
-        TRY(check_shape(fn, "flow_b", d.flow_b, N, 2, H, W));
-        TRY(check_shape(fn, "metric_f", d.metric_f, N, 1, H, W));
-        TRY(check_shape(fn, "metric_b", d.metric_b, N, 1, H, W));
         const int dt = d.first->dtype;
-        if (dt != DCB_F32 && dt != DCB_BF16) return set_error(DCB_E_DTYPE, "%s: F32 or BF16 only, got %d", fn, dt);
-        if (dt != lv[0].first->dtype || d.last->dtype != dt || d.flow_f->dtype != dt || d.flow_b->dtype != dt ||
-            (d.metric_f && d.metric_f->dtype != dt) || (d.metric_b && d.metric_b->dtype != dt))
-            return set_error(DCB_E_DTYPE, "%s: all tensors of all levels must share one dtype", fn);
-        const DcbTensor* in32[6] = {d.first, d.last, d.flow_f, d.flow_b, d.metric_f, d.metric_b};
-        for (int i = 0; i < 6; ++i) {
-            if (!in32[i]) continue;
-            long long span = 0;
-            for (int k = 0; k < 4; ++k) span += (in32[i]->size[k] - 1) * (in32[i]->stride[k] < 0 ? -in32[i]->stride[k] : in32[i]->stride[k]);
-            if (span >= (1ll << 31)) return set_error(DCB_E_LIMIT, "%s: level %d: a tensor spans 2^31 elements or more", fn, l);
-        }
         if (N * C * H * W > 0 && !d.fused) return set_error(DCB_E_NULL, "%s: level %d: fused is required", fn, l);
         void* outs[7] = {d.fused, d.warped_f, d.warped_b, d.norm_f, d.norm_b, d.occ_f, d.occ_b};
         for (int i = 0; i < 7; ++i)                                   // norm_f / norm_b are fp32 whatever the tensor dtype
@@ -635,13 +647,52 @@ int64_t dcb_bidir_pyramid_workspace_bytes(const DcbPyramidLevel* levels, int32_t
 
 int dcb_bidir_pyramid_fwd(const DcbPyramidLevel* levels, int32_t n_levels, void* ws, int64_t ws_bytes, int32_t flags, void* stream) {
     const char* fn = "dcb_bidir_pyramid_fwd";
-    if (flags & ~(DCB_FLAG_WS_CLEAN | DCB_PYRAMID_NO_MASKS)) return set_error(DCB_E_MODE, "%s: unknown flags 0x%x", fn, flags);
+    if (flags & ~(DCB_FLAG_WS_CLEAN | DCB_PYRAMID_NO_MASKS | DCB_PYRAMID_NO_HOLES)) return set_error(DCB_E_MODE, "%s: unknown flags 0x%x", fn, flags);
     TRY(check_pyramid(fn, levels, n_levels));
     if (n_levels == 0) return DCB_OK;
     const long long need = pyramid_workspace(levels, n_levels);
     if (need > 0 && (!ws || ws_bytes < need || ((uintptr_t)ws & 255)))
         return set_error(DCB_E_WORKSPACE, "%s: workspace of %lld bytes (256 B aligned) required, got %lld", fn, need, (long long)ws_bytes);
     return bidir_pyramid_fwd_impl(levels, n_levels, ws, flags, (cudaStream_t)stream);
+}
+
+int64_t dcb_bidir_pyramid_bwd_workspace_bytes(const DcbPyramidBwdLevel* levels, int32_t n_levels) {
+    if (!levels || n_levels <= 0 || n_levels > 4) return 0;
+    for (int l = 0; l < n_levels; ++l) {
+        const DcbTensor* f = levels[l].first;
+        if (!f || f->size[0] < 0 || f->size[1] < 0 || f->size[2] < 0 || f->size[3] < 0) return 0;
+    }
+    return (int64_t)pyramid_bwd_workspace(levels, n_levels);
+}
+
+int dcb_bidir_pyramid_bwd(const DcbPyramidBwdLevel* levels, int32_t n_levels, void* ws, int64_t ws_bytes, int32_t flags, void* stream) {
+    const char* fn = "dcb_bidir_pyramid_bwd";
+    if (flags & ~DCB_PYRAMID_NO_HOLES) return set_error(DCB_E_MODE, "%s: flags 0x%x (only DCB_PYRAMID_NO_HOLES; NO_MASKS has no backward)", fn, flags);
+    if (n_levels < 1 || n_levels > 4) return set_error(DCB_E_LIMIT, "%s: %d levels (1 to 4 per call)", fn, n_levels);
+    if (!levels) return set_error(DCB_E_NULL, "%s: levels is required", fn);
+    TRY(check_tensor(fn, "first", levels[0].first, true));
+    for (int l = 0; l < n_levels; ++l) {
+        const DcbPyramidBwdLevel& d = levels[l];
+        TRY(check_pyramid_inputs(fn, {d.first, d.last, d.flow_f, d.flow_b, d.metric_f, d.metric_b}, l, levels[0].first));
+        const long long N = d.first->size[0], C = d.first->size[1], H = d.first->size[2], W = d.first->size[3];
+        const int dt = d.first->dtype;
+        TRY(check_tensor(fn, "grad_fused", d.grad_fused, true));
+        TRY(check_shape(fn, "grad_fused", d.grad_fused, N, C, H, W));
+        if (d.grad_fused->dtype != dt) return set_error(DCB_E_DTYPE, "%s: level %d: grad_fused dtype differs", fn, l);
+        if ((d.grad_metric_f && !d.metric_f) || (d.grad_metric_b && !d.metric_b))
+            return set_error(DCB_E_MODE, "%s: level %d: a metric gradient for an all-ones (NULL) metric", fn, l);
+        const void* saved[6] = {d.warped_f, d.warped_b, d.norm_f, d.norm_b, d.occ_f, d.occ_b};
+        const void* grads[6] = {d.grad_first, d.grad_last, d.grad_flow_f, d.grad_flow_b, d.grad_metric_f, d.grad_metric_b};
+        for (int i = 0; i < 6; ++i) {
+            if (N * C * H * W > 0 && !saved[i]) return set_error(DCB_E_NULL, "%s: level %d: saved forward output %d is required", fn, l, i);
+            if ((uintptr_t)saved[i] % (uintptr_t)((i == 2 || i == 3) ? 4 : elem_size(dt)) || (uintptr_t)grads[i] % (uintptr_t)elem_size(dt))
+                return set_error(DCB_E_ALIGN, "%s: level %d: a pointer is not aligned to its element size", fn, l);
+        }
+    }
+    const long long need = pyramid_bwd_workspace(levels, n_levels);
+    if (need > 0 && (!ws || ws_bytes < need || ((uintptr_t)ws & 255)))
+        return set_error(DCB_E_WORKSPACE, "%s: workspace of %lld bytes (256 B aligned) required, got %lld", fn, need, (long long)ws_bytes);
+    return bidir_pyramid_bwd_impl(levels, n_levels, ws, !(flags & DCB_PYRAMID_NO_HOLES), (cudaStream_t)stream);
 }
 
 int dcb_resample_batch(const DcbResampleJob* jobs, int32_t n_jobs, void* stream) {

@@ -7,27 +7,25 @@
 // kernels, 4 NVRTC cache lookups and one device->host stall per scale; in round 1 five library calls from Python. Here
 // the host enters the library once. Scales whose accumulators fit the L2 (every pyramid level of the live consumer) run
 // as TWO launches (pyramid.cu: all four scatter jobs, then masks + normalisation + fusion); bigger tensors run the
-// kernels of recipe.cu / splat_*.cu / fuse.cu back to back on the caller's stream.
+// kernels of recipe.cu / splat_*.cu / fuse.cu back to back on the caller's stream. The backward of every size is the
+// one-level pyramid backward (pyramid_bwd.cu, two launches).
 #include "dcb_common.cuh"
 
 namespace dcb {
 
 long long mask_workspace(long long N, long long H, long long W);
 long long splat_fwd_workspace(long long N, long long C, long long H, long long W, int dtype, int mode);
-long long splat_bwd_workspace(long long N, long long C, long long H, long long W, int dtype, int mode);
 int occlusion_mask_impl(const DcbTensor*, const DcbTensor*, const DcbTensor*, void*, long long, int, cudaStream_t);
 int splat_fwd_impl(const DcbTensor*, const DcbTensor*, const DcbTensor*, const DcbTensor*, const DcbTensor*, const DcbTensor*, void*,
                    long long, int, int, int, cudaStream_t);
-int splat_bwd_impl(const DcbTensor*, const DcbTensor*, const DcbTensor*, const DcbTensor*, const DcbTensor*, const DcbTensor*,
-                   const DcbTensor*, const DcbTensor*, const DcbTensor*, const DcbTensor*, void*, long long, int, int, cudaStream_t);
 int bidir_fuse_fwd_impl(const DcbTensor*, const DcbTensor*, const DcbTensor*, const DcbTensor*, const DcbTensor*, const DcbTensor*,
                         const DcbTensor*, cudaStream_t);
-int bidir_fuse_bwd_impl(const DcbTensor*, const DcbTensor*, const DcbTensor*, const DcbTensor*, const DcbTensor*, const DcbTensor*,
-                        const DcbTensor*, const DcbTensor*, const DcbTensor*, const DcbTensor*, const DcbTensor*, cudaStream_t);
 
 // pyramid.cu: the two-launch form (every scatter job in one launch, everything else in a second)
 long long pyramid_workspace(const DcbPyramidLevel* lv, int n);
 int bidir_pyramid_fwd_impl(const DcbPyramidLevel* lv, int n, void* ws, int flags, cudaStream_t st);
+long long pyramid_bwd_workspace(const DcbPyramidBwdLevel* lv, int n);
+int bidir_pyramid_bwd_impl(const DcbPyramidBwdLevel* lv, int n, void* ws, bool holes, cudaStream_t st);
 
 // One scale goes through the two-launch pyramid kernels when the accumulators of BOTH directions fit the L2 together
 // (every pyramid level of the live consumer does); bigger tensors keep the launch sequence below (frame-group pipeline
@@ -64,10 +62,13 @@ long long block_fwd_scratch_bytes(long long N, long long C, long long H, long lo
     return 2 * align_up(N * C * H * W * s, 256) + 2 * align_up(N * H * W * s, 256);
 }
 
-// scratch of the backward: splat backward scalars + gradients w.r.t. both warped maps + both fusion-confidence gradients
+// scratch of the backward: that of the one-level pyramid backward (both directions' target scalars, both confidence gradients)
 long long block_bwd_scratch_bytes(long long N, long long C, long long H, long long W, int dtype) {
-    const long long s = elem_size(dtype);
-    return align_up(splat_bwd_workspace(N, C, H, W, dtype, DCB_MODE_SOFT), 256) + 2 * align_up(N * C * H * W * s, 256) + 2 * align_up(N * H * W * s, 256);
+    DcbTensor t = {};
+    t.dtype = dtype; t.size[0] = N; t.size[1] = C; t.size[2] = H; t.size[3] = W;
+    DcbPyramidBwdLevel lv = {};
+    lv.first = &t;
+    return pyramid_bwd_workspace(&lv, 1);
 }
 
 int bidir_block_fwd_impl(const DcbTensor* first, const DcbTensor* last, const DcbTensor* flow_f, const DcbTensor* flow_b,
@@ -125,19 +126,7 @@ int bidir_block_fwd_impl(const DcbTensor* first, const DcbTensor* last, const Dc
     return bidir_fuse_fwd_impl(wf, wb, metric_f, metric_b, of, ob, fused, st);
 }
 
-template <class T> __global__ void __launch_bounds__(256) k_add_inplace(T* dst, const T* src, long long n) {
-    const long long i = (long long)blockIdx.x * 256 + threadIdx.x;
-    if (i < n) st<T, float>(dst + i, add_rn(ld<float>(dst + i), ld<float>(src + i)));
-}
-
-static int add_inplace(int dt, void* dst, const void* src, long long n, cudaStream_t st) {
-    const unsigned blocks = (unsigned)((n + 255) / 256);
-    if (dt == DCB_F32) k_add_inplace<float><<<blocks, 256, 0, st>>>((float*)dst, (const float*)src, n);
-    else k_add_inplace<__nv_bfloat16><<<blocks, 256, 0, st>>>((__nv_bfloat16*)dst, (const __nv_bfloat16*)src, n);
-    DCB_CHECK_LAUNCH("k_add_inplace");
-    return DCB_OK;
-}
-
+// the one-level pyramid backward (pyramid_bwd.cu): two launches whatever the size, with the double-hole fill of the forward
 int bidir_block_bwd_impl(const DcbTensor* g, const DcbTensor* first, const DcbTensor* last, const DcbTensor* flow_f,
                          const DcbTensor* flow_b, const DcbTensor* metric_f, const DcbTensor* metric_b, const DcbTensor* warped_f,
                          const DcbTensor* warped_b, const DcbTensor* norm_f, const DcbTensor* norm_b, const DcbTensor* occ_f,
@@ -145,32 +134,16 @@ int bidir_block_bwd_impl(const DcbTensor* g, const DcbTensor* first, const DcbTe
                          const DcbTensor* g_metric_b, void* ws, long long ws_bytes, cudaStream_t st) {
     const long long N = first->size[0], C = first->size[1], H = first->size[2], W = first->size[3];
     if (N * C * H * W == 0) return DCB_OK;
-    const int dt = first->dtype;
-    const long long s = elem_size(dt), big = align_up(N * C * H * W * s, 256), plane = align_up(N * H * W * s, 256);
-    const long long bwd = align_up(splat_bwd_workspace(N, C, H, W, dt, DCB_MODE_SOFT), 256);
-    const long long need = bwd + 2 * big + 2 * plane;
+    const long long need = block_bwd_scratch_bytes(N, C, H, W, first->dtype);
     if (!ws || ws_bytes < need || ((uintptr_t)ws & 255))
         return set_error(DCB_E_WORKSPACE, "bidir_block_bwd: scratch of %lld bytes (256 B aligned) required, got %lld", need, ws_bytes);
-    char* sc = (char*)ws;
-    const DcbTensor gA = contiguous_like(first, C, dt, sc + bwd), gB = contiguous_like(first, C, dt, sc + bwd + big);
-    const DcbTensor gca = contiguous_like(first, 1, dt, sc + bwd + 2 * big), gcb = contiguous_like(first, 1, dt, sc + bwd + 2 * big + plane);
-    const bool wf = g_first || g_metric_f, wb = g_last || g_metric_b;
-    // fusion backward: gradients w.r.t. both warped maps and, when the metric is learned, both confidences
-    int rc = bidir_fuse_bwd_impl(g, warped_f, warped_b, metric_f, metric_b, occ_f, occ_b, wf ? &gA : nullptr, wb ? &gB : nullptr,
-                                 g_metric_f ? &gca : nullptr, g_metric_b ? &gcb : nullptr, st);
-    if (rc != DCB_OK) return rc;
-    // splat backward of each direction (flows carry no gradient in the extractors: extractors.py:286-287 are no_grad inputs)
-    if (wf) {
-        rc = splat_bwd_impl(&gA, first, flow_f, metric_f, warped_f, norm_f, occ_f, g_first, nullptr, g_metric_f, sc, bwd, DCB_MODE_SOFT, DCB_EPS_ADD, st);
-        if (rc != DCB_OK) return rc;
-        if (g_metric_f) { rc = add_inplace(dt, g_metric_f->ptr, gca.ptr, N * H * W, st); if (rc != DCB_OK) return rc; }
-    }
-    if (wb) {
-        rc = splat_bwd_impl(&gB, last, flow_b, metric_b, warped_b, norm_b, occ_b, g_last, nullptr, g_metric_b, sc, bwd, DCB_MODE_SOFT, DCB_EPS_ADD, st);
-        if (rc != DCB_OK) return rc;
-        if (g_metric_b) { rc = add_inplace(dt, g_metric_b->ptr, gcb.ptr, N * H * W, st); if (rc != DCB_OK) return rc; }
-    }
-    return DCB_OK;
+    auto ptr = [](const DcbTensor* t) -> void* { return t ? t->ptr : nullptr; };
+    DcbPyramidBwdLevel lv = {};
+    lv.grad_fused = g; lv.first = first; lv.last = last; lv.flow_f = flow_f; lv.flow_b = flow_b; lv.metric_f = metric_f; lv.metric_b = metric_b;
+    lv.warped_f = warped_f->ptr; lv.warped_b = warped_b->ptr; lv.norm_f = norm_f->ptr; lv.norm_b = norm_b->ptr;
+    lv.occ_f = occ_f->ptr; lv.occ_b = occ_b->ptr;
+    lv.grad_first = ptr(g_first); lv.grad_last = ptr(g_last); lv.grad_metric_f = ptr(g_metric_f); lv.grad_metric_b = ptr(g_metric_b);
+    return bidir_pyramid_bwd_impl(&lv, 1, ws, true, st);
 }
 
 }  // namespace dcb

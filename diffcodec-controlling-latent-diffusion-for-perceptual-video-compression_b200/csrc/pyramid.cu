@@ -178,6 +178,7 @@ struct PyrFuseArgs {
     PyrLevel lv[kMaxLevels];
     int n_levels;
     int masks;               // 0: identity masks (notebook cell 5): no occlusion test, no (1 - mask), no holes
+    int holes;               // 0: no double-hole fill (DCB_PYRAMID_NO_HOLES; extractors.py:193-199)
 };
 
 template <class T>
@@ -224,7 +225,7 @@ __global__ void __launch_bounds__(32, 16) k_pyr_fuse(const __grid_constant__ Pyr
         ca = fmaxf(ca, 0.f); cb = fmaxf(cb, 0.f);
         const float s = add_rn(add_rn(ca, cb), 0.000001f);
         w0[i] = ca / s; w1[i] = cb / s;
-        hole[i] = a.masks && add_rn(of, ob) > 1.5f;                                                         // extractors.py:306
+        hole[i] = a.masks && a.holes && add_rn(of, ob) > 1.5f;                                                        // extractors.py:306
         if (cgi == 0) {
             if (L.occ_f) st<T, float>((T*)L.occ_f + fpix + r, of);
             if (L.occ_b) st<T, float>((T*)L.occ_b + fpix + r, ob);
@@ -311,6 +312,7 @@ int bidir_pyramid_fwd_impl(const DcbPyramidLevel* lv, int n, void* ws, int flags
     PyrScatterArgs sa; PyrFuseArgs fa;
     sa.n_jobs = 0; fa.n_levels = 0;
     fa.masks = (flags & DCB_PYRAMID_NO_MASKS) ? 0 : 1;
+    fa.holes = (flags & DCB_PYRAMID_NO_HOLES) ? 0 : 1;
     long long shared_total = 0;
     for (int l = 0; l < n; ++l) shared_total += level_shared_bytes(lv[l].first->size[0], lv[l].first->size[2], lv[l].first->size[3]);
     const long long total = pyramid_workspace(lv, n);

@@ -95,8 +95,9 @@ _lib._option_hooks.append(_block_ws.clear)
 
 class _bidir_block_func(torch.autograd.Function):
     """The whole block -- both occlusion masks, both masked soft splats, confidence fusion, double-hole fill -- as ONE
-    autograd node and ONE library call each way (dcb_bidir_block_fwd / _bwd), with the learned metric of the live
-    consumer (gradients reach the features and, through the splat weights AND the fusion weights, the metric)."""
+    autograd node and ONE library call each way (dcb_bidir_block_fwd / the one-level dcb_bidir_pyramid_bwd), with the
+    learned metric of the live consumer (gradients reach the features, the flows and, through the splat weights AND the
+    fusion weights, the metric)."""
 
     @staticmethod
     @torch.amp.custom_fwd(device_type="cuda", cast_inputs=torch.float32)       # the splats run in fp32 (control_utils.py:61)
@@ -104,7 +105,7 @@ class _bidir_block_func(torch.autograd.Function):
         lib = _lib.lib()
         n, c, h, w = first.shape
         dev, dt = first.device, first.dtype
-        need = any(ctx.needs_input_grad[i] for i in (0, 1, 4, 5))
+        need = any(ctx.needs_input_grad[:6])
         fused = torch.empty((n, c, h, w), dtype=dt, device=dev)
         saved = None
         if need:
@@ -133,23 +134,8 @@ class _bidir_block_func(torch.autograd.Function):
     @staticmethod
     @torch.amp.custom_bwd(device_type="cuda")
     def backward(ctx, g):
-        first, last, flow_f, flow_b, metric_f, metric_b, wf, wb, nf, nb, of, ob = ctx.saved_tensors
-        lib = _lib.lib()
-        n, c, h, w = first.shape
-        dev, dt = first.device, first.dtype
-        need = ctx.needs_input_grad
-        g = g.to(dt)
-        g1 = torch.empty_like(first, memory_format=torch.contiguous_format) if need[0] else None
-        g2 = torch.empty_like(last, memory_format=torch.contiguous_format) if need[1] else None
-        gm1 = torch.empty((n, 1, h, w), dtype=dt, device=dev) if need[4] else None
-        gm2 = torch.empty((n, 1, h, w), dtype=dt, device=dev) if need[5] else None
-        ws = _lib.workspace(dev, _block_sizes(n, c, h, w, _lib._DTYPES[dt])[2], "scratch")
-        D = _lib.desc
-        with _lib.on_device(dev):
-            rc = lib.dcb_bidir_block_bwd(D(g), D(first), D(last), D(flow_f), D(flow_b), D(metric_f), D(metric_b), D(wf), D(wb), D(nf), D(nb),
-                                         D(of), D(ob), D(g1), D(g2), D(gm1), D(gm2), ws.data_ptr(), ws.numel(), _lib.stream_ptr(dev))
-        _lib.check(rc, "dcb_bidir_block_bwd")
-        return g1, g2, None, None, gm1, gm2, None
+        t = ctx.saved_tensors
+        return tuple(_pyramid_backward([t[:6]], [t[6:]], [g], [ctx.needs_input_grad[:6]], 0)[0]) + (None,)
 
 
 def _block_forward_nograd(first, last, flow_f, flow_b, metric_f, metric_b):
@@ -175,14 +161,14 @@ def _block_forward_nograd(first, last, flow_f, flow_b, metric_f, metric_b):
 def bidirectional_block(first_features, last_features, flow_f, flow_b, metric_f=None, metric_b=None):
     """masks + both masked soft splats + confidence fusion + double-hole fill of ONE pyramid scale
     (``extractors.py:289-310``), given the two metric maps (``metric_net`` outputs, or None for a warper without one).
-    One library call forward, one backward; no host sync. Flows must not require a gradient (they do not in
-    ``Bi_Dir_FeatureExtractor``); otherwise use ``bidirectional_warp_fuse``."""
+    One library call forward, one backward (two launches); no host sync. Gradients reach the features, the flows and the
+    metrics; the occlusion masks carry none (``compute_mask`` thresholds, as in the reference)."""
     dt = first_features.dtype
     if metric_f is None:
         metric_f = torch.ones_like(flow_f[:, :1], dtype=dt)
     if metric_b is None:
         metric_b = torch.ones_like(flow_b[:, :1], dtype=dt)
-    needs_grad = torch.is_grad_enabled() and (first_features.requires_grad or last_features.requires_grad or metric_f.requires_grad or metric_b.requires_grad)
+    needs_grad = torch.is_grad_enabled() and any(t.requires_grad for t in (first_features, last_features, flow_f, flow_b, metric_f, metric_b))
     if (not needs_grad and not torch.is_autocast_enabled("cuda") and dt in (torch.float32, torch.bfloat16)
             and last_features.dtype == dt and flow_f.dtype == dt and flow_b.dtype == dt and metric_f.dtype == dt and metric_b.dtype == dt):
         return _block_forward_nograd(first_features, last_features, flow_f, flow_b, metric_f, metric_b)
@@ -251,16 +237,44 @@ def _pyramid_forward(levels, flags, want_saved, want_warped=False):
     return fused, saved
 
 
+def _pyramid_backward(levels, saved, grads, needs, flags):
+    """ONE dcb_bidir_pyramid_bwd call (two kernel launches) for every scale that wants a gradient. levels: per scale (first,
+    last, flow_f, flow_b, metric_f | None, metric_b | None); saved: per scale the six forward outputs; grads: grad_fused per
+    scale; needs: per scale six flags in the order of `levels`. Returns per scale the six gradients (None where not wanted)."""
+    res, ins, svs, outs = [], [], [], []
+    for lv, sv, g, need in zip(levels, saved, grads, needs):
+        if g is None or not any(need):
+            res.append((None,) * 6)
+            continue
+        first = lv[0]
+        n, c, h, w = first.shape
+        gr = tuple(torch.empty((n, ch, h, w), dtype=first.dtype, device=first.device) if want else None
+                   for ch, want in zip((c, c, 2, 2, 1, 1), need))
+        ins.append((g.to(first.dtype),) + tuple(lv)); svs.append(sv); outs.append(gr); res.append(gr)
+    if not ins:
+        return res
+    lib = _lib.lib()
+    dev = ins[0][1].device
+    stream = _lib.stream_ptr(dev)
+    with _lib.on_device(dev):
+        arr = _lib.pack_pyramid_bwd(ins, svs, outs)
+        ws = _lib.workspace(dev, int(lib.dcb_bidir_pyramid_bwd_workspace_bytes(arr, len(ins))), "scratch", stream)
+        rc = lib.dcb_bidir_pyramid_bwd(arr, len(ins), ws.data_ptr(), ws.numel(), flags, stream)
+    _lib.check(rc, "dcb_bidir_pyramid_bwd")
+    return res
+
+
 class _bidir_pyramid_func(torch.autograd.Function):
-    """All scales of a bi-directional conditioning pyramid as ONE autograd node: one library call forward (two launches),
-    one dcb_bidir_block_bwd call per scale backward. Inputs per scale: first, last, flow_f, flow_b, metric_f, metric_b."""
+    """All scales of a bi-directional conditioning pyramid as ONE autograd node: one library call forward, one backward (two
+    launches each). Inputs: the holes flag, then per scale first, last, flow_f, flow_b, metric_f | None, metric_b | None."""
 
     @staticmethod
     @torch.amp.custom_fwd(device_type="cuda", cast_inputs=torch.float32)       # the splats run in fp32 (control_utils.py:61)
-    def forward(ctx, *tensors):
+    def forward(ctx, holes, *tensors):
         levels = [tuple(tensors[i:i + 6]) for i in range(0, len(tensors), 6)]
-        need = any(ctx.needs_input_grad[6 * l + k] for l in range(len(levels)) for k in (0, 1, 4, 5))
-        fused, saved = _pyramid_forward(levels, 0, need)
+        need = any(ctx.needs_input_grad[1:])
+        ctx.flags = 0 if holes else _lib.PYRAMID_NO_HOLES
+        fused, saved = _pyramid_forward(levels, ctx.flags, need)
         ctx.n_levels = len(levels)
         if need:
             flat = []
@@ -272,57 +286,37 @@ class _bidir_pyramid_func(torch.autograd.Function):
     @staticmethod
     @torch.amp.custom_bwd(device_type="cuda")
     def backward(ctx, *grads):
-        lib = _lib.lib()
-        t = ctx.saved_tensors
-        res = []
-        D = _lib.desc
-        for l in range(ctx.n_levels):
-            first, last, flow_f, flow_b, metric_f, metric_b, wf, wb, nf, nb, of, ob = t[12 * l:12 * l + 12]
-            need = ctx.needs_input_grad[6 * l:6 * l + 6]
-            g = grads[l]
-            if g is None or not any(need[k] for k in (0, 1, 4, 5)):
-                res += [None] * 6
-                continue
-            n, c, h, w = first.shape
-            dev, dt = first.device, first.dtype
-            g = g.to(dt)
-            g1 = torch.empty_like(first, memory_format=torch.contiguous_format) if need[0] else None
-            g2 = torch.empty_like(last, memory_format=torch.contiguous_format) if need[1] else None
-            gm1 = torch.empty((n, 1, h, w), dtype=dt, device=dev) if need[4] else None
-            gm2 = torch.empty((n, 1, h, w), dtype=dt, device=dev) if need[5] else None
-            ws = _lib.workspace(dev, _block_sizes(n, c, h, w, _lib._DTYPES[dt])[2], "scratch")
-            with _lib.on_device(dev):
-                rc = lib.dcb_bidir_block_bwd(D(g), D(first), D(last), D(flow_f), D(flow_b), D(metric_f), D(metric_b), D(wf), D(wb), D(nf), D(nb),
-                                             D(of), D(ob), D(g1), D(g2), D(gm1), D(gm2), ws.data_ptr(), ws.numel(), _lib.stream_ptr(dev))
-            _lib.check(rc, "dcb_bidir_block_bwd")
-            res += [g1, g2, None, None, gm1, gm2]
-        return tuple(res)
+        t, L = ctx.saved_tensors, ctx.n_levels
+        need = ctx.needs_input_grad[1:]
+        res = _pyramid_backward([t[12 * l:12 * l + 6] for l in range(L)], [t[12 * l + 6:12 * l + 12] for l in range(L)], grads,
+                                [need[6 * l:6 * l + 6] for l in range(L)], ctx.flags)
+        return (None,) + tuple(x for r in res for x in r)
 
 
 _PYRAMID_MAX_LEVELS = 4
 
 
-def bidirectional_pyramid(levels):
+def bidirectional_pyramid(levels, holes=True):
     """Every scale of ``Bi_Dir_FeatureExtractor.forward`` between the conv stacks (``extractors.py:282-310``) in one call:
     levels = [(first, last, flow_f, flow_b, metric_f | None, metric_b | None), ...] -> [fused, ...]. Two kernel launches
-    for the whole pyramid, no host sync; gradients reach the features and the metrics (not the flows)."""
+    for the whole pyramid each way, no host sync; gradients reach the features, the flows and the metrics (the occlusion
+    masks carry none, as in the reference). ``holes=False``: the fusion without the double-hole fill, as
+    ``Bi_Dir_ResidueExtractor`` (``extractors.py:193-199``)."""
     levels = [tuple(lv) for lv in levels]
     if len(levels) > _PYRAMID_MAX_LEVELS:
-        return bidirectional_pyramid(levels[:_PYRAMID_MAX_LEVELS]) + bidirectional_pyramid(levels[_PYRAMID_MAX_LEVELS:])
+        return bidirectional_pyramid(levels[:_PYRAMID_MAX_LEVELS], holes) + bidirectional_pyramid(levels[_PYRAMID_MAX_LEVELS:], holes)
     dt = levels[0][0].dtype
     grad = torch.is_grad_enabled() and any(t is not None and t.requires_grad for lv in levels for t in lv)
     plain = (not grad and not torch.is_autocast_enabled("cuda") and dt in (torch.float32, torch.bfloat16)
              and all(t is None or t.dtype == dt for lv in levels for t in lv))
     if plain:
-        return _pyramid_forward(levels, 0, False)[0]
+        return _pyramid_forward(levels, 0 if holes else _lib.PYRAMID_NO_HOLES, False)[0]
     flat = []
     for first, last, ff, fb, mf, mb in levels:
         d = first.dtype
-        cast = lambda t: t if t.dtype == d else t.to(d)
-        mf = torch.ones_like(ff[:, :1], dtype=d) if mf is None else mf          # the backward entry wants the metric tensors
-        mb = torch.ones_like(fb[:, :1], dtype=d) if mb is None else mb
+        cast = lambda t: t if t is None or t.dtype == d else t.to(d)
         flat += [first, cast(last), cast(ff), cast(fb), cast(mf), cast(mb)]
-    return list(_bidir_pyramid_func.apply(*flat))
+    return list(_bidir_pyramid_func.apply(holes, *flat))
 
 
 def pyramid_conditioning(img1, img2, flow1, flow2, sizes=(128, 64, 32)):
@@ -350,8 +344,7 @@ def pyramid_conditioning(img1, img2, flow1, flow2, sizes=(128, 64, 32)):
 
 def _block_fusable(first, last, flow_f, flow_b):
     from .softsplat import is_deterministic
-    return (first.is_cuda and first.shape == last.shape and first.dtype in (torch.float32, torch.bfloat16, torch.float16)
-            and not (torch.is_grad_enabled() and (flow_f.requires_grad or flow_b.requires_grad)) and not is_deterministic())
+    return first.is_cuda and first.shape == last.shape and first.dtype in (torch.float32, torch.bfloat16, torch.float16) and not is_deterministic()
 
 
 def bidirectional_warp_fuse(first_features, last_features, flow_f, flow_b, warper):
@@ -410,8 +403,9 @@ class WarpExtractor(nn.Module):                               # extractors.py:26
 
 
 class Bi_Dir_FeatureExtractor(nn.Module):
-    """``controlnet/extractors.py:209-316``. Per scale, everything between the stride-2 convs and the zero conv is ONE
-    fused call (``bidirectional_block``): no ``holes.any()`` host sync, ~9 launches instead of ~45."""
+    """``controlnet/extractors.py:209-316``. Everything between the stride-2 convs and the zero convs of all four scales is
+    ONE fused call each way (``bidirectional_pyramid``, two launches forward and two backward): no ``holes.any()`` host
+    sync. Flows that carry a gradient receive it through the same call."""
 
     def __init__(self, inject_channels):
         super().__init__()
@@ -432,9 +426,8 @@ class Bi_Dir_FeatureExtractor(nn.Module):
         flow_fwd, flow_bwd = flow[:, :2], flow[:, 2:]
         flow_res = (64, 32, 16, 8)                                               # extractors.py:278
         from .softsplat import is_deterministic
-        whole = (first_features.is_cuda and flow.dtype in (torch.float32, torch.bfloat16)
-                 and not (torch.is_grad_enabled() and flow.requires_grad) and not is_deterministic())
-        if not whole:                                                            # flows that carry a gradient: scale by scale
+        whole = first_features.is_cuda and flow.dtype in (torch.float32, torch.bfloat16) and not is_deterministic()
+        if not whole:                                                            # what the pyramid does not take: scale by scale
             outs = []
             for idx, res in enumerate(flow_res):
                 first_features = self.extractors_first[idx](first_features)
@@ -452,13 +445,16 @@ class Bi_Dir_FeatureExtractor(nn.Module):
             first_features = self.extractors_first[idx](first_features)
             last_features = self.extractors_last[idx](last_features)
             feats.append((first_features, last_features))
-        with torch.no_grad():
-            jobs = []
-            for (f, _), res in zip(feats, flow_res):
-                dt = torch.float32 if (torch.is_autocast_enabled("cuda") or f.dtype not in (torch.float32, torch.bfloat16)) else f.dtype
-                for fl in (flow_fwd, flow_bwd):
-                    jobs.append((fl, (res, res), False, _lib.RESAMPLE_DIV, (res - 1) / 2.0, (res - 1) / 2.0, dt))
-            flows = resample_batch(jobs)
+        if torch.is_grad_enabled() and flow.requires_grad:                      # differentiable resizes (dcb_resample_batch has no backward)
+            flows = [resize_and_normalize_flow_batched(fl, res, res) for res in flow_res for fl in (flow_fwd, flow_bwd)]
+        else:
+            with torch.no_grad():
+                jobs = []
+                for (f, _), res in zip(feats, flow_res):
+                    dt = torch.float32 if (torch.is_autocast_enabled("cuda") or f.dtype not in (torch.float32, torch.bfloat16)) else f.dtype
+                    for fl in (flow_fwd, flow_bwd):
+                        jobs.append((fl, (res, res), False, _lib.RESAMPLE_DIV, (res - 1) / 2.0, (res - 1) / 2.0, dt))
+                flows = resample_batch(jobs)
         levels = []
         for idx, (f, l) in enumerate(feats):
             learn = getattr(self.wrapper[idx], "with_learnable_metric", False)
@@ -471,8 +467,9 @@ class Bi_Dir_FeatureExtractor(nn.Module):
 
 
 class Bi_Dir_ResidueExtractor(nn.Module):
-    """``controlnet/extractors.py:67-205``. The flows pass through learned refiners here, so they carry a gradient and
-    the block runs as masks + two differentiable splats + the fusion kernel (no hole branch in this class, :193-199)."""
+    """``controlnet/extractors.py:67-205``. The flows pass through learned refiners here and carry a gradient; the motion
+    compensation of all four scales (masks, both splats, fusion without the hole branch, :193-199) is ONE
+    ``bidirectional_pyramid(..., holes=False)`` call each way, whose backward reaches the refiners through the flows."""
 
     def __init__(self, inject_channels):
         super().__init__()
@@ -499,13 +496,24 @@ class Bi_Dir_ResidueExtractor(nn.Module):
         for enc_prev, enc_next in zip(self.prev_pyramids, self.next_pyramids):
             x_prev, x_next = enc_prev(x_prev), enc_next(x_next)
             prev_feats.append(x_prev); next_feats.append(x_next)
-        outs = []
+        flows = []
         for i, res in enumerate(self.resolutions):
             factor = H // res                                                    # extractors.py:181-183: resize, then divide by the scale factor
             flow_f = self.flow_refiners[i](F.interpolate(flow_fwd, size=(res, res), mode="bilinear", align_corners=False) / factor)
             flow_b = self.flow_refiners[i](F.interpolate(flow_bwd, size=(res, res), mode="bilinear", align_corners=False) / factor)
-            occ_f, occ_b = compute_mask(flow_f, flow_b), compute_mask(flow_b, flow_f)
-            warped_prev, conf_prev = self.warpers[i](prev_feats[i], flow_f, mask=occ_f)
-            warped_next, conf_next = self.warpers[i](next_feats[i], flow_b, mask=occ_b)
-            outs.append(self.zero_convs[i](bidir_fuse(warped_prev, warped_next, conf_prev, conf_next)))
-        return outs
+            flows.append((flow_f, flow_b))
+        from .softsplat import is_deterministic
+        if not (prev_frame.is_cuda and flow_fwd.dtype in (torch.float32, torch.bfloat16) and not is_deterministic()):
+            outs = []                                                            # what the pyramid does not take: scale by scale
+            for i, (flow_f, flow_b) in enumerate(flows):
+                occ_f, occ_b = compute_mask(flow_f, flow_b), compute_mask(flow_b, flow_f)
+                warped_prev, conf_prev = self.warpers[i](prev_feats[i], flow_f, mask=occ_f)
+                warped_next, conf_next = self.warpers[i](next_feats[i], flow_b, mask=occ_b)
+                outs.append(self.zero_convs[i](bidir_fuse(warped_prev, warped_next, conf_prev, conf_next)))
+            return outs
+        # no refined flow or metric depends on a splat: all of them first, then the four scales in one call
+        levels = [(prev_feats[i], next_feats[i], flow_f, flow_b, self.warpers[i].metric_net(prev_feats[i]), self.warpers[i].metric_net(next_feats[i]))
+                  for i, (flow_f, flow_b) in enumerate(flows)]
+        with torch.autocast(device_type="cuda", enabled=False):
+            fused = bidirectional_pyramid(levels, holes=False)
+        return [zc(x) for zc, x in zip(self.zero_convs, fused)]

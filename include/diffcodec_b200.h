@@ -276,8 +276,8 @@ int dcb_bidir_fuse_bwd(const DcbTensor* grad_fused, const DcbTensor* A, const Dc
  *   warped_*, norm_* (F32), occ_*: optional outputs (NULL = kept in scratch / not produced); the backward needs all six
  *   ws_acc        accumulator workspace (dcb_bidir_block_workspace_bytes(.., 0)); DCB_FLAG_WS_CLEAN protocol as dcb_splat_fwd
  *   ws_scratch    plain scratch (.., 1) for the optional outputs the caller left NULL
- * Backward: gradients w.r.t. both feature maps and both metrics (splat path + fusion path summed); flows carry no
- * gradient in the extractors. ws: plain scratch (dcb_bidir_block_workspace_bytes(.., 2)).
+ * Backward: gradients w.r.t. both feature maps and both metrics (splat path + fusion path summed); it is the one-level
+ * dcb_bidir_pyramid_bwd (two launches). ws: plain scratch (dcb_bidir_block_workspace_bytes(.., 2)).
  */
 int64_t dcb_bidir_block_workspace_bytes(int64_t N, int64_t C, int64_t H, int64_t W, int32_t elem_dtype, int32_t which);
 int dcb_bidir_block_fwd(const DcbTensor* first, const DcbTensor* last, const DcbTensor* flow_f, const DcbTensor* flow_b,
@@ -303,16 +303,41 @@ int dcb_bidir_block_bwd(const DcbTensor* grad_fused, const DcbTensor* first, con
  *   levels[l].first, last [N,C,H,W]; flow_f, flow_b [N,2,H,W] at the level's resolution; metric_f, metric_b [N,1,H,W]
  *   or NULL = all-ones (never materialised); one dtype (F32 or BF16) for all tensors of all levels
  *   outputs are raw device pointers to NCHW-contiguous buffers of the level's shape and dtype (norm_*: F32):
- *   fused (required); warped_*, norm_*, occ_* optional (NULL = never stored; dcb_bidir_block_bwd needs all six)
+ *   fused (required); warped_*, norm_*, occ_* optional (NULL = never stored; dcb_bidir_pyramid_bwd needs all six)
  *   n_levels <= 4;  workspace: dcb_bidir_pyramid_workspace_bytes(), DCB_FLAG_WS_CLEAN protocol as dcb_splat_fwd
+ *   flags: DCB_PYRAMID_NO_MASKS, or DCB_PYRAMID_NO_HOLES: masks and (1 - mask) as usual, the fusion without the double-hole
+ *   fill (Bi_Dir_ResidueExtractor, controlnet/extractors.py:193-199); NO_MASKS | NO_HOLES equals NO_MASKS
  */
 typedef struct DcbPyramidLevel {
     const DcbTensor *first, *last, *flow_f, *flow_b, *metric_f, *metric_b;
     void *fused, *warped_f, *warped_b, *norm_f, *norm_b, *occ_f, *occ_b;
 } DcbPyramidLevel;
-enum { DCB_PYRAMID_NO_MASKS = 4 /* flag of dcb_bidir_pyramid_fwd */ };
+enum { DCB_PYRAMID_NO_MASKS = 4, DCB_PYRAMID_NO_HOLES = 8 /* flags of dcb_bidir_pyramid_fwd (NO_HOLES: also of _bwd) */ };
 int64_t dcb_bidir_pyramid_workspace_bytes(const DcbPyramidLevel* levels, int32_t n_levels);
 int dcb_bidir_pyramid_fwd(const DcbPyramidLevel* levels, int32_t n_levels, void* workspace, int64_t workspace_bytes,
+                          int32_t flags, void* stream);
+
+/*
+ * Backward of dcb_bidir_pyramid_fwd (with masks; with or without holes) for ALL levels in ONE call and TWO kernel launches
+ * (every target pixel of every level; then one source-side gather per level and direction). Gradients w.r.t. both feature
+ * maps, both flows (the splat weights' dependence on the flow, as dcb_splat_bwd) and both metrics (splat weights + fusion
+ * confidences). The occlusion masks carry no gradient (compute_mask thresholds). No atomics: bit-identical run to run.
+ *
+ *   grad_fused [N,C,H,W] any strides; first, last, flow_f, flow_b, metric_f, metric_b as given to the forward (a NULL metric
+ *   is the all-ones metric); one dtype (F32 or BF16) for all tensors of all levels
+ *   warped_*, norm_* (F32), occ_*: what the forward stored for the level (raw pointers, NCHW-contiguous), all six required
+ *   grad_*: raw pointers to NCHW-contiguous buffers of the level's dtype, or NULL (not computed); fully overwritten.
+ *   grad_metric_* must be NULL where the metric is NULL.
+ *   1 <= n_levels <= 4;  flags: 0 or DCB_PYRAMID_NO_HOLES (as passed to the forward); workspace: plain scratch of
+ *   dcb_bidir_pyramid_bwd_workspace_bytes() bytes (24 per pixel and level), 256-byte aligned
+ */
+typedef struct DcbPyramidBwdLevel {
+    const DcbTensor *grad_fused, *first, *last, *flow_f, *flow_b, *metric_f, *metric_b;
+    const void *warped_f, *warped_b, *norm_f, *norm_b, *occ_f, *occ_b;
+    void *grad_first, *grad_last, *grad_flow_f, *grad_flow_b, *grad_metric_f, *grad_metric_b;
+} DcbPyramidBwdLevel;
+int64_t dcb_bidir_pyramid_bwd_workspace_bytes(const DcbPyramidBwdLevel* levels, int32_t n_levels);
+int dcb_bidir_pyramid_bwd(const DcbPyramidBwdLevel* levels, int32_t n_levels, void* workspace, int64_t workspace_bytes,
                           int32_t flags, void* stream);
 
 /*
