@@ -18,7 +18,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("DCB_LIB_PATH") or os.path.join(_HERE, "libdiffcodec_b200.so")   # override: A/B builds only
 
 DCB_F32, DCB_BF16, DCB_F64 = 0, 1, 2
-DCB_U8, DCB_F16 = 3, 4          # storage types of dcb_convert only
+DCB_U8, DCB_F16 = 3, 4          # U8: a storage type of dcb_convert only; F16: a tensor dtype wherever BF16 is one
 MODE_SUM, MODE_AVG, MODE_LINEAR, MODE_SOFT = 0, 1, 2, 3
 EPS_ADD, EPS_ZERO, EPS_CLIP = 0, 1, 2
 FLAG_DETERMINISTIC, FLAG_WS_CLEAN = 1, 2
@@ -29,7 +29,7 @@ RESAMPLE_NONE, RESAMPLE_MUL, RESAMPLE_DIV = 0, 1, 2
 
 E_NULL, E_SHAPE, E_DTYPE, E_MODE, E_WORKSPACE, E_LIMIT, E_ALIGN = -1, -2, -3, -4, -5, -6, -7
 
-_DTYPES = {torch.float32: DCB_F32, torch.bfloat16: DCB_BF16, torch.float64: DCB_F64}
+_DTYPES = {torch.float32: DCB_F32, torch.bfloat16: DCB_BF16, torch.float16: DCB_F16, torch.float64: DCB_F64}
 
 
 class DcbTensor(ctypes.Structure):
@@ -184,7 +184,7 @@ def desc(t: torch.Tensor | None):
     if t.dim() != 4:
         raise AssertionError(f"expected a 4-d NCHW tensor, got {tuple(t.shape)}")
     if t.dtype not in _DTYPES:
-        raise ValueError(f"unsupported dtype {t.dtype}: float32, bfloat16 and float64 are implemented")
+        raise ValueError(f"unsupported dtype {t.dtype}: float32, bfloat16, float16 and float64 are implemented")
     return _pack_desc(t.data_ptr(), _DTYPES[t.dtype], 0, *t.shape, *t.stride())
 
 
@@ -214,7 +214,7 @@ def _tensor_fields(t: torch.Tensor):
     if t.dim() != 4:
         raise AssertionError(f"expected a 4-d NCHW tensor, got {tuple(t.shape)}")
     if t.dtype not in _DTYPES:
-        raise ValueError(f"unsupported dtype {t.dtype}: float32, bfloat16 and float64 are implemented")
+        raise ValueError(f"unsupported dtype {t.dtype}: float32, bfloat16, float16 and float64 are implemented")
     return (t.data_ptr(), _DTYPES[t.dtype], 0, *t.shape, *t.stride())
 
 

@@ -2,6 +2,7 @@
 // error reporting, launch accounting. No allocation, no synchronisation, no stream creation.
 #include "dcb_common.cuh"
 
+#include <initializer_list>
 #include <string.h>
 
 namespace dcb {
@@ -96,7 +97,7 @@ int tile_merge_impl(const DcbTensor*, const long long*, int, const DcbTensor*, l
 // ---------------------------------------------------------------------------------------------
 static int check_tensor(const char* fn, const char* name, const DcbTensor* t, bool required) {
     if (!t) return required ? set_error(DCB_E_NULL, "%s: %s is required", fn, name) : DCB_OK;
-    if (t->dtype != DCB_F32 && t->dtype != DCB_BF16 && t->dtype != DCB_F64)
+    if (t->dtype != DCB_F32 && t->dtype != DCB_BF16 && t->dtype != DCB_F16 && t->dtype != DCB_F64)
         return set_error(DCB_E_DTYPE, "%s: %s has unsupported dtype %d", fn, name, t->dtype);
     long long numel = 1;
     for (int d = 0; d < 4; ++d) {
@@ -136,8 +137,15 @@ static int check_limits(const char* fn, const DcbTensor* t) {
 
 static int flow_dtype_ok(const char* fn, const DcbTensor* in, const DcbTensor* flow) {
     if (flow->dtype == in->dtype) return DCB_OK;
-    if (in->dtype == DCB_BF16 && flow->dtype == DCB_F32) return DCB_OK;
+    if (is_half_storage(in->dtype) && flow->dtype == DCB_F32) return DCB_OK;
     return set_error(DCB_E_DTYPE, "%s: flow dtype %d does not go with tensor dtype %d", fn, flow->dtype, in->dtype);
+}
+
+// the entries without fp16 kernels (backwarp, occlusion mask, conditioning recipes, flow resize) refuse F16 before any launch
+static int refuse_f16(const char* fn, std::initializer_list<const DcbTensor*> ts) {
+    for (const DcbTensor* t : ts)
+        if (t && t->dtype == DCB_F16) return set_error(DCB_E_DTYPE, "%s: F16 is not supported by this entry", fn);
+    return DCB_OK;
 }
 
 #define TRY(expr)                  \
@@ -289,6 +297,7 @@ int dcb_splat_bwd(const DcbTensor* gout, const DcbTensor* in, const DcbTensor* f
 int dcb_backwarp_fwd(const DcbTensor* image, const DcbTensor* flow, const DcbTensor* gt, const DcbTensor* warped,
                      const DcbTensor* residual, int32_t align_corners, void* stream) {
     const char* fn = "dcb_backwarp_fwd";
+    TRY(refuse_f16(fn, {image, flow, gt, warped, residual}));
     TRY(check_tensor(fn, "image", image, true));
     TRY(check_tensor(fn, "flow", flow, true));
     TRY(check_tensor(fn, "gt", gt, false));
@@ -315,6 +324,7 @@ int64_t dcb_backwarp_bwd_workspace_bytes(int64_t N, int64_t C, int64_t H, int64_
 int dcb_backwarp_bwd(const DcbTensor* gout, const DcbTensor* image, const DcbTensor* flow, const DcbTensor* gimage,
                      const DcbTensor* gflow, int32_t align_corners, void* ws, int64_t ws_bytes, void* stream) {
     const char* fn = "dcb_backwarp_bwd";
+    TRY(refuse_f16(fn, {gout, image, flow, gimage, gflow}));
     TRY(check_tensor(fn, "grad_warped", gout, true));
     TRY(check_tensor(fn, "image", image, true));
     TRY(check_tensor(fn, "flow", flow, true));
@@ -338,6 +348,7 @@ int64_t dcb_occlusion_mask_workspace_bytes(int64_t N, int64_t H, int64_t W) { re
 int dcb_occlusion_mask(const DcbTensor* flow_a, const DcbTensor* flow_b, const DcbTensor* mask, void* ws, int64_t ws_bytes,
                        int32_t flags, void* stream) {
     const char* fn = "dcb_occlusion_mask";
+    TRY(refuse_f16(fn, {flow_a, flow_b, mask}));
     TRY(check_tensor(fn, "flow_a", flow_a, true));
     TRY(check_tensor(fn, "flow_b", flow_b, true));
     TRY(check_tensor(fn, "mask", mask, true));
@@ -360,6 +371,7 @@ int dcb_residual_fused(const DcbTensor* image1, const DcbTensor* flow1, const Dc
                        const DcbTensor* occ_bwd, void* ws, int64_t ws_bytes, int32_t variant, int32_t flags,
                        void* stream) {
     const char* fn = "dcb_residual_fused";
+    TRY(refuse_f16(fn, {image1, flow1, flow2, gt, fused, residual, occ_fwd, occ_bwd}));
     TRY(check_tensor(fn, "image1", image1, true));
     TRY(check_tensor(fn, "flow1", flow1, true));
     TRY(check_tensor(fn, "flow2", flow2, true));
@@ -393,6 +405,7 @@ int dcb_residual_bidir(const DcbTensor* image1, const DcbTensor* image2, const D
                        const DcbTensor* gt, const DcbTensor* fused, const DcbTensor* residual, const DcbTensor* occ_fwd,
                        const DcbTensor* occ_bwd, void* ws, int64_t ws_bytes, int32_t flags, void* stream) {
     const char* fn = "dcb_residual_bidir";
+    TRY(refuse_f16(fn, {image1, image2, flow1, flow2, gt, fused, residual, occ_fwd, occ_bwd}));
     TRY(check_tensor(fn, "image1", image1, true));
     TRY(check_tensor(fn, "image2", image2, true));
     TRY(check_tensor(fn, "flow1", flow1, true));
@@ -485,7 +498,7 @@ int dcb_tile_merge(const DcbTensor* tiles, const int64_t* pixel_coords, int32_t 
                    int64_t W_px, double eps, void* ws, int64_t ws_bytes, void* stream) {
     const char* fn = "dcb_tile_merge";
     TRY(check_tensor(fn, "out", out, true));
-    if (out->dtype != DCB_F32 && out->dtype != DCB_BF16) return set_error(DCB_E_DTYPE, "%s: F32 or BF16 only, got %d", fn, out->dtype);
+    if (out->dtype != DCB_F32 && !is_half_storage(out->dtype)) return set_error(DCB_E_DTYPE, "%s: F32, BF16 or F16 only, got %d", fn, out->dtype);
     TRY(check_out(fn, "out", out, out->dtype, elem_size(out->dtype)));
     TRY(check_limits(fn, out));
     if (n_tiles < 0) return set_error(DCB_E_SHAPE, "%s: n_tiles = %d", fn, n_tiles);
@@ -521,7 +534,7 @@ static int check_block_common(const char* fn, const DcbTensor* first, const DcbT
     TRY(check_shape(fn, "metric_f", metric_f, N, 1, H, W));
     TRY(check_shape(fn, "metric_b", metric_b, N, 1, H, W));
     const int dt = first->dtype;
-    if (dt != DCB_F32 && dt != DCB_BF16) return set_error(DCB_E_DTYPE, "%s: F32 or BF16 only, got %d", fn, dt);
+    if (dt != DCB_F32 && !is_half_storage(dt)) return set_error(DCB_E_DTYPE, "%s: F32, BF16 or F16 only, got %d", fn, dt);
     if (last->dtype != dt || flow_f->dtype != dt || flow_b->dtype != dt || metric_f->dtype != dt || metric_b->dtype != dt)
         return set_error(DCB_E_DTYPE, "%s: all tensors must share one dtype", fn);
     return DCB_OK;
@@ -606,7 +619,7 @@ static int check_pyramid_inputs(const char* fn, const PyramidInputs& d, int l, c
     TRY(check_shape(fn, "metric_f", d.metric_f, N, 1, H, W));
     TRY(check_shape(fn, "metric_b", d.metric_b, N, 1, H, W));
     const int dt = d.first->dtype;
-    if (dt != DCB_F32 && dt != DCB_BF16) return set_error(DCB_E_DTYPE, "%s: F32 or BF16 only, got %d", fn, dt);
+    if (dt != DCB_F32 && !is_half_storage(dt)) return set_error(DCB_E_DTYPE, "%s: F32, BF16 or F16 only, got %d", fn, dt);
     if (dt != first0->dtype || d.last->dtype != dt || d.flow_f->dtype != dt || d.flow_b->dtype != dt ||
         (d.metric_f && d.metric_f->dtype != dt) || (d.metric_b && d.metric_b->dtype != dt))
         return set_error(DCB_E_DTYPE, "%s: all tensors of all levels must share one dtype", fn);
@@ -703,8 +716,8 @@ int dcb_resample_batch(const DcbResampleJob* jobs, int32_t n_jobs, void* stream)
         const DcbTensor* s = jobs[j].src; const DcbTensor* d = jobs[j].dst;
         TRY(check_tensor(fn, "src", s, true));
         TRY(check_tensor(fn, "dst", d, true));
-        if ((s->dtype != DCB_F32 && s->dtype != DCB_BF16) || (d->dtype != DCB_F32 && d->dtype != DCB_BF16))
-            return set_error(DCB_E_DTYPE, "%s: job %d: F32 or BF16 only", fn, j);
+        if ((s->dtype != DCB_F32 && !is_half_storage(s->dtype)) || (d->dtype != DCB_F32 && !is_half_storage(d->dtype)))
+            return set_error(DCB_E_DTYPE, "%s: job %d: F32, BF16 or F16 only", fn, j);
         if (s->size[0] != d->size[0] || s->size[1] != d->size[1])
             return set_error(DCB_E_SHAPE, "%s: job %d: src [N,C,H,W] -> dst [N,C,th,tw] expected", fn, j);
         if (s->size[2] * s->size[3] == 0 && d->size[0] * d->size[1] * d->size[2] * d->size[3] > 0)
@@ -719,6 +732,7 @@ int dcb_resample_batch(const DcbResampleJob* jobs, int32_t n_jobs, void* stream)
 
 int dcb_flow_resize(const DcbTensor* flow, const DcbTensor* out, int32_t convention, void* stream) {
     const char* fn = "dcb_flow_resize";
+    TRY(refuse_f16(fn, {flow, out}));
     TRY(check_tensor(fn, "flow", flow, true));
     TRY(check_tensor(fn, "out", out, true));
     if (convention < DCB_FLOW_BILINEAR_RESCALE || convention > DCB_FLOW_BILINEAR_NORMALIZE) return set_error(DCB_E_MODE, "%s: unknown convention %d", fn, convention);

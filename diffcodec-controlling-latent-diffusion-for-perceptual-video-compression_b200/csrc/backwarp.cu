@@ -356,6 +356,8 @@ int backwarp_fwd_impl(const DcbTensor* image, const DcbTensor* flow, const DcbTe
     a.warped = warped->ptr; a.residual = residual ? residual->ptr : nullptr;
     a.align = align;
     fill(a, image);
+    // no fp16 kernels here: every dispatch below reads a 16-bit tensor as bf16
+    if (image->dtype == DCB_F16 || flow->dtype == DCB_F16) return set_error(DCB_E_DTYPE, "backwarp_fwd: F16 is not supported");
     if (a.total == 0 || a.C == 0) return DCB_OK;
     if (rows_supported(image, flow, gt, warped, residual)) return launch_warp_rows(image, flow, gt, warped, residual, align, st);
     const bool ff = flow->dtype == DCB_F32;
@@ -386,6 +388,7 @@ int backwarp_bwd_impl(const DcbTensor* gout, const DcbTensor* image, const DcbTe
     a.gflow = gflow ? gflow->ptr : nullptr;
     a.align = align;
     fill(a, image);
+    if (image->dtype == DCB_F16 || flow->dtype == DCB_F16) return set_error(DCB_E_DTYPE, "backwarp_bwd: F16 is not supported");
     if (a.total == 0 || a.C == 0 || (!a.gimage && !a.gflow)) return DCB_OK;
     const long long nelem = (long long)a.total * a.C;
     void* acc = a.gimage;

@@ -39,7 +39,7 @@ static long long fused_level_bytes(long long N, long long C, long long H, long l
     return pyramid_workspace(&lv, 1);
 }
 static bool block_is_fused(long long N, long long C, long long H, long long W, int dtype) {
-    return (dtype == DCB_F32 || dtype == DCB_BF16) && fused_level_bytes(N, C, H, W, dtype) <= kFusedLevelBytes;
+    return (dtype == DCB_F32 || is_half_storage(dtype)) && fused_level_bytes(N, C, H, W, dtype) <= kFusedLevelBytes;
 }
 
 static DcbTensor contiguous_like(const DcbTensor* t, long long C, int dtype, void* ptr) {

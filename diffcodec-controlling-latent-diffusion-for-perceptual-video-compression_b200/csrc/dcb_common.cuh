@@ -3,6 +3,7 @@
 
 #include <cuda_runtime.h>
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <stdint.h>
 #include <stdio.h>
 #include <stdarg.h>
@@ -80,7 +81,10 @@ inline bool is_contig(const DcbTensor* t) {
     return true;
 }
 
-inline int elem_size(int dtype) { return dtype == DCB_F64 ? 8 : (dtype == DCB_BF16 ? 2 : 4); }
+inline int elem_size(int dtype) { return dtype == DCB_F64 ? 8 : ((dtype == DCB_BF16 || dtype == DCB_F16) ? 2 : 4); }
+// 16-bit storage (BF16 or F16): the kernels widen every load to fp32 and round once at each store, so both formats take the
+// same path, group size and workspace for a given shape
+inline bool is_half_storage(int dtype) { return dtype == DCB_BF16 || dtype == DCB_F16; }
 
 inline long long align_up(long long v, long long a) { return (v + a - 1) / a * a; }
 
@@ -101,9 +105,11 @@ template <> struct Acc<double> { using type = double; };
 
 template <class A, class T> __device__ __forceinline__ A ld(const T* p) { return (A)(*p); }
 template <> __device__ __forceinline__ float ld<float, __nv_bfloat16>(const __nv_bfloat16* p) { return __bfloat162float(*p); }
+template <> __device__ __forceinline__ float ld<float, __half>(const __half* p) { return __half2float(*p); }
 
 template <class T, class A> __device__ __forceinline__ void st(T* p, A v) { *p = (T)v; }
 template <> __device__ __forceinline__ void st<__nv_bfloat16, float>(__nv_bfloat16* p, float v) { *p = __float2bfloat16_rn(v); }
+template <> __device__ __forceinline__ void st<__half, float>(__half* p, float v) { *p = __float2half_rn(v); }
 
 // streaming variants (ld.global.cs / st.global.cs: evict-first in L1 and L2) for data touched once:
 // they keep the inputs / outputs from pushing the fp32 accumulators out of L2
@@ -113,16 +119,23 @@ __device__ __forceinline__ void st_stream(double* p, double v) { __stcs(p, v); }
 // the value a store of `v` into a T would leave behind
 template <class T> __device__ __forceinline__ float round_as(float v) { return v; }
 template <> __device__ __forceinline__ float round_as<__nv_bfloat16>(float v) { return __bfloat162float(__float2bfloat16_rn(v)); }
+template <> __device__ __forceinline__ float round_as<__half>(float v) { return __half2float(__float2half_rn(v)); }
 template <class T> __device__ __forceinline__ double round_as(double v) { return v; }
 __device__ __forceinline__ float ld_stream(const __nv_bfloat16* p) { return __bfloat162float(__ldcs(p)); }
 __device__ __forceinline__ void st_stream(float* p, float v) { __stcs(p, v); }
 __device__ __forceinline__ void st_stream(__nv_bfloat16* p, float v) { __stcs(p, __float2bfloat16_rn(v)); }
+__device__ __forceinline__ float ld_stream(const __half* p) { return __half2float(__ldcs(p)); }
+__device__ __forceinline__ void st_stream(__half* p, float v) { __stcs(p, __float2half_rn(v)); }
 
 // two neighbouring elements with one load (the address is aligned to the pair)
 __device__ __forceinline__ float2 ld2_stream(const float* p) { return __ldcs((const float2*)p); }
 __device__ __forceinline__ float2 ld2_stream(const __nv_bfloat16* p) {
     const unsigned u = __ldcs((const unsigned*)p);
     return __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&u));
+}
+__device__ __forceinline__ float2 ld2_stream(const __half* p) {
+    const unsigned u = __ldcs((const unsigned*)p);
+    return __half22float2(*reinterpret_cast<const __half2*>(&u));
 }
 
 // rounded (non-contracted) arithmetic: the reference rounds every product before the atomic add

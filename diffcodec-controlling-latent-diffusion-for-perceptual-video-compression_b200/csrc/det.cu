@@ -141,7 +141,7 @@ static DetLayout det_layout(long long N, long long C, long long H, long long W, 
     L.sorted_off = align_up(nkeys * 8, 256);
     L.temp_off = L.sorted_off + align_up(nkeys * 8, 256);
     L.acc_off = L.temp_off + align_up((long long)L.temp_bytes, 256);
-    const bool acc_is_out = mode == DCB_MODE_SUM && dtype != DCB_BF16;
+    const bool acc_is_out = mode == DCB_MODE_SUM && (dtype == DCB_F32 || dtype == DCB_F64);   // 16-bit outputs need the fp32 planes
     L.total_bytes = L.acc_off + (acc_is_out ? 0 : align_up(total * cacc * (dtype == DCB_F64 ? 8 : 4), 256));
     return L;
 }
@@ -191,7 +191,7 @@ int splat_fwd_det_impl(const DcbTensor* in, const DcbTensor* flow, const DcbTens
     char* base = (char*)ws;
     a.keys = (unsigned long long*)(base + L.keys_off);
     a.sorted = (const unsigned long long*)(base + L.sorted_off);
-    const bool acc_is_out = mode == DCB_MODE_SUM && in->dtype != DCB_BF16;
+    const bool acc_is_out = mode == DCB_MODE_SUM && (in->dtype == DCB_F32 || in->dtype == DCB_F64);
     a.acc = acc_is_out ? out->ptr : (void*)(base + L.acc_off);
 
     const bool ff = flow->dtype == DCB_F32;
@@ -202,6 +202,7 @@ int splat_fwd_det_impl(const DcbTensor* in, const DcbTensor* flow, const DcbTens
         case DCB_BF16:
             rc = ff ? launch_det<__nv_bfloat16, float>(a, L, base, st) : launch_det<__nv_bfloat16, __nv_bfloat16>(a, L, base, st);
             break;
+        case DCB_F16: rc = ff ? launch_det<__half, float>(a, L, base, st) : launch_det<__half, __half>(a, L, base, st); break;
         default: return set_error(DCB_E_DTYPE, "splat_fwd(deterministic): unsupported dtype %d", in->dtype);
     }
     if (rc != DCB_OK || acc_is_out) return rc;

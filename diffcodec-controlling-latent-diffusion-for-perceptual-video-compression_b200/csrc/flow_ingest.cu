@@ -98,6 +98,7 @@ int flow_ingest_impl(const DcbTensor* flow, const DcbTensor* out, int mode, cuda
     } else {                                            // control_utils.py:90-95: u / ((w - 1) / 2.0)
         a.mu = (float)((double)(a.tw - 1) / 2.0); a.mv = (float)((double)(a.th - 1) / 2.0);
     }
+    if (out->dtype != DCB_F32 && out->dtype != DCB_BF16) return set_error(DCB_E_DTYPE, "flow_resize: out must be F32 or BF16, got %d", out->dtype);
     const bool of32 = out->dtype == DCB_F32;
     if (flow->dtype == DCB_F32) return of32 ? launch_ingest<float, float>(a, st) : launch_ingest<float, __nv_bfloat16>(a, st);
     if (flow->dtype == DCB_BF16) return of32 ? launch_ingest<__nv_bfloat16, float>(a, st) : launch_ingest<__nv_bfloat16, __nv_bfloat16>(a, st);

@@ -155,7 +155,8 @@ int bidir_fuse_fwd_impl(const DcbTensor* A, const DcbTensor* B, const DcbTensor*
     const unsigned blocks = (a.total + px - 1) / px;
     if (A->dtype == DCB_F32) k_bidir_fuse_fwd<float><<<blocks, block, 0, st>>>(a);
     else if (A->dtype == DCB_BF16) k_bidir_fuse_fwd<__nv_bfloat16><<<blocks, block, 0, st>>>(a);
-    else return set_error(DCB_E_DTYPE, "bidir_fuse: F32 or BF16 only, got %d", A->dtype);
+    else if (A->dtype == DCB_F16) k_bidir_fuse_fwd<__half><<<blocks, block, 0, st>>>(a);
+    else return set_error(DCB_E_DTYPE, "bidir_fuse: F32, BF16 or F16 only, got %d", A->dtype);
     DCB_CHECK_LAUNCH("k_bidir_fuse_fwd");
     return DCB_OK;
 }
@@ -176,7 +177,8 @@ int bidir_fuse_bwd_impl(const DcbTensor* g, const DcbTensor* A, const DcbTensor*
     const size_t smem = cs > 1 ? (size_t)256 * 2 * sizeof(float) : 0;
     if (A->dtype == DCB_F32) k_bidir_fuse_bwd<float><<<blocks, block, smem, st>>>(a);
     else if (A->dtype == DCB_BF16) k_bidir_fuse_bwd<__nv_bfloat16><<<blocks, block, smem, st>>>(a);
-    else return set_error(DCB_E_DTYPE, "bidir_fuse: F32 or BF16 only, got %d", A->dtype);
+    else if (A->dtype == DCB_F16) k_bidir_fuse_bwd<__half><<<blocks, block, smem, st>>>(a);
+    else return set_error(DCB_E_DTYPE, "bidir_fuse: F32, BF16 or F16 only, got %d", A->dtype);
     DCB_CHECK_LAUNCH("k_bidir_fuse_bwd");
     return DCB_OK;
 }

@@ -40,7 +40,7 @@ struct ResampleJob {
     void* dst;               // [N,C,th,tw] contiguous
     int N, C, H, W, th, tw;
     int align, op;           // align_corners; DCB_RESAMPLE_*
-    int src_bf16, dst_bf16;
+    int src_st, dst_st;      // storage of src / dst: kStF32, kStBF16 or kStF16
     float sx, sy, f0, f1;    // source-index scales; post factor of channel 0 / of every other channel
     unsigned block0, blocks; // 256-thread blocks of this job inside the launch
 };
@@ -49,11 +49,16 @@ struct ResampleArgs {
     int n_jobs;
 };
 
-__device__ __forceinline__ float ld_rt(const void* p, long long i, int bf16) {
-    return bf16 ? __bfloat162float(((const __nv_bfloat16*)p)[i]) : ((const float*)p)[i];
+// storage of a resample tensor; a batch with any F16 tensor runs k_resample_batch_f16, which knows all three codes
+enum { kStF32 = 0, kStBF16 = 1, kStF16 = 2 };
+static int storage_code(int dtype) { return dtype == DCB_BF16 ? kStBF16 : (dtype == DCB_F16 ? kStF16 : kStF32); }
+template <bool F16> __device__ __forceinline__ float ld_rt(const void* p, long long i, int code) {
+    if (F16 && code == kStF16) return __half2float(((const __half*)p)[i]);
+    return code ? __bfloat162float(((const __nv_bfloat16*)p)[i]) : ((const float*)p)[i];
 }
-__device__ __forceinline__ void st_rt(void* p, long long i, int bf16, float v) {
-    if (bf16) ((__nv_bfloat16*)p)[i] = __float2bfloat16_rn(v); else ((float*)p)[i] = v;
+template <bool F16> __device__ __forceinline__ void st_rt(void* p, long long i, int code, float v) {
+    if (F16 && code == kStF16) ((__half*)p)[i] = __float2half_rn(v);
+    else if (code) ((__nv_bfloat16*)p)[i] = __float2bfloat16_rn(v); else ((float*)p)[i] = v;
 }
 __device__ __forceinline__ float src_index_rt(float scale, int dst, bool align) {
     if (align) return mul_rn(scale, (float)dst);
@@ -61,7 +66,7 @@ __device__ __forceinline__ float src_index_rt(float scale, int dst, bool align) 
     return s < 0.f ? 0.f : s;
 }
 
-__global__ void __launch_bounds__(256) k_resample_batch(const __grid_constant__ ResampleArgs a) {
+template <bool F16> __device__ __forceinline__ void resample_batch(const ResampleArgs& a) {
     pdl_wait();
     int j = 0;
     while (j + 1 < a.n_jobs && blockIdx.x >= a.job[j + 1].block0) ++j;
@@ -78,17 +83,19 @@ __global__ void __launch_bounds__(256) k_resample_batch(const __grid_constant__ 
     const long long plane = (long long)b.th * b.tw;
     for (int c = 0; c < b.C; ++c) {
         const long long q = base + c * b.src.sC;
-        const float v00 = ld_rt(b.src.p, q, b.src_bf16), v01 = ld_rt(b.src.p, q + px * b.src.sW, b.src_bf16);
-        const float v10 = ld_rt(b.src.p, q + py * b.src.sH, b.src_bf16), v11 = ld_rt(b.src.p, q + py * b.src.sH + px * b.src.sW, b.src_bf16);
+        const float v00 = ld_rt<F16>(b.src.p, q, b.src_st), v01 = ld_rt<F16>(b.src.p, q + px * b.src.sW, b.src_st);
+        const float v10 = ld_rt<F16>(b.src.p, q + py * b.src.sH, b.src_st), v11 = ld_rt<F16>(b.src.p, q + py * b.src.sH + px * b.src.sW, b.src_st);
         // torch: h0lambda * (w0lambda * v00 + w1lambda * v01) + h1lambda * (w0lambda * v10 + w1lambda * v11)
         const float top = add_rn(mul_rn(lx0, v00), mul_rn(lx1, v01)), bot = add_rn(mul_rn(lx0, v10), mul_rn(lx1, v11));
         float r = add_rn(mul_rn(ly0, top), mul_rn(ly1, bot));
         const float f = c == 0 ? b.f0 : b.f1;
         if (b.op == DCB_RESAMPLE_MUL) r = mul_rn(r, f);
         else if (b.op == DCB_RESAMPLE_DIV) r = r / f;
-        st_rt(b.dst, ((long long)n * b.C + c) * plane + (long long)y * b.tw + x, b.dst_bf16, r);
+        st_rt<F16>(b.dst, ((long long)n * b.C + c) * plane + (long long)y * b.tw + x, b.dst_st, r);
     }
 }
+__global__ void __launch_bounds__(256) k_resample_batch(const __grid_constant__ ResampleArgs a) { resample_batch<false>(a); }
+__global__ void __launch_bounds__(256) k_resample_batch_f16(const __grid_constant__ ResampleArgs a) { resample_batch<true>(a); }
 
 int resample_batch_impl(const DcbResampleJob* jobs, int n_jobs, cudaStream_t st) {
     for (int j0 = 0; j0 < n_jobs; j0 += kMaxResample) {
@@ -104,7 +111,7 @@ int resample_batch_impl(const DcbResampleJob* jobs, int n_jobs, cudaStream_t st)
             b.N = (int)d->size[0]; b.C = (int)d->size[1]; b.H = (int)s->size[2]; b.W = (int)s->size[3];
             b.th = (int)d->size[2]; b.tw = (int)d->size[3];
             b.align = jobs[j].align_corners ? 1 : 0; b.op = jobs[j].op;
-            b.src_bf16 = s->dtype == DCB_BF16; b.dst_bf16 = d->dtype == DCB_BF16;
+            b.src_st = storage_code(s->dtype); b.dst_st = storage_code(d->dtype);
             // torch area_pixel_compute_scale<float>
             b.sy = b.align ? (b.th > 1 ? (float)(b.H - 1) / (float)(b.th - 1) : 0.f) : (float)b.H / (float)b.th;
             b.sx = b.align ? (b.tw > 1 ? (float)(b.W - 1) / (float)(b.tw - 1) : 0.f) : (float)b.W / (float)b.tw;
@@ -113,7 +120,9 @@ int resample_batch_impl(const DcbResampleJob* jobs, int n_jobs, cudaStream_t st)
             blocks += b.blocks;
         }
         if (a.n_jobs == 0) continue;
-        DCB_CHECK_CUDA(launch_pdl(k_resample_batch, dim3(blocks), dim3(256), 0, st, a));
+        bool f16 = false;
+        for (int j = 0; j < a.n_jobs; ++j) f16 = f16 || a.job[j].src_st == kStF16 || a.job[j].dst_st == kStF16;
+        DCB_CHECK_CUDA(launch_pdl(f16 ? k_resample_batch_f16 : k_resample_batch, dim3(blocks), dim3(256), 0, st, a));
         count_launch();
     }
     return DCB_OK;
@@ -306,7 +315,7 @@ static int launch_pyramid(const PyrScatterArgs& sa, unsigned s_items, const PyrF
     return DCB_OK;
 }
 
-// Preconditions (checked by the caller): 1 <= n <= kMaxLevels, all tensors of one dtype (F32 / BF16), shapes consistent,
+// Preconditions (checked by the caller): 1 <= n <= kMaxLevels, all tensors of one dtype (F32 / BF16 / F16), shapes consistent,
 // ws holds pyramid_workspace() bytes, 256-byte aligned, all-zero if DCB_FLAG_WS_CLEAN.
 int bidir_pyramid_fwd_impl(const DcbPyramidLevel* lv, int n, void* ws, int flags, cudaStream_t st) {
     PyrScatterArgs sa; PyrFuseArgs fa;
@@ -364,7 +373,13 @@ int bidir_pyramid_fwd_impl(const DcbPyramidLevel* lv, int n, void* ws, int flags
         f_items += L.items;
     }
     if (fa.n_levels == 0) return DCB_OK;
-    const int rc = dt == DCB_F32 ? launch_pyramid<float>(sa, s_items, fa, f_items, st) : launch_pyramid<__nv_bfloat16>(sa, s_items, fa, f_items, st);
+    int rc;
+    switch (dt) {
+        case DCB_F32: rc = launch_pyramid<float>(sa, s_items, fa, f_items, st); break;
+        case DCB_BF16: rc = launch_pyramid<__nv_bfloat16>(sa, s_items, fa, f_items, st); break;
+        case DCB_F16: rc = launch_pyramid<__half>(sa, s_items, fa, f_items, st); break;
+        default: return set_error(DCB_E_DTYPE, "bidir_pyramid_fwd: unsupported dtype %d", dt);
+    }
     if (rc != DCB_OK) return rc;
     // the per-pixel planes have several readers (one warp per channel group): re-zeroed behind the kernel
     DCB_CHECK_CUDA(cudaMemsetAsync(ws, 0, (size_t)shared_total, st));

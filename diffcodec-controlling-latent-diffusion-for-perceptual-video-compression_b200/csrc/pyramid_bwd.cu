@@ -148,7 +148,7 @@ static int launch_pyramid_bwd(const PyrBwdTargetArgs& ta, unsigned t_blocks, con
     return DCB_OK;
 }
 
-// Preconditions (checked by the caller): 1 <= n <= kBwdMaxLevels, one dtype (F32 / BF16) for all tensors, shapes consistent,
+// Preconditions (checked by the caller): 1 <= n <= kBwdMaxLevels, one dtype (F32 / BF16 / F16) for all tensors, shapes consistent,
 // the six saved forward outputs present, ws holds pyramid_bwd_workspace() bytes, 256-byte aligned.
 int bidir_pyramid_bwd_impl(const DcbPyramidBwdLevel* lv, int n, void* ws, bool holes, cudaStream_t st) {
     PyrBwdTargetArgs ta; PyrBwdSourceArgs sa;
@@ -206,8 +206,12 @@ int bidir_pyramid_bwd_impl(const DcbPyramidBwdLevel* lv, int n, void* ws, bool h
         if (want_b) add_job(d.last, d.flow_b, d.metric_b, ts_b, d.grad_last, d.grad_flow_b, d.grad_metric_b, conf_b);
     }
     if (ta.n_levels == 0) return DCB_OK;
-    return lv[0].first->dtype == DCB_F32 ? launch_pyramid_bwd<float>(ta, t_blocks, sa, s_blocks, st)
-                                         : launch_pyramid_bwd<__nv_bfloat16>(ta, t_blocks, sa, s_blocks, st);
+    switch (lv[0].first->dtype) {
+        case DCB_F32: return launch_pyramid_bwd<float>(ta, t_blocks, sa, s_blocks, st);
+        case DCB_BF16: return launch_pyramid_bwd<__nv_bfloat16>(ta, t_blocks, sa, s_blocks, st);
+        case DCB_F16: return launch_pyramid_bwd<__half>(ta, t_blocks, sa, s_blocks, st);
+    }
+    return set_error(DCB_E_DTYPE, "bidir_pyramid_bwd: unsupported dtype %d", lv[0].first->dtype);
 }
 
 }  // namespace dcb

@@ -158,8 +158,9 @@ int occlusion_mask_impl(const DcbTensor* flow_a, const DcbTensor* flow_b, const 
     const long long need = mask_workspace(N, H, W);
     if (need > 0 && (!ws || ws_bytes < need || ((uintptr_t)ws & 255)))
         return set_error(DCB_E_WORKSPACE, "occlusion_mask: workspace of %lld bytes required, got %lld", need, ws_bytes);
-    if (flow_a->dtype != DCB_F32 && flow_a->dtype != DCB_BF16)
-        return set_error(DCB_E_DTYPE, "occlusion_mask: F32 or BF16 only, got %d", flow_a->dtype);
+    // F16 comes only from the bi-directional block's launch sequence (dcb_bidir_block_fwd); dcb_occlusion_mask refuses it
+    if (flow_a->dtype != DCB_F32 && !is_half_storage(flow_a->dtype))
+        return set_error(DCB_E_DTYPE, "occlusion_mask: F32, BF16 or F16 only, got %d", flow_a->dtype);
     const bool owner = use_owner(flow_a->dtype, DCB_MODE_SOFT, 2, H, W), clean = (flags & DCB_FLAG_WS_CLEAN) != 0;
     const int rc = ones_splat(flow_a, flow_b, nullptr, mask, ws, owner, clean, st);
     if (rc == DCB_OK && owner && clean && need > 0) DCB_CHECK_CUDA(cudaMemsetAsync(ws, 0, (size_t)need, st));

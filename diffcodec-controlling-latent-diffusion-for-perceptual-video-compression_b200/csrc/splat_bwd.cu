@@ -343,6 +343,8 @@ static int launch_bwd(BwdArgs& a, int dtype, cudaStream_t st) {
                            (long long)(a.W - 1) * (a.gout.sW < 0 ? -a.gout.sW : a.gout.sW);
     if (span < (1ll << 30))
         k_bwd_source<T, TF, int><<<blocks, block, smem, st>>>(a);
+    else if constexpr (std::is_same<T, __half>::value)   // the 64-bit form spills; fp16 keeps the limit of the pyramid backward
+        return set_error(DCB_E_LIMIT, "splat_bwd: F16 grad_out spanning 2^30 elements per plane or more is not supported");
     else
         k_bwd_source<T, TF, long long><<<blocks, block, smem, st>>>(a);
     DCB_CHECK_LAUNCH("k_bwd_source");
@@ -385,6 +387,7 @@ int splat_bwd_impl(const DcbTensor* gout, const DcbTensor* in, const DcbTensor* 
         case DCB_F64: return launch_bwd<double, double>(a, DCB_F64, st);
         case DCB_BF16:
             return flow_f32 ? launch_bwd<__nv_bfloat16, float>(a, DCB_BF16, st) : launch_bwd<__nv_bfloat16, __nv_bfloat16>(a, DCB_BF16, st);
+        case DCB_F16: return flow_f32 ? launch_bwd<__half, float>(a, DCB_F16, st) : launch_bwd<__half, __half>(a, DCB_F16, st);
     }
     return set_error(DCB_E_DTYPE, "splat_bwd: unsupported dtype %d", in->dtype);
 }

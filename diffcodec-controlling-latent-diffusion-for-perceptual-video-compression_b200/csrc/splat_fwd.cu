@@ -4,8 +4,8 @@
 // Replaces controlnet/softsplat.py:232-274 (mode wrapper: cat / exp / mul pre-ops, eps + divide
 // post-ops) and :277-355 (softsplat_func.forward, kernel `softsplat_out`) of the reference.
 //
-//   fp32 / bf16, C + 1 <= 4 (frames, flows, SD latents)  -> splat_pipe.cu   (float4 accumulators)
-//   fp32 / bf16, more channels (feature maps)             -> splat_planar.cu (channel-quad accumulators),
+//   fp32 / bf16 / fp16, C + 1 <= 4 (frames, flows, SD latents)  -> splat_pipe.cu   (float4 accumulators)
+//   fp32 / bf16 / fp16, more channels (feature maps)             -> splat_planar.cu (channel-quad accumulators),
 //                                      and >= 16 MB of them -> splat_lists.cu  (per-target lists + gather)
 //   fp64 (the reference supports double; gradcheck uses it) -> this file
 //
@@ -184,9 +184,9 @@ bool small_frames(int dtype, int mode, long long N, long long C, long long H, lo
 
 // C+1 <= 8 channels in fp32 / bf16: target-tile ownership, accumulators in shared memory (splat_owner.cu)
 // Opt-in only: measured on B200 (profiles/r02/NOTES.md) it needs 2-3x the instructions of the accumulator pipeline and loses
-// at every size, so the automatic dispatch never picks it.
+// at every size, so the automatic dispatch never picks it. It has no fp16 instantiation: fp16 stays on the pipelines.
 bool use_owner(int dtype, int mode, long long C, long long H, long long W) {
-    if (dtype == DCB_F64 || g_fwd_path != 2) return false;
+    if (dtype == DCB_F64 || dtype == DCB_F16 || g_fwd_path != 2) return false;
     return owner_supported(C, mode, H, W);
 }
 
@@ -240,6 +240,7 @@ int normalize_planar_launch(int dtype, const DcbTensor* in, const DcbTensor* out
         case DCB_F32: k_normalize<float><<<blocks, kThreads, 0, st>>>(a); break;
         case DCB_F64: k_normalize<double><<<blocks, kThreads, 0, st>>>(a); break;
         case DCB_BF16: k_normalize<__nv_bfloat16><<<blocks, kThreads, 0, st>>>(a); break;
+        case DCB_F16: k_normalize<__half><<<blocks, kThreads, 0, st>>>(a); break;
         default: return set_error(DCB_E_DTYPE, "normalize: unsupported dtype %d", dtype);
     }
     DCB_CHECK_LAUNCH("k_normalize");
@@ -285,7 +286,7 @@ int splat_fwd_impl(const DcbTensor* in, const DcbTensor* flow, const DcbTensor* 
         fill_args(a, in, flow, metric, mask, out, norm, mode, eps);
         return splat_fwd_f64(a, out, ws, ws_bytes, mode, ws_clean, mask != nullptr, st);
     }
-    if (in->dtype != DCB_F32 && in->dtype != DCB_BF16) return set_error(DCB_E_DTYPE, "splat_fwd: unsupported dtype %d", in->dtype);
+    if (in->dtype != DCB_F32 && !is_half_storage(in->dtype)) return set_error(DCB_E_DTYPE, "splat_fwd: unsupported dtype %d", in->dtype);
     if (use_owner(in->dtype, mode, C, H, W)) {
         if (!pipe_supported(in, flow, metric))
             return set_error(DCB_E_LIMIT, "splat_fwd: tensor spans beyond 2^31 elements are not supported (32-bit in-frame offsets)");

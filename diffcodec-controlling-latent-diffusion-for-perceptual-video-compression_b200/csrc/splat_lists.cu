@@ -1,4 +1,4 @@
-// splat_lists.cu -- forward splat for MANY channels on LARGE tensors (fp32 / bf16): per-target
+// splat_lists.cu -- forward splat for MANY channels on LARGE tensors (fp32 / bf16 / fp16): per-target
 // contribution lists built once per flow field, then ONE gather pass per channel. sm_100a.
 //
 // Replaces controlnet/softsplat.py:240-270 (pre/post ops) + :281-345 (zero-init + softsplat_out)
@@ -26,7 +26,7 @@
 // Frames are processed in groups whose lists (32 B per pixel) stay L2-resident.
 //
 // Channels-last (NHWC) input takes its own gather (k_list_gather_nhwc): eight lanes walk the CHANNELS of one target, so a
-// list entry is one 16-byte (fp32) / 8-byte (bf16) load per lane and channel quad, 128 contiguous bytes per group, and there
+// list entry is one 16-byte (fp32) / 8-byte (bf16, fp16) load per lane and channel quad, 128 contiguous bytes per group, and there
 // is one address computation per four channels; the entries of a list are read once and reused for all channels. The NCHW output the
 // reference's callers expect is written through a shared-memory transpose, 128 contiguous bytes per store.
 #include "dcb_common.cuh"
@@ -55,6 +55,11 @@ __device__ __forceinline__ float ld_global_ro(const __nv_bfloat16* p) {
     unsigned short v;
     asm("ld.global.nc.u16 %0, [%1];" : "=h"(v) : "l"(p));
     return __uint_as_float((unsigned)v << 16);
+}
+__device__ __forceinline__ float ld_global_ro(const __half* p) {
+    unsigned short v;
+    asm("ld.global.nc.u16 %0, [%1];" : "=h"(v) : "l"(p));
+    return __half2float(__ushort_as_half(v));
 }
 
 // dcb_set_option("lists_nhwc", 0): A/B switch, channels-last input through the NCHW gather (strided scalar loads)
@@ -244,6 +249,12 @@ __device__ __forceinline__ void ld_quad_ro(const __nv_bfloat16* p, float (&o)[4]
     o[0] = __uint_as_float(lo << 16); o[1] = __uint_as_float(lo & 0xffff0000u);
     o[2] = __uint_as_float(hi << 16); o[3] = __uint_as_float(hi & 0xffff0000u);
 }
+__device__ __forceinline__ void ld_quad_ro(const __half* p, float (&o)[4]) {
+    unsigned lo, hi;
+    asm("ld.global.nc.v2.u32 {%0,%1}, [%2];" : "=r"(lo), "=r"(hi) : "l"(p));
+    const float2 a = __half22float2(*reinterpret_cast<const __half2*>(&lo)), b = __half22float2(*reinterpret_cast<const __half2*>(&hi));
+    o[0] = a.x; o[1] = a.y; o[2] = b.x; o[3] = b.y;
+}
 
 #ifndef DCB_LQ_CBLK
 #define DCB_LQ_CBLK 64        // channels per pass through the transpose tile (8.25 KB of shared memory; measured: 64 beats 32 and 128 at C = 64)
@@ -373,7 +384,7 @@ long long lists_workspace(long long N, long long H, long long W) { return lists_
 bool lists_supported(const DcbTensor* in, const DcbTensor* flow, const DcbTensor* metric, int mode) {
     (void)flow; (void)metric;
     const long long N = in->size[0], C = in->size[1], H = in->size[2], W = in->size[3];
-    if (in->dtype != DCB_F32 && in->dtype != DCB_BF16) return false;
+    if (in->dtype != DCB_F32 && !is_half_storage(in->dtype)) return false;
     // building the lists costs about as much as scattering 8-16 channels (measured crossover on
     // 1080p, 540p and 256 x 256 batches with a rough random flow: lists lose at C = 8, win from C = 16)
     if (C < 16) return false;
@@ -458,6 +469,8 @@ int splat_lists_impl(const DcbTensor* in, const DcbTensor* flow, const DcbTensor
     if (in->dtype == DCB_F32) rc = launch_lists<float, float>(a, L, base, N, clean, st);
     else if (in->dtype == DCB_BF16)
         rc = ff ? launch_lists<__nv_bfloat16, float>(a, L, base, N, clean, st) : launch_lists<__nv_bfloat16, __nv_bfloat16>(a, L, base, N, clean, st);
+    else if (in->dtype == DCB_F16)
+        rc = ff ? launch_lists<__half, float>(a, L, base, N, clean, st) : launch_lists<__half, __half>(a, L, base, N, clean, st);
     else return set_error(DCB_E_DTYPE, "splat_lists: unsupported dtype %d", in->dtype);
     return rc;
 }

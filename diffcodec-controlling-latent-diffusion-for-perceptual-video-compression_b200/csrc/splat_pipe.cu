@@ -410,6 +410,11 @@ __device__ __forceinline__ void st_stream4(__nv_bfloat16* p, float a, float b, f
     uint2 u; u.x = *reinterpret_cast<const unsigned*>(&lo); u.y = *reinterpret_cast<const unsigned*>(&hi);
     __stcs((uint2*)p, u);
 }
+__device__ __forceinline__ void st_stream4(__half* p, float a, float b, float c, float d) {
+    const __half2 lo = __floats2half2_rn(a, b), hi = __floats2half2_rn(c, d);
+    uint2 u; u.x = *reinterpret_cast<const unsigned*>(&lo); u.y = *reinterpret_cast<const unsigned*>(&hi);
+    __stcs((uint2*)p, u);
+}
 
 template <class T, int MODE, int CA>
 __device__ __forceinline__ void normalize_chunk_v4(const PipeArgs& a, int frame, int chunk, float* acc, int lane) {
@@ -475,6 +480,10 @@ __device__ __forceinline__ void zero_cells2(float* p) {
 __device__ __forceinline__ void st_stream2(float* p, float a, float b) { __stcs((float2*)p, make_float2(a, b)); }
 __device__ __forceinline__ void st_stream2(__nv_bfloat16* p, float a, float b) {
     const __nv_bfloat162 v = __floats2bfloat162_rn(a, b);
+    __stcs((unsigned*)p, *reinterpret_cast<const unsigned*>(&v));
+}
+__device__ __forceinline__ void st_stream2(__half* p, float a, float b) {
+    const __half2 v = __floats2half2_rn(a, b);
     __stcs((unsigned*)p, *reinterpret_cast<const unsigned*>(&v));
 }
 __device__ __forceinline__ float comp(const float4& v, int i) { return i == 0 ? v.x : (i == 1 ? v.y : (i == 2 ? v.z : v.w)); }
@@ -1063,7 +1072,7 @@ static bool planes_pair_aligned(const DcbTensor* t, long long W) {
     return t->stride[3] == 1 && t->stride[2] == W && t->stride[1] % 2 == 0 && t->stride[0] % 2 == 0 && ((uintptr_t)t->ptr % (2 * es)) == 0;
 }
 
-// Preconditions (checked by the caller): C + (mode != SUM) <= 4, dtype F32/BF16, workspace >= pipe_workspace().
+// Preconditions (checked by the caller): C + (mode != SUM) <= 4, dtype F32/BF16/F16, workspace >= pipe_workspace().
 int splat_pipe_impl(const DcbTensor* in, const DcbTensor* flow, const DcbTensor* metric, const DcbTensor* out,
                     const DcbTensor* norm, const DcbTensor* mask, void* ws, int mode, int eps, bool ws_clean,
                     cudaStream_t st, bool ones_metric, const DcbTensor* mask_out) {
@@ -1096,6 +1105,7 @@ int splat_pipe_impl(const DcbTensor* in, const DcbTensor* flow, const DcbTensor*
     if (in->dtype == DCB_F32) return launch_pipe<float, float>(a, mode, st);
     if (in->dtype == DCB_BF16)
         return ff ? launch_pipe<__nv_bfloat16, float>(a, mode, st) : launch_pipe<__nv_bfloat16, __nv_bfloat16>(a, mode, st);
+    if (in->dtype == DCB_F16) return ff ? launch_pipe<__half, float>(a, mode, st) : launch_pipe<__half, __half>(a, mode, st);
     return set_error(DCB_E_DTYPE, "splat_pipe: unsupported dtype %d", in->dtype);
 }
 

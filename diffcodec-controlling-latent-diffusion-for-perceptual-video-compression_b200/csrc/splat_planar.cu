@@ -1,4 +1,4 @@
-// splat_planar.cu -- forward splat for MANY channels (feature maps: C = 64 .. 640) in fp32 / bf16,
+// splat_planar.cu -- forward splat for MANY channels (feature maps: C = 64 .. 640) in fp32 / bf16 / fp16,
 // as the same kernel-per-step software pipeline as splat_pipe.cu, with planar accumulators.
 //
 // Replaces controlnet/softsplat.py:240-270 (pre/post ops) + :281-345 (zero-init + softsplat_out)
@@ -18,6 +18,8 @@
 //     normalises frame group k-1 (and re-zeroes it) while it scatters group k; the kernel boundary
 //     is the only synchronisation; inputs/outputs use streaming loads/stores.
 #include "splat_planar.cuh"
+
+#include <type_traits>
 
 namespace dcb {
 
@@ -230,16 +232,19 @@ static void split_channels(long long items, int channels, int min_cg, int* cg, i
 template <class T, class TF> static int launch_planar(PlanarArgs& a, cudaStream_t st) {
     const int groups = (a.N + a.G - 1) / a.G;
     const bool normalised = a.mode != DCB_MODE_SUM;
-    if (g_planar_one && groups == 1) {
-        // every scatter item needs its own warp; the normalise items are looped over. Half of the CTA slots at most.
-        const long long s_items = (long long)a.N * a.ts * a.ncg_s;
-        const long long ctas = (s_items + kPWarps - 1) / kPWarps;
-        if (ctas > 0 && 2 * ctas <= one_launch_slots<T, TF>()) {
-            a.step = 0; a.s_frame0 = a.n_frame0 = 0; a.s_frames = a.n_frames = a.N;
-            DCB_CHECK_CUDA(launch_pdl(k_planar_one<T, TF>, dim3((unsigned)ctas), dim3(kPThreads), 0, st, a));
-            count_launch();
-            if (normalised && a.ncg_n > 1) DCB_CHECK_CUDA(cudaMemsetAsync(a.dacc, 0, (size_t)a.G * a.HW * 4, st));
-            return DCB_OK;
+    // the single-launch kernel is opt-in evidence (measured slower) and has no fp16 instantiation
+    if constexpr (!std::is_same<T, __half>::value) {
+        if (g_planar_one && groups == 1) {
+            // every scatter item needs its own warp; the normalise items are looped over. Half of the CTA slots at most.
+            const long long s_items = (long long)a.N * a.ts * a.ncg_s;
+            const long long ctas = (s_items + kPWarps - 1) / kPWarps;
+            if (ctas > 0 && 2 * ctas <= one_launch_slots<T, TF>()) {
+                a.step = 0; a.s_frame0 = a.n_frame0 = 0; a.s_frames = a.n_frames = a.N;
+                DCB_CHECK_CUDA(launch_pdl(k_planar_one<T, TF>, dim3((unsigned)ctas), dim3(kPThreads), 0, st, a));
+                count_launch();
+                if (normalised && a.ncg_n > 1) DCB_CHECK_CUDA(cudaMemsetAsync(a.dacc, 0, (size_t)a.G * a.HW * 4, st));
+                return DCB_OK;
+            }
         }
     }
     for (int k = 0; k <= groups; ++k) {
@@ -266,7 +271,7 @@ template <class T, class TF> static int launch_planar(PlanarArgs& a, cudaStream_
     return DCB_OK;
 }
 
-// fp32 / bf16, any channel count. `ws` must hold planar_workspace() bytes (all-zero if ws_clean).
+// fp32 / bf16 / fp16, any channel count. `ws` must hold planar_workspace() bytes (all-zero if ws_clean).
 int splat_planar_impl(const DcbTensor* in, const DcbTensor* flow, const DcbTensor* metric, const DcbTensor* out,
                       const DcbTensor* norm, const DcbTensor* mask, void* ws, int mode, int eps, bool ws_clean,
                       cudaStream_t st) {
@@ -296,6 +301,7 @@ int splat_planar_impl(const DcbTensor* in, const DcbTensor* flow, const DcbTenso
     if (in->dtype == DCB_F32) return launch_planar<float, float>(a, st);
     if (in->dtype == DCB_BF16)
         return ff ? launch_planar<__nv_bfloat16, float>(a, st) : launch_planar<__nv_bfloat16, __nv_bfloat16>(a, st);
+    if (in->dtype == DCB_F16) return ff ? launch_planar<__half, float>(a, st) : launch_planar<__half, __half>(a, st);
     return set_error(DCB_E_DTYPE, "splat_planar: unsupported dtype %d", in->dtype);
 }
 

@@ -42,7 +42,7 @@ struct PlanarArgs {
     unsigned* bar;           // single-launch kernel (k_planar_one): arrive / depart counters in the workspace, zero between calls
 };
 
-// the four channels of a quad of a channels-last (NHWC) tensor in one load: 16 bytes fp32, 8 bytes bf16
+// the four channels of a quad of a channels-last (NHWC) tensor in one load: 16 bytes fp32, 8 bytes bf16 / fp16
 __device__ __forceinline__ void ld_quad(const float* p, float (&o)[4]) {
     const float4 t = __ldcs((const float4*)p);
     o[0] = t.x; o[1] = t.y; o[2] = t.z; o[3] = t.w;
@@ -52,11 +52,16 @@ __device__ __forceinline__ void ld_quad(const __nv_bfloat16* p, float (&o)[4]) {
     o[0] = __uint_as_float(u.x << 16); o[1] = __uint_as_float(u.x & 0xffff0000u);
     o[2] = __uint_as_float(u.y << 16); o[3] = __uint_as_float(u.y & 0xffff0000u);
 }
+__device__ __forceinline__ void ld_quad(const __half* p, float (&o)[4]) {
+    const uint2 u = __ldcs((const uint2*)p);
+    const float2 lo = __half22float2(*reinterpret_cast<const __half2*>(&u.x)), hi = __half22float2(*reinterpret_cast<const __half2*>(&u.y));
+    o[0] = lo.x; o[1] = lo.y; o[2] = hi.x; o[3] = hi.y;
+}
 
 // host: can `in` ([N,C,H,W] view) be read quad-wise?
 inline bool planar_vec_ok(const DcbTensor* in) {
-    const long long es = in->dtype == DCB_BF16 ? 2 : 4;
-    if (in->dtype != DCB_F32 && in->dtype != DCB_BF16) return false;
+    const long long es = elem_size(in->dtype);
+    if (in->dtype != DCB_F32 && !is_half_storage(in->dtype)) return false;
     if (in->stride[1] != 1 || in->size[1] % 4 != 0 || in->size[1] < 4) return false;
     if (((uintptr_t)in->ptr) % (uintptr_t)(4 * es)) return false;
     return in->stride[0] % 4 == 0 && in->stride[2] % 4 == 0 && in->stride[3] % 4 == 0;

@@ -171,7 +171,7 @@ static long long small_quads(long long C, int mode) { return (C + (mode == DCB_M
 // but 4x4x135x240 latents (8 rounds per frame, 32 of 148 SMs busy) 45.6 / 16.4 and 4x3x256x256 47.6 / 12.3: bigger frames stay
 // on the pipelines, whose two launches spread a frame over the whole machine.
 bool use_cluster(int dtype, int mode, long long N, long long C, long long H, long long W) {
-    if (!g_small_path || (dtype != DCB_F32 && dtype != DCB_BF16)) return false;
+    if (!g_small_path || (dtype != DCB_F32 && !is_half_storage(dtype))) return false;
     const long long P = H * W;
     return P > 0 && P <= 8192 && small_quads(C, mode) <= 2 && N <= 64;
 }
@@ -208,6 +208,7 @@ int splat_cluster_impl(const DcbTensor* in, const DcbTensor* flow, const DcbTens
     if (in->dtype == DCB_F32) return launch_small<float, float>(a, st);
     if (in->dtype == DCB_BF16)
         return ff ? launch_small<__nv_bfloat16, float>(a, st) : launch_small<__nv_bfloat16, __nv_bfloat16>(a, st);
+    if (in->dtype == DCB_F16) return ff ? launch_small<__half, float>(a, st) : launch_small<__half, __half>(a, st);
     return set_error(DCB_E_DTYPE, "splat_cluster: unsupported dtype %d", in->dtype);
 }
 

@@ -167,7 +167,8 @@ int tile_merge_impl(const DcbTensor* tiles, const long long* pixel_coords, int n
     auto flush = [&](int last) -> int {
         a.last = last;
         if (out->dtype == DCB_F32) k_tile_merge<float><<<blocks, 256, 0, st>>>(a);
-        else k_tile_merge<__nv_bfloat16><<<blocks, 256, 0, st>>>(a);
+        else if (out->dtype == DCB_BF16) k_tile_merge<__nv_bfloat16><<<blocks, 256, 0, st>>>(a);
+        else k_tile_merge<__half><<<blocks, 256, 0, st>>>(a);
         DCB_CHECK_LAUNCH("k_tile_merge");
         a.first = 0;
         a.n = 0;

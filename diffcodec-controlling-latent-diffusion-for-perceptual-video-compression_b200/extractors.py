@@ -169,7 +169,7 @@ def bidirectional_block(first_features, last_features, flow_f, flow_b, metric_f=
     if metric_b is None:
         metric_b = torch.ones_like(flow_b[:, :1], dtype=dt)
     needs_grad = torch.is_grad_enabled() and any(t.requires_grad for t in (first_features, last_features, flow_f, flow_b, metric_f, metric_b))
-    if (not needs_grad and not torch.is_autocast_enabled("cuda") and dt in (torch.float32, torch.bfloat16)
+    if (not needs_grad and not torch.is_autocast_enabled("cuda") and dt in (torch.float32, torch.bfloat16, torch.float16)
             and last_features.dtype == dt and flow_f.dtype == dt and flow_b.dtype == dt and metric_f.dtype == dt and metric_b.dtype == dt):
         return _block_forward_nograd(first_features, last_features, flow_f, flow_b, metric_f, metric_b)
     cast = lambda t: t if t.dtype == dt else t.to(dt)
@@ -307,7 +307,7 @@ def bidirectional_pyramid(levels, holes=True):
         return bidirectional_pyramid(levels[:_PYRAMID_MAX_LEVELS], holes) + bidirectional_pyramid(levels[_PYRAMID_MAX_LEVELS:], holes)
     dt = levels[0][0].dtype
     grad = torch.is_grad_enabled() and any(t is not None and t.requires_grad for lv in levels for t in lv)
-    plain = (not grad and not torch.is_autocast_enabled("cuda") and dt in (torch.float32, torch.bfloat16)
+    plain = (not grad and not torch.is_autocast_enabled("cuda") and dt in (torch.float32, torch.bfloat16, torch.float16)
              and all(t is None or t.dtype == dt for lv in levels for t in lv))
     if plain:
         return _pyramid_forward(levels, 0 if holes else _lib.PYRAMID_NO_HOLES, False)[0]
@@ -426,7 +426,7 @@ class Bi_Dir_FeatureExtractor(nn.Module):
         flow_fwd, flow_bwd = flow[:, :2], flow[:, 2:]
         flow_res = (64, 32, 16, 8)                                               # extractors.py:278
         from .softsplat import is_deterministic
-        whole = first_features.is_cuda and flow.dtype in (torch.float32, torch.bfloat16) and not is_deterministic()
+        whole = first_features.is_cuda and flow.dtype in (torch.float32, torch.bfloat16, torch.float16) and not is_deterministic()
         if not whole:                                                            # what the pyramid does not take: scale by scale
             outs = []
             for idx, res in enumerate(flow_res):
@@ -451,7 +451,7 @@ class Bi_Dir_FeatureExtractor(nn.Module):
             with torch.no_grad():
                 jobs = []
                 for (f, _), res in zip(feats, flow_res):
-                    dt = torch.float32 if (torch.is_autocast_enabled("cuda") or f.dtype not in (torch.float32, torch.bfloat16)) else f.dtype
+                    dt = torch.float32 if (torch.is_autocast_enabled("cuda") or f.dtype not in (torch.float32, torch.bfloat16, torch.float16)) else f.dtype
                     for fl in (flow_fwd, flow_bwd):
                         jobs.append((fl, (res, res), False, _lib.RESAMPLE_DIV, (res - 1) / 2.0, (res - 1) / 2.0, dt))
                 flows = resample_batch(jobs)
@@ -503,7 +503,7 @@ class Bi_Dir_ResidueExtractor(nn.Module):
             flow_b = self.flow_refiners[i](F.interpolate(flow_bwd, size=(res, res), mode="bilinear", align_corners=False) / factor)
             flows.append((flow_f, flow_b))
         from .softsplat import is_deterministic
-        if not (prev_frame.is_cuda and flow_fwd.dtype in (torch.float32, torch.bfloat16) and not is_deterministic()):
+        if not (prev_frame.is_cuda and flow_fwd.dtype in (torch.float32, torch.bfloat16, torch.float16) and not is_deterministic()):
             outs = []                                                            # what the pyramid does not take: scale by scale
             for i, (flow_f, flow_b) in enumerate(flows):
                 occ_f, occ_b = compute_mask(flow_f, flow_b), compute_mask(flow_b, flow_f)

@@ -36,7 +36,8 @@ def crop_into_tiles(img, tile_size, overlap=0, order="hwc"):
 
 
 def merge_latent_tiles_from_pixel_coords(latents, pixel_coords, full_latent_shape, original_image_size, eps: float = 1e-8):
-    """latents: list of (1, C, th, tw) CUDA tensors (one dtype: float32 or bfloat16); pixel_coords:
+    """latents: list of (1, C, th, tw) CUDA tensors (one dtype: float32, bfloat16 or float16; the 16-bit merges
+    accumulate in fp32 and round once); pixel_coords:
     list of 4-tuples in original pixel space; returns the merged (1, C, H_lat, W_lat) tensor.
     Inference utility: no autograd (the reference's in-place accumulation has none worth keeping)."""
     assert len(latents) == len(pixel_coords), "latents and coords length mismatch"
@@ -46,7 +47,7 @@ def merge_latent_tiles_from_pixel_coords(latents, pixel_coords, full_latent_shap
     n, c, h_lat, w_lat = (int(v) for v in full_latent_shape)
     h_px, w_px = (int(v) for v in original_image_size)
     if dtype not in _lib._DTYPES:
-        raise ValueError(f"unsupported dtype {dtype}: float32 and bfloat16 are implemented")
+        raise ValueError(f"unsupported dtype {dtype}: float32, bfloat16 and float16 are implemented")
     dt = _lib._DTYPES[dtype]
     lib = _lib.lib()
     out = torch.empty((n, c, h_lat, w_lat), dtype=dtype, device=dev)

@@ -94,7 +94,7 @@ def _composed_bidir(image1, image2, flow1, flow2, gt):
     occ_fwd = compute_mask(flow1, flow2).to(image1.dtype)
     occ_bwd = compute_mask(flow2, flow1).to(image1.dtype)
     if image1.dtype == torch.float64:
-        # the fusion kernel is F32/BF16 only: the fp64 composition fuses as _composed does (soft_fuse, improv_experiments.ipynb
+        # the fusion kernel is F32/BF16/F16 only: the fp64 composition fuses as _composed does (soft_fuse, improv_experiments.ipynb
         # cell 3, on the valid masks; no .any() host sync)
         conf = torch.cat([1 - occ_fwd, 1 - occ_bwd], dim=1)
         w = conf / (conf.sum(dim=1, keepdim=True) + 1e-6)

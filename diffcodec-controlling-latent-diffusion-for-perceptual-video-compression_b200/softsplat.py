@@ -15,6 +15,9 @@ There is no CPU path (the reference has none either, ``softsplat.py:347-348``) a
 Extensions over the reference (all opt-in, defaults reproduce the reference):
   * bfloat16 tensors (the reference asserts on them, ``softsplat.py:105-107``): inputs bf16,
     positions / weights / accumulation fp32, one rounding at the output;
+  * float16 tensors (the reference's kernel names ``half`` but cannot compile it): the same rule
+    as bf16 -- loads widened to fp32, fp32 arithmetic, one ``__float2half_rn`` at each store; a
+    value beyond the fp16 range becomes +-inf, as a torch fp16 op gives;
   * ``deterministic(True)``: bit-reproducible sort-then-reduce forward.
 """
 from __future__ import annotations
@@ -64,8 +67,8 @@ def _check_inputs(tenIn, tenFlow):
 
 
 def _match_flow(tenIn, tenFlow):
-    # the reference compiles ONE element type into the kernel; a bf16 tensor may keep an fp32 flow
-    if tenFlow.dtype == tenIn.dtype or (tenIn.dtype == torch.bfloat16 and tenFlow.dtype == torch.float32):
+    # the reference compiles ONE element type into the kernel; a bf16 / fp16 tensor may keep an fp32 flow
+    if tenFlow.dtype == tenIn.dtype or (tenIn.dtype in (torch.bfloat16, torch.float16) and tenFlow.dtype == torch.float32):
         return tenFlow
     return tenFlow.to(tenIn.dtype)
 
@@ -81,7 +84,7 @@ def _forward(tenIn, tenFlow, tenMetric, mask, mode: int, eps: int, det: bool, wa
     flags = _lib.FLAG_DETERMINISTIC if det else 0
     dt = _lib._DTYPES.get(tenIn.dtype)
     if dt is None:
-        raise ValueError(f"softsplat: unsupported dtype {tenIn.dtype} (float32, bfloat16, float64)")
+        raise ValueError(f"softsplat: unsupported dtype {tenIn.dtype} (float32, bfloat16, float16, float64)")
     key = (n, c, h, w, dt, mode, flags)
     need = _ws_sizes.get(key)
     if need is None:

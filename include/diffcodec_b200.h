@@ -35,7 +35,10 @@ extern "C" {
 
 /* element types */
 enum { DCB_F32 = 0, DCB_BF16 = 1, DCB_F64 = 2,
-       DCB_U8 = 3, DCB_F16 = 4 /* storage types of dcb_convert only (host-buffer path); the splat kernels take the first three */ };
+       DCB_U8 = 3 /* storage type of dcb_convert only (host-buffer path) */,
+       DCB_F16 = 4 /* IEEE binary16: a tensor dtype wherever BF16 is one (same kernel family, group size and workspace;
+                      loads widened to fp32, each store rounded once). Refused (DCB_E_DTYPE) by dcb_backwarp_*,
+                      dcb_occlusion_mask, dcb_residual_fused, dcb_residual_bidir and dcb_flow_resize */ };
 
 /* splat modes: controlnet/softsplat.py:232-274 (strMode.split('-')[0]) */
 enum { DCB_MODE_SUM = 0, DCB_MODE_AVG = 1, DCB_MODE_LINEAR = 2, DCB_MODE_SOFT = 3 };
@@ -78,7 +81,7 @@ enum {
 /* 4-d NCHW-indexed view with arbitrary element strides. */
 typedef struct DcbTensor {
     void* ptr;
-    int32_t dtype;     /* DCB_F32 / DCB_BF16 / DCB_F64 */
+    int32_t dtype;     /* DCB_F32 / DCB_BF16 / DCB_F16 / DCB_F64 */
     int32_t reserved;
     int64_t size[4];   /* N, C, H, W */
     int64_t stride[4]; /* in elements */
@@ -116,7 +119,7 @@ int32_t dcb_splat_fwd_workspace_is_scratch(int64_t N, int64_t C, int64_t H, int6
 /*
  * Tuning / test knobs (process-wide, not thread-safe against concurrent calls; defaults are what ships):
  *   "fwd_path"          0 automatic | 1 round-1 accumulator pipeline (red.global into L2-resident cells)
- *                       | 2 target-tile owner kernels wherever they apply
+ *                       | 2 target-tile owner kernels wherever they apply (F32 / BF16 only: F16 stays on the pipelines)
  *   "pipe_group_bytes"  accumulator bytes per ring slot of the accumulator pipelines (tests shrink it so that
  *                       small tensors run through many ring groups); 0 restores the default
  *   "pipe_ring_slots"   1 (default) one accumulator slot, scatter and normalise of a frame group in alternating
@@ -126,7 +129,7 @@ int32_t dcb_splat_fwd_workspace_is_scratch(int64_t N, int64_t C, int64_t H, int6
  *   "bwd_group_bytes"   packed-cell bytes per frame group of the packed backward; 0 = one group
  *   "planar_one_launch" 0 (default) two chained launches | 1 a many-channel call whose frames fit one group and whose warps
  *                       are all resident at once (latents, small feature maps) runs as ONE launch with a grid barrier
- *                       (measured slower on B200: 20.6-22.2 us against 16.4 us for C2 under graph replay)
+ *                       (measured slower on B200: 20.6-22.2 us against 16.4 us for C2 under graph replay); F32 / BF16 only
  *   "bwd_flat"          1 (default) contiguous frames take the compile-time (C, mode) form of the packed backward | 0 never
  *   "lists_nhwc"        1 (default) channels-last many-channel tensors take the channel-quad gather | 0 the NCHW gather
  * Returns DCB_OK, or DCB_E_MODE for an unknown name. There is no equivalent in the reference (its kernels are
@@ -141,11 +144,11 @@ int dcb_set_option(const char* name, int64_t value);
  * softsplat_func.apply(tenIn, tenFlow).
  *
  *   in      [N,C,H,W]  any strides
- *   flow    [N,2,H,W]  any strides; same dtype as `in`, or F32 when `in` is BF16
+ *   flow    [N,2,H,W]  any strides; same dtype as `in`, or F32 when `in` is BF16 or F16
  *   metric  [N,1,H,W]  required for LINEAR/SOFT, must be NULL for SUM/AVG (softsplat.py:235-238)
  *   out     [N,C,H,W]  contiguous NCHW, same dtype as `in` (softsplat.py:281)
  *   norm    [N,1,H,W]  optional (may be NULL): receives the normaliser AFTER the eps rule, in the
- *                      accumulator type (F32 for F32/BF16 input, F64 for F64); dcb_splat_bwd needs it
+ *                      accumulator type (F32 for F32/BF16/F16 input, F64 for F64); dcb_splat_bwd needs it
  *   mask    [N,1,H,W]  optional: out is multiplied by (1 - mask) -- controlnet/control_utils.py:69-70
  */
 int dcb_splat_fwd(const DcbTensor* in, const DcbTensor* flow, const DcbTensor* metric,
@@ -160,7 +163,8 @@ int dcb_splat_fwd(const DcbTensor* in, const DcbTensor* flow, const DcbTensor* m
  * product. Any of grad_in / grad_flow / grad_metric may be NULL (needs_input_grad gating,
  * softsplat.py:364-365). With mode = DCB_MODE_SUM it is exactly softsplat_func.backward.
  *
- *   grad_out [N,C,H,W] any strides;  in/flow/metric/mask as given to the forward
+ *   grad_out [N,C,H,W] any strides (F16: at most 2^30 elements per plane, else DCB_E_LIMIT);  in/flow/metric/mask as
+ *   given to the forward
  *   out, norm: what the forward produced (ignored for SUM)
  *   grad_in [N,C,H,W], grad_flow [N,2,H,W], grad_metric [N,1,H,W]: contiguous, fully overwritten
  */
@@ -301,7 +305,7 @@ int dcb_bidir_block_bwd(const DcbTensor* grad_fused, const DcbTensor* first, con
  * soft_fuse with identity masks, cell 3: no occlusion test, no (1 - mask), no holes).
  *
  *   levels[l].first, last [N,C,H,W]; flow_f, flow_b [N,2,H,W] at the level's resolution; metric_f, metric_b [N,1,H,W]
- *   or NULL = all-ones (never materialised); one dtype (F32 or BF16) for all tensors of all levels
+ *   or NULL = all-ones (never materialised); one dtype (F32, BF16 or F16) for all tensors of all levels
  *   outputs are raw device pointers to NCHW-contiguous buffers of the level's shape and dtype (norm_*: F32):
  *   fused (required); warped_*, norm_*, occ_* optional (NULL = never stored; dcb_bidir_pyramid_bwd needs all six)
  *   n_levels <= 4;  workspace: dcb_bidir_pyramid_workspace_bytes(), DCB_FLAG_WS_CLEAN protocol as dcb_splat_fwd
@@ -324,7 +328,7 @@ int dcb_bidir_pyramid_fwd(const DcbPyramidLevel* levels, int32_t n_levels, void*
  * confidences). The occlusion masks carry no gradient (compute_mask thresholds). No atomics: bit-identical run to run.
  *
  *   grad_fused [N,C,H,W] any strides; first, last, flow_f, flow_b, metric_f, metric_b as given to the forward (a NULL metric
- *   is the all-ones metric); one dtype (F32 or BF16) for all tensors of all levels
+ *   is the all-ones metric); one dtype (F32, BF16 or F16) for all tensors of all levels
  *   warped_*, norm_* (F32), occ_*: what the forward stored for the level (raw pointers, NCHW-contiguous), all six required
  *   grad_*: raw pointers to NCHW-contiguous buffers of the level's dtype, or NULL (not computed); fully overwritten.
  *   grad_metric_* must be NULL where the metric is NULL.
@@ -341,8 +345,8 @@ int dcb_bidir_pyramid_bwd(const DcbPyramidBwdLevel* levels, int32_t n_levels, vo
                           int32_t flags, void* stream);
 
 /*
- * Batched bilinear resampling: every (tensor, scale) pair of a pyramid in ONE launch. dst[j] [N,C,th,tw] (contiguous, F32
- * or BF16) = bilinear(src[j] [N,C,H,W], any strides), then channel 0 (op) factor0 and every other channel (op) factor1.
+ * Batched bilinear resampling: every (tensor, scale) pair of a pyramid in ONE launch. dst[j] [N,C,th,tw] (contiguous, F32,
+ * BF16 or F16; src and dst in any mix) = bilinear(src[j] [N,C,H,W], any strides), then channel 0 (op) factor0 and every other channel (op) factor1.
  * The index and weight arithmetic is torch's upsample_bilinear2d (fp32, same operation order). Replaces the
  * F.interpolate calls in front of the splats: resize_and_normalize_flow_batched (controlnet/control_utils.py:74-97:
  * align_corners = 0, DIV by ((tw - 1) / 2, (th - 1) / 2)), extractors.py:182-183 (align_corners = 0, DIV by H // res),
@@ -367,7 +371,7 @@ int dcb_resample_batch(const DcbResampleJob* jobs, int32_t n_jobs, void* stream)
  *   merged = out / max(weight, eps).
  * tiles: array of n_tiles descriptors, each [1,C,th,tw] (any strides, dtype of `out`);
  * pixel_coords: n_tiles * 4 int64; out [N,C,H,W] contiguous (N > 1 receives N copies, like the
- * reference's broadcast); F32 or BF16. Tiles whose rectangle is empty are skipped. Lists longer than
+ * reference's broadcast); F32, BF16 or F16. Tiles whose rectangle is empty are skipped. Lists longer than
  * 48 tiles need a workspace (dcb_tile_merge_workspace_bytes), shorter ones none.
  */
 int64_t dcb_tile_merge_workspace_bytes(int64_t C, int64_t H, int64_t W, int32_t n_tiles);
