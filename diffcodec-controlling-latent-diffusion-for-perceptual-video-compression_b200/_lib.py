@@ -82,6 +82,7 @@ SYMBOLS = {
     "dcb_bidir_block_bwd": (ctypes.c_int, [_P] * 17 + [ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p]),
     "dcb_flow_resize": (ctypes.c_int, [_P, _P, ctypes.c_int32, ctypes.c_void_p]),
     "dcb_bidir_pyramid_workspace_bytes": (ctypes.c_int64, [ctypes.c_void_p, ctypes.c_int32]),
+    "dcb_bidir_pyramid_det_workspace_bytes": (ctypes.c_int64, [ctypes.c_void_p, ctypes.c_int32]),
     "dcb_bidir_pyramid_fwd": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int32, ctypes.c_void_p, ctypes.c_int64, ctypes.c_int32, ctypes.c_void_p]),
     "dcb_bidir_pyramid_bwd_workspace_bytes": (ctypes.c_int64, [ctypes.c_void_p, ctypes.c_int32]),
     "dcb_bidir_pyramid_bwd": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int32, ctypes.c_void_p, ctypes.c_int64, ctypes.c_int32, ctypes.c_void_p]),

@@ -71,6 +71,8 @@ int bidir_block_bwd_impl(const DcbTensor*, const DcbTensor*, const DcbTensor*, c
                          cudaStream_t);
 int flow_ingest_impl(const DcbTensor* flow, const DcbTensor* out, int mode, cudaStream_t st);
 long long pyramid_workspace(const DcbPyramidLevel* lv, int n);
+long long pyramid_det_workspace(const DcbPyramidLevel* lv, int n);
+long long pyramid_det_keys(const DcbPyramidLevel* lv, int n);
 int bidir_pyramid_fwd_impl(const DcbPyramidLevel* lv, int n, void* ws, int flags, cudaStream_t st);
 long long pyramid_bwd_workspace(const DcbPyramidBwdLevel* lv, int n);
 int bidir_pyramid_bwd_impl(const DcbPyramidBwdLevel* lv, int n, void* ws, bool holes, cudaStream_t st);
@@ -170,7 +172,7 @@ const char* dcb_build_info(void) {
     return "libdiffcodec_b200 " __DATE__ " nvcc " DCB_STR(__CUDACC_VER_MAJOR__) "." DCB_STR(__CUDACC_VER_MINOR__)
            " target sm_100a; kernels: k_splat_step k_planar_step k_list_count k_list_alloc k_list_fill k_list_gather k_scatter_planar k_normalize k_bwd_target k_bwd_source "
            "k_backwarp_rows k_backwarp_fwd k_backwarp_bwd k_cast_f32_bf16 k_recipe_fuse k_bidir_fuse_fwd k_bidir_fuse_bwd "
-           "k_det_emit k_det_reduce k_tile_merge k_splat_owner k_strip_box k_convert k_flow_ingest k_pyr_scatter k_pyr_fuse k_resample_batch k_splat_cluster";
+           "k_det_emit k_det_reduce k_tile_merge k_splat_owner k_strip_box k_convert k_flow_ingest k_pyr_scatter k_pyr_fuse k_pyr_det_emit k_pyr_det_reduce k_resample_batch k_splat_cluster";
 }
 
 int64_t dcb_splat_fwd_workspace_bytes(int64_t N, int64_t C, int64_t H, int64_t W, int32_t dtype, int32_t mode, int32_t flags) {
@@ -658,12 +660,29 @@ int64_t dcb_bidir_pyramid_workspace_bytes(const DcbPyramidLevel* levels, int32_t
     return (int64_t)pyramid_workspace(levels, n_levels);
 }
 
+int64_t dcb_bidir_pyramid_det_workspace_bytes(const DcbPyramidLevel* levels, int32_t n_levels) {
+    if (!levels || n_levels <= 0 || n_levels > 4) return 0;
+    for (int l = 0; l < n_levels; ++l)
+        if (!levels[l].first) return 0;
+    return (int64_t)pyramid_det_workspace(levels, n_levels);
+}
+
 int dcb_bidir_pyramid_fwd(const DcbPyramidLevel* levels, int32_t n_levels, void* ws, int64_t ws_bytes, int32_t flags, void* stream) {
     const char* fn = "dcb_bidir_pyramid_fwd";
-    if (flags & ~(DCB_FLAG_WS_CLEAN | DCB_PYRAMID_NO_MASKS | DCB_PYRAMID_NO_HOLES)) return set_error(DCB_E_MODE, "%s: unknown flags 0x%x", fn, flags);
+    if (flags & ~(DCB_FLAG_DETERMINISTIC | DCB_FLAG_WS_CLEAN | DCB_PYRAMID_NO_MASKS | DCB_PYRAMID_NO_HOLES))
+        return set_error(DCB_E_MODE, "%s: unknown flags 0x%x", fn, flags);
+    const bool det = (flags & DCB_FLAG_DETERMINISTIC) != 0;
+    if (det && (flags & DCB_FLAG_WS_CLEAN))
+        return set_error(DCB_E_MODE, "%s: DCB_FLAG_DETERMINISTIC takes a scratch workspace, not DCB_FLAG_WS_CLEAN", fn);
     TRY(check_pyramid(fn, levels, n_levels));
     if (n_levels == 0) return DCB_OK;
-    const long long need = pyramid_workspace(levels, n_levels);
+    if (det) {
+        const long long nkeys = pyramid_det_keys(levels, n_levels);
+        if (nkeys >= (1ll << 31))
+            return set_error(DCB_E_LIMIT, "%s(deterministic): 4 x the pixels of all levels and directions must stay below 2^31 (got %lld)",
+                             fn, nkeys);
+    }
+    const long long need = det ? pyramid_det_workspace(levels, n_levels) : pyramid_workspace(levels, n_levels);
     if (need > 0 && (!ws || ws_bytes < need || ((uintptr_t)ws & 255)))
         return set_error(DCB_E_WORKSPACE, "%s: workspace of %lld bytes (256 B aligned) required, got %lld", fn, need, (long long)ws_bytes);
     return bidir_pyramid_fwd_impl(levels, n_levels, ws, flags, (cudaStream_t)stream);

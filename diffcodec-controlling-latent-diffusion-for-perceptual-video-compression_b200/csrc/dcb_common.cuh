@@ -225,6 +225,16 @@ template <class A> struct Foot {
     bool finite;
 };
 
+// One contribution of the deterministic splat (det.cu, and the deterministic pyramid in pyramid.cu): the pre-multiplied value
+// v times the corner weight w, rounded, added to the running sum that starts from +0 and walks the sources in ascending order.
+template <class A> __device__ __forceinline__ A det_add(A sum, A v, A w) { return add_rn(sum, mul_rn(v, w)); }
+
+// det.cu: the one radix sort of the deterministic paths. Keys reach maxkey = total * span (the sentinel of invalid corners).
+int key_bits(long long total, long long span);
+size_t cub_temp_bytes(long long nkeys, int end_bit);
+int det_sort_keys(void* temp, size_t temp_bytes, const unsigned long long* keys, unsigned long long* sorted, long long nkeys,
+                  int end_bit, cudaStream_t st);
+
 template <class A> __device__ __forceinline__ Foot<A> make_foot(int x, int y, A flow_x, A flow_y) {
     Foot<A> f;
     f.fx = add_rn((A)x, flow_x);

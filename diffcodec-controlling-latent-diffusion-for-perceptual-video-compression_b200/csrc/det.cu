@@ -98,7 +98,7 @@ __global__ void __launch_bounds__(256) k_det_reduce(const DetArgs a) {
                     } else {
                         v = g;
                     }
-                    sum[i] = add_rn(sum[i], mul_rn(v, w));
+                    sum[i] = det_add(sum[i], v, w);
                 }
             }
         }
@@ -108,7 +108,7 @@ __global__ void __launch_bounds__(256) k_det_reduce(const DetArgs a) {
     }
 }
 
-static size_t cub_temp_bytes(long long nkeys, int end_bit) {
+size_t cub_temp_bytes(long long nkeys, int end_bit) {
     size_t bytes = 0;
     const cudaError_t e = cub::DeviceRadixSort::SortKeys(nullptr, bytes, (const unsigned long long*)nullptr,
                                                          (unsigned long long*)nullptr, (int)nkeys, 0, end_bit);
@@ -119,12 +119,19 @@ static size_t cub_temp_bytes(long long nkeys, int end_bit) {
     return bytes;
 }
 
-static int key_bits(long long total, long long HW) {
-    // keys go up to total*HW (the "invalid" key) inclusive
-    const unsigned long long maxkey = (unsigned long long)total * (unsigned long long)HW;
+int key_bits(long long total, long long span) {
+    // keys go up to total*span (the "invalid" key) inclusive
+    const unsigned long long maxkey = (unsigned long long)total * (unsigned long long)span;
     int bits = 1;
     while (bits < 64 && (maxkey >> bits) != 0) ++bits;
     return bits;
+}
+
+int det_sort_keys(void* temp, size_t temp_bytes, const unsigned long long* keys, unsigned long long* sorted, long long nkeys,
+                  int end_bit, cudaStream_t st) {
+    DCB_CHECK_CUDA(cub::DeviceRadixSort::SortKeys(temp, temp_bytes, keys, sorted, (int)nkeys, 0, end_bit, st));
+    count_launch(8);   // histogram + onesweep passes (library kernels)
+    return DCB_OK;
 }
 
 struct DetLayout {
@@ -159,11 +166,9 @@ static int launch_det(DetArgs& a, const DetLayout& L, char* ws, cudaStream_t st)
     const unsigned blocks = (a.total + 255) / 256;
     k_det_emit<T, TF><<<blocks, 256, 0, st>>>(a);
     DCB_CHECK_LAUNCH("k_det_emit");
-    size_t temp = L.temp_bytes;
-    DCB_CHECK_CUDA(cub::DeviceRadixSort::SortKeys(ws + L.temp_off, temp, (const unsigned long long*)a.keys,
-                                                  (unsigned long long*)a.sorted, (int)a.nkeys, 0,
-                                                  key_bits(a.total, a.HW), st));
-    count_launch(8);   // histogram + onesweep passes (library kernels)
+    const int rc = det_sort_keys(ws + L.temp_off, L.temp_bytes, a.keys, (unsigned long long*)a.sorted, a.nkeys,
+                                 key_bits(a.total, a.HW), st);
+    if (rc != DCB_OK) return rc;
     k_det_reduce<T, TF, 4><<<blocks, 256, 0, st>>>(a);
     DCB_CHECK_LAUNCH("k_det_reduce");
     return DCB_OK;

@@ -24,6 +24,15 @@
 //                             caller asks for them (the backward does).
 //   one cudaMemsetAsync re-zeroes the per-pixel planes that several warps read (48 B per pixel); the channel-quad
 //   accumulators are re-zeroed by their only reader. The workspace follows the DCB_FLAG_WS_CLEAN protocol.
+//
+// DCB_FLAG_DETERMINISTIC replaces launch A by the sort-then-reduce of det.cu, over every splat of the pyramid at once:
+//   k_pyr_det_emit   : one key per (source, corner) of every footprint field (level x direction), see PyrDetField
+//   sort             : ONE cub::DeviceRadixSort over all keys (det_sort_keys, det.cu)
+//   k_pyr_det_reduce : per (target, channel quad) the contributions in ascending source order, with k_det_reduce's
+//                      arithmetic (det_add), written into the cells launch B reads
+//   k_pyr_fuse<T, 1> : launch B dividing as k_normalize does; nothing is re-zeroed, the workspace is plain scratch.
+// The outputs are then bit-identical, run to run, to the composition of deterministic single ops (compute_mask, the masked
+// soft splat, bidir_fuse) in fp32.
 #include "splat_planar.cuh"
 
 namespace dcb {
@@ -190,7 +199,9 @@ struct PyrFuseArgs {
     int holes;               // 0: no double-hole fill (DCB_PYRAMID_NO_HOLES; extractors.py:193-199)
 };
 
-template <class T>
+// DET: the cells come from k_pyr_det_reduce. The division and the (1 - mask) product are those of k_normalize (o = S / d,
+// then o * (1 - mask), one rounding to T), and the cells are plain scratch: nothing is re-zeroed.
+template <class T, bool DET>
 __global__ void __launch_bounds__(32, 16) k_pyr_fuse(const __grid_constant__ PyrFuseArgs a) {
     pdl_wait();
     int l = 0;
@@ -206,11 +217,13 @@ __global__ void __launch_bounds__(32, 16) k_pyr_fuse(const __grid_constant__ Pyr
     const unsigned base = chunk * kPChunk + lane;
     const size_t fpix = (size_t)fi * L.HW;
     float sf[kPer], sb[kPer], w0[kPer], w1[kPer];
+    float kf[kPer], kb[kPer];                        // DET: the (1 - mask) factors
     bool hole[kPer];
 #pragma unroll
     for (int i = 0; i < kPer; ++i) {
         const unsigned r = base + i * 32;
         sf[i] = sb[i] = w0[i] = w1[i] = 0.f; hole[i] = false;
+        if constexpr (DET) kf[i] = kb[i] = 1.f;
         if (r >= L.HW) continue;
         const int y = (int)(r / (unsigned)L.W), x = (int)(r - (unsigned)y * (unsigned)L.W);
         float of = 0.f, ob = 0.f;
@@ -225,8 +238,13 @@ __global__ void __launch_bounds__(32, 16) k_pyr_fuse(const __grid_constant__ Pyr
         }
         // normalisers of both feature splats: softsplat.py:256-258 ('soft' = add 1e-7), one reciprocal per pixel
         const float df = add_rn(__ldcg(L.dacc_f + fpix + r), 0.0000001f), db = add_rn(__ldcg(L.dacc_b + fpix + r), 0.0000001f);
-        sf[i] = __frcp_rn(df); sb[i] = __frcp_rn(db);
-        if (a.masks) { sf[i] = mul_rn(sf[i], sub_rn(1.f, of)); sb[i] = mul_rn(sb[i], sub_rn(1.f, ob)); }   // control_utils.py:69-70
+        if constexpr (DET) {
+            sf[i] = df; sb[i] = db;
+            if (a.masks) { kf[i] = sub_rn(1.f, of); kb[i] = sub_rn(1.f, ob); }
+        } else {
+            sf[i] = __frcp_rn(df); sb[i] = __frcp_rn(db);
+            if (a.masks) { sf[i] = mul_rn(sf[i], sub_rn(1.f, of)); sb[i] = mul_rn(sb[i], sub_rn(1.f, ob)); }   // control_utils.py:69-70
+        }
         // confidences = the warpers' metrics (extractors.py:298-303)
         float ca = 1.f, cb = 1.f;
         if (L.metric_f.p) ca = ld<float>((const T*)L.metric_f.p + fi * L.metric_f.sN + (long long)y * L.metric_f.sH + (long long)x * L.metric_f.sW);
@@ -262,21 +280,135 @@ __global__ void __launch_bounds__(32, 16) k_pyr_fuse(const __grid_constant__ Pyr
         for (int i = 0; i < kPer; ++i) {
             const unsigned r = base + i * 32;
             if (r >= L.HW) continue;
-            __stcg(pf + r, make_float4(0.f, 0.f, 0.f, 0.f));
-            __stcg(pb + r, make_float4(0.f, 0.f, 0.f, 0.f));
+            if constexpr (!DET) {
+                __stcg(pf + r, make_float4(0.f, 0.f, 0.f, 0.f));
+                __stcg(pb + r, make_float4(0.f, 0.f, 0.f, 0.f));
+            }
             const float af[4] = {vf[i].x, vf[i].y, vf[i].z, vf[i].w}, ab[4] = {vb[i].x, vb[i].y, vb[i].z, vb[i].w};
 #pragma unroll
             for (int jj = 0; jj < 4; ++jj) {
                 const int c = 4 * qq + jj;
                 if (c >= C) break;
                 // the warped maps as the unfused path stores them (rounded to T), then extractors.py:303-310
-                const float A = round_as<T>(mul_rn(af[jj], sf[i])), B = round_as<T>(mul_rn(ab[jj], sb[i]));
+                float A, B;
+                if constexpr (DET) {
+                    A = af[jj] / sf[i]; B = ab[jj] / sb[i];
+                    if (a.masks) { A = mul_rn(A, kf[i]); B = mul_rn(B, kb[i]); }
+                    A = round_as<T>(A); B = round_as<T>(B);
+                } else {
+                    A = round_as<T>(mul_rn(af[jj], sf[i])); B = round_as<T>(mul_rn(ab[jj], sb[i]));
+                }
                 const float v = hole[i] ? mul_rn(0.5f, add_rn(A, B)) : add_rn(mul_rn(w0[i], A), mul_rn(w1[i], B));
                 st_stream(fo + (size_t)c * L.HW + r, v);
                 if (wf) st_stream(wf + (size_t)c * L.HW + r, A);
                 if (wb) st_stream(wb + (size_t)c * L.HW + r, B);
             }
         }
+    }
+}
+
+// ---------------------------------------------------------------------------------------------
+// DCB_FLAG_DETERMINISTIC: emit + sort + reduce in place of launch A
+// ---------------------------------------------------------------------------------------------
+// A footprint field is one (level, direction): every source pixel of every frame of the level, landing where its flow
+// (flow_f forward, flow_b backward) takes it. The feature splat of the direction (first by flow_f, last by flow_b) and the
+// mask splat by the same flow (flow_b by flow_f behind occ_b, flow_f by flow_b behind occ_f) land on the same footprints, so
+// they share one key set. The targets of all fields are numbered one after the other (global target); a key is
+// global_target << s | source_in_frame with 2^s >= the largest H*W, so within a target the keys ascend with the source index:
+// the order of k_det_reduce (key = target * HW + source).
+struct PyrDetField {
+    View flow, in, metric, mflow;    // footprint flow; feature input, its metric (NULL: all-ones); the mask splat's input
+    float *acc, *dacc;               // feature cells [N][Cq][HW] float4, normaliser [N][HW]
+    float *acc_m, *dacc_m;           // mask cells [N][HW] float4 (x, y, 0, 0), normaliser [N][HW]
+    int C, Cq, H, W;
+    unsigned HW, NHW;
+    unsigned src0, tgt0;             // first source (emit thread, key group of 4) and first global target of the field
+    long long item0;                 // first reduce thread of the field: NHW * Cq threads, channel quad major
+};
+struct PyrDetArgs {
+    PyrDetField f[2 * kMaxLevels];
+    int n_fields, masks, s;
+    unsigned long long* keys;
+    const unsigned long long* sorted;
+    long long nkeys;
+    unsigned long long invalid;      // sorts behind every real key
+};
+
+template <class T>
+__global__ void __launch_bounds__(256) k_pyr_det_emit(const __grid_constant__ PyrDetArgs a) {
+    pdl_wait();
+    const unsigned p = blockIdx.x * 256 + threadIdx.x;
+    int j = 0;
+    while (j + 1 < a.n_fields && p >= a.f[j + 1].src0) ++j;
+    const PyrDetField& F = a.f[j];
+    const unsigned q = p - F.src0;
+    if (q >= F.NHW) return;
+    const unsigned n = q / F.HW, r = q - n * F.HW;
+    const int y = (int)(r / (unsigned)F.W), x = (int)(r - (unsigned)y * (unsigned)F.W);
+    const T* fp = (const T*)F.flow.p + n * F.flow.sN + (long long)y * F.flow.sH + (long long)x * F.flow.sW;
+    const Foot<float> f = make_foot<float>(x, y, ld<float>(fp), ld<float>(fp + F.flow.sC));
+    const int x1 = (int)((unsigned)f.x0 + 1u), y1 = (int)((unsigned)f.y0 + 1u);
+    const bool vx0 = (unsigned)f.x0 < (unsigned)F.W, vx1 = (unsigned)x1 < (unsigned)F.W;
+    const bool vy0 = (unsigned)f.y0 < (unsigned)F.H, vy1 = (unsigned)y1 < (unsigned)F.H;
+    const bool b[4] = {f.finite && vx0 && vy0, f.finite && vx1 && vy0, f.finite && vx0 && vy1, f.finite && vx1 && vy1};
+    const long long t0 = (long long)F.tgt0 + (long long)n * F.HW + (long long)f.y0 * F.W + f.x0;
+    const long long off[4] = {0, 1, F.W, (long long)F.W + 1};
+#pragma unroll
+    for (int k = 0; k < 4; ++k)
+        a.keys[4ull * p + k] = b[k] ? ((unsigned long long)(t0 + off[k]) << a.s) | r : a.invalid;
+}
+
+template <class T>
+__global__ void __launch_bounds__(256) k_pyr_det_reduce(const __grid_constant__ PyrDetArgs a) {
+    pdl_wait();
+    const long long i = (long long)blockIdx.x * 256 + threadIdx.x;
+    int j = 0;
+    while (j + 1 < a.n_fields && i >= a.f[j + 1].item0) ++j;
+    const PyrDetField& F = a.f[j];
+    const long long it = i - F.item0;
+    if (it >= (long long)F.NHW * F.Cq) return;
+    const unsigned qd = (unsigned)(it / F.NHW), t = (unsigned)(it - (long long)qd * F.NHW);   // channel quad, target
+    const unsigned n = t / F.HW, r = t - n * F.HW;
+    const int ty = (int)(r / (unsigned)F.W), tx = (int)(r - (unsigned)ty * (unsigned)F.W);
+    const unsigned long long lo_key = (unsigned long long)(F.tgt0 + t) << a.s, hi_key = lo_key + (1ull << a.s);
+    long long lo = 0, hi = a.nkeys;                       // lower_bound(lo_key)
+    while (lo < hi) {
+        const long long mid = (lo + hi) >> 1;
+        if (a.sorted[mid] < lo_key) lo = mid + 1; else hi = mid;
+    }
+    const bool cells = qd == 0;                           // quad 0 also owns the normalisers and the mask cells
+    const bool masks = cells && a.masks;
+    const float g1 = exp_det_t(1.f);                      // the all-ones metric of compute_mask and of a NULL metric
+    const int c0 = 4 * (int)qd;
+    float sum[4] = {0.f, 0.f, 0.f, 0.f}, d = 0.f, mx = 0.f, my = 0.f, dm = 0.f;
+    for (long long k = lo; k < a.nkeys; ++k) {
+        const unsigned long long key = a.sorted[k];
+        if (key >= hi_key) break;
+        const unsigned src = (unsigned)(key - lo_key);
+        const int y = (int)(src / (unsigned)F.W), x = (int)(src - (unsigned)y * (unsigned)F.W);
+        const T* fp = (const T*)F.flow.p + n * F.flow.sN + (long long)y * F.flow.sH + (long long)x * F.flow.sW;
+        const Foot<float> f = make_foot<float>(x, y, ld<float>(fp), ld<float>(fp + F.flow.sC));
+        const int kx = tx - f.x0, ky = ty - f.y0;         // which of the source's corners this target is: 0 or 1 each
+        const float w = ky == 0 ? (kx == 0 ? f.wnw : f.wne) : (kx == 0 ? f.wsw : f.wse);
+        float g = g1;
+        if (F.metric.p) g = exp_det_t(ld<float>((const T*)F.metric.p + n * F.metric.sN + (long long)y * F.metric.sH + (long long)x * F.metric.sW));
+        const T* ip = (const T*)F.in.p + n * F.in.sN + (long long)y * F.in.sH + (long long)x * F.in.sW + (long long)c0 * F.in.sC;
+#pragma unroll
+        for (int jj = 0; jj < 4; ++jj)
+            if (c0 + jj < F.C) sum[jj] = det_add(sum[jj], mul_rn(ld<float>(ip + jj * F.in.sC), g), w);
+        if (cells) d = det_add(d, g, w);
+        if (masks) {
+            const T* mp = (const T*)F.mflow.p + n * F.mflow.sN + (long long)y * F.mflow.sH + (long long)x * F.mflow.sW;
+            mx = det_add(mx, mul_rn(ld<float>(mp), g1), w);
+            my = det_add(my, mul_rn(ld<float>(mp + F.mflow.sC), g1), w);
+            dm = det_add(dm, g1, w);
+        }
+    }
+    ((float4*)F.acc)[((size_t)n * F.Cq + qd) * F.HW + r] = make_float4(sum[0], sum[1], sum[2], sum[3]);
+    if (cells) F.dacc[t] = d;
+    if (masks) {
+        ((float4*)F.acc_m)[t] = make_float4(mx, my, 0.f, 0.f);
+        F.dacc_m[t] = dm;
     }
 }
 
@@ -306,29 +438,89 @@ static void split_quads(long long items, int quads, int* cg, int* ncg) {
     *ncg = (quads + *cg - 1) / *cg;
 }
 
+// deterministic workspace: keys | sorted keys | cub temp | the cells of pyramid_workspace()
+struct PyrDetLayout {
+    long long nsrc, nkeys, sorted_off, temp_off, cells_off, total_bytes;
+    size_t temp_bytes;
+    int s, end_bit;
+};
+
+static PyrDetLayout pyr_det_layout(const DcbPyramidLevel* lv, int n) {
+    PyrDetLayout L;
+    long long nhw = 0, max_hw = 1;
+    for (int l = 0; l < n; ++l) {
+        const DcbTensor* f = lv[l].first;
+        if (!f || f->size[0] * f->size[1] * f->size[2] * f->size[3] <= 0) continue;
+        nhw += f->size[0] * f->size[2] * f->size[3];
+        if (f->size[2] * f->size[3] > max_hw) max_hw = f->size[2] * f->size[3];
+    }
+    L.nsrc = 2 * nhw;                                  // two footprint fields per level; as many targets as sources
+    L.nkeys = 4 * L.nsrc;
+    L.s = 0;
+    while ((1ll << L.s) < max_hw) ++L.s;
+    L.end_bit = key_bits(L.nsrc, 1ll << L.s);
+    L.temp_bytes = L.nkeys > 0 && L.nkeys < (1ll << 31) ? cub_temp_bytes(L.nkeys, L.end_bit) : 0;
+    L.sorted_off = align_up(L.nkeys * 8, 256);
+    L.temp_off = L.sorted_off + align_up(L.nkeys * 8, 256);
+    L.cells_off = L.temp_off + align_up((long long)L.temp_bytes, 256);
+    L.total_bytes = L.cells_off + pyramid_workspace(lv, n);
+    return L;
+}
+
+long long pyramid_det_keys(const DcbPyramidLevel* lv, int n) { return pyr_det_layout(lv, n).nkeys; }
+long long pyramid_det_workspace(const DcbPyramidLevel* lv, int n) { return pyr_det_layout(lv, n).total_bytes; }
+
 template <class T>
 static int launch_pyramid(const PyrScatterArgs& sa, unsigned s_items, const PyrFuseArgs& fa, unsigned f_items, cudaStream_t st) {
     DCB_CHECK_CUDA(launch_pdl(k_pyr_scatter<T>, dim3(s_items), dim3(32), 0, st, sa));
     count_launch();
-    DCB_CHECK_CUDA(launch_pdl(k_pyr_fuse<T>, dim3(f_items), dim3(32), 0, st, fa));
+    DCB_CHECK_CUDA(launch_pdl(k_pyr_fuse<T, false>, dim3(f_items), dim3(32), 0, st, fa));
+    count_launch();
+    return DCB_OK;
+}
+
+template <class T>
+static int launch_pyramid_det(const PyrDetArgs& da, const PyrDetLayout& D, char* ws, long long r_items, const PyrFuseArgs& fa,
+                              unsigned f_items, cudaStream_t st) {
+    DCB_CHECK_CUDA(launch_pdl(k_pyr_det_emit<T>, dim3((unsigned)((D.nsrc + 255) / 256)), dim3(256), 0, st, da));
+    count_launch();
+    const int rc = det_sort_keys(ws + D.temp_off, D.temp_bytes, da.keys, (unsigned long long*)da.sorted, D.nkeys, D.end_bit, st);
+    if (rc != DCB_OK) return rc;
+    DCB_CHECK_CUDA(launch_pdl(k_pyr_det_reduce<T>, dim3((unsigned)((r_items + 255) / 256)), dim3(256), 0, st, da));
+    count_launch();
+    DCB_CHECK_CUDA(launch_pdl(k_pyr_fuse<T, true>, dim3(f_items), dim3(32), 0, st, fa));
     count_launch();
     return DCB_OK;
 }
 
 // Preconditions (checked by the caller): 1 <= n <= kMaxLevels, all tensors of one dtype (F32 / BF16 / F16), shapes consistent,
-// ws holds pyramid_workspace() bytes, 256-byte aligned, all-zero if DCB_FLAG_WS_CLEAN.
+// ws holds pyramid_workspace() bytes, 256-byte aligned, all-zero if DCB_FLAG_WS_CLEAN; with DCB_FLAG_DETERMINISTIC (never with
+// WS_CLEAN) ws is plain scratch of pyramid_det_workspace() bytes and pyramid_det_keys() < 2^31.
 int bidir_pyramid_fwd_impl(const DcbPyramidLevel* lv, int n, void* ws, int flags, cudaStream_t st) {
-    PyrScatterArgs sa; PyrFuseArgs fa;
-    sa.n_jobs = 0; fa.n_levels = 0;
+    PyrScatterArgs sa; PyrFuseArgs fa; PyrDetArgs da;
+    sa.n_jobs = 0; fa.n_levels = 0; da.n_fields = 0;
     fa.masks = (flags & DCB_PYRAMID_NO_MASKS) ? 0 : 1;
     fa.holes = (flags & DCB_PYRAMID_NO_HOLES) ? 0 : 1;
+    const bool det = (flags & DCB_FLAG_DETERMINISTIC) != 0;
     long long shared_total = 0;
     for (int l = 0; l < n; ++l) shared_total += level_shared_bytes(lv[l].first->size[0], lv[l].first->size[2], lv[l].first->size[3]);
     const long long total = pyramid_workspace(lv, n);
-    if (!(flags & DCB_FLAG_WS_CLEAN)) DCB_CHECK_CUDA(cudaMemsetAsync(ws, 0, (size_t)total, st));
-    char* shared = (char*)ws;
-    char* feat = (char*)ws + shared_total;
-    unsigned s_items = 0, f_items = 0;
+    PyrDetLayout D = {};
+    char* cells = (char*)ws;
+    if (det) {
+        D = pyr_det_layout(lv, n);
+        cells += D.cells_off;
+        da.masks = fa.masks; da.s = D.s; da.nkeys = D.nkeys;
+        da.keys = (unsigned long long*)ws;
+        da.sorted = (const unsigned long long*)((char*)ws + D.sorted_off);
+        da.invalid = (unsigned long long)D.nsrc << D.s;
+    } else if (!(flags & DCB_FLAG_WS_CLEAN)) {
+        DCB_CHECK_CUDA(cudaMemsetAsync(ws, 0, (size_t)total, st));
+    }
+    char* shared = cells;
+    char* feat = cells + shared_total;
+    unsigned s_items = 0, f_items = 0, d_src = 0, d_tgt = 0;
+    long long r_items = 0;
     const int dt = lv[0].first->dtype;
     for (int l = 0; l < n; ++l) {
         const DcbPyramidLevel& d = lv[l];
@@ -353,12 +545,27 @@ int bidir_pyramid_fwd_impl(const DcbPyramidLevel* lv, int n, void* ws, int flags
             b.item0 = s_items; b.items = (unsigned)(N * ts * b.ncg);
             s_items += b.items;
         };
-        if (fa.masks) {
-            add_job(d.flow_f, d.flow_b, nullptr, acc_mf, dacc_mf, 2);        // compute_mask(flow_f, flow_b)
-            add_job(d.flow_b, d.flow_f, nullptr, acc_mb, dacc_mb, 2);        // compute_mask(flow_b, flow_f)
+        auto add_field = [&](const DcbTensor* flow, const DcbTensor* in, const DcbTensor* metric, const DcbTensor* mflow, float* acc,
+                             float* dacc, float* acc_m, float* dacc_m) {
+            PyrDetField& F = da.f[da.n_fields++];
+            F.flow = make_view(flow); F.in = make_view(in); F.metric = make_view(metric); F.mflow = make_view(mflow);
+            F.acc = acc; F.dacc = dacc; F.acc_m = acc_m; F.dacc_m = dacc_m;
+            F.C = (int)C; F.Cq = (int)Cq; F.H = (int)H; F.W = (int)W;
+            F.HW = (unsigned)HW; F.NHW = (unsigned)(N * HW);
+            F.src0 = d_src; F.tgt0 = d_tgt; F.item0 = r_items;
+            d_src += F.NHW; d_tgt += F.NHW; r_items += (long long)F.NHW * F.Cq;
+        };
+        if (det) {
+            add_field(d.flow_f, d.first, d.metric_f, d.flow_b, acc_f, dacc_f, acc_mb, dacc_mb);   // compute_mask(flow_b, flow_f)
+            add_field(d.flow_b, d.last, d.metric_b, d.flow_f, acc_b, dacc_b, acc_mf, dacc_mf);    // compute_mask(flow_f, flow_b)
+        } else {
+            if (fa.masks) {
+                add_job(d.flow_f, d.flow_b, nullptr, acc_mf, dacc_mf, 2);        // compute_mask(flow_f, flow_b)
+                add_job(d.flow_b, d.flow_f, nullptr, acc_mb, dacc_mb, 2);        // compute_mask(flow_b, flow_f)
+            }
+            add_job(d.first, d.flow_f, d.metric_f, acc_f, dacc_f, C);
+            add_job(d.last, d.flow_b, d.metric_b, acc_b, dacc_b, C);
         }
-        add_job(d.first, d.flow_f, d.metric_f, acc_f, dacc_f, C);
-        add_job(d.last, d.flow_b, d.metric_b, acc_b, dacc_b, C);
         PyrLevel& L = fa.lv[fa.n_levels++];
         L.flow_f = make_view(d.flow_f); L.flow_b = make_view(d.flow_b);
         L.metric_f = make_view(d.metric_f); L.metric_b = make_view(d.metric_b);
@@ -374,6 +581,16 @@ int bidir_pyramid_fwd_impl(const DcbPyramidLevel* lv, int n, void* ws, int flags
     }
     if (fa.n_levels == 0) return DCB_OK;
     int rc;
+    if (det) {
+        if ((r_items + 255) / 256 >= (1ll << 31))
+            return set_error(DCB_E_LIMIT, "bidir_pyramid_fwd(deterministic): %lld (pixel, channel quad) cells exceed the grid", r_items);
+        switch (dt) {
+            case DCB_F32: return launch_pyramid_det<float>(da, D, (char*)ws, r_items, fa, f_items, st);
+            case DCB_BF16: return launch_pyramid_det<__nv_bfloat16>(da, D, (char*)ws, r_items, fa, f_items, st);
+            case DCB_F16: return launch_pyramid_det<__half>(da, D, (char*)ws, r_items, fa, f_items, st);
+            default: return set_error(DCB_E_DTYPE, "bidir_pyramid_fwd: unsupported dtype %d", dt);
+        }
+    }
     switch (dt) {
         case DCB_F32: rc = launch_pyramid<float>(sa, s_items, fa, f_items, st); break;
         case DCB_BF16: rc = launch_pyramid<__nv_bfloat16>(sa, s_items, fa, f_items, st); break;

@@ -19,6 +19,7 @@ import torch.nn.functional as F
 
 from . import _lib
 from .control_utils import FeatureWarperSoftsplat, compute_mask, resize_and_normalize_flow_batched, zero_module
+from .softsplat import is_deterministic
 
 __all__ = ["bidir_fuse", "bidirectional_warp_fuse", "bidirectional_block", "Bi_Dir_FeatureExtractor", "Bi_Dir_ResidueExtractor",
            "WarpExtractor", "ConvBlock"]
@@ -168,6 +169,8 @@ def bidirectional_block(first_features, last_features, flow_f, flow_b, metric_f=
         metric_f = torch.ones_like(flow_f[:, :1], dtype=dt)
     if metric_b is None:
         metric_b = torch.ones_like(flow_b[:, :1], dtype=dt)
+    if is_deterministic():                                     # the deterministic form of the block is the one-level pyramid
+        return bidirectional_pyramid([(first_features, last_features, flow_f, flow_b, metric_f, metric_b)])[0]
     needs_grad = torch.is_grad_enabled() and any(t.requires_grad for t in (first_features, last_features, flow_f, flow_b, metric_f, metric_b))
     if (not needs_grad and not torch.is_autocast_enabled("cuda") and dt in (torch.float32, torch.bfloat16, torch.float16)
             and last_features.dtype == dt and flow_f.dtype == dt and flow_b.dtype == dt and metric_f.dtype == dt and metric_b.dtype == dt):
@@ -202,7 +205,9 @@ _lib._option_hooks.append(_pyr_ws.clear)
 
 def _pyramid_forward(levels, flags, want_saved, want_warped=False):
     """levels: per scale (first, last, flow_f, flow_b, metric_f | None, metric_b | None), one dtype. One dcb_bidir_pyramid_fwd
-    call: two kernel launches for the whole pyramid. Returns (fused list, per-scale saved tensors or None)."""
+    call: two kernel launches for the whole pyramid, or under ``deterministic()`` the bit-reproducible sort-then-reduce form
+    (11 launches). Returns (fused list, per-scale saved tensors or None)."""
+    det = is_deterministic()
     lib = _lib.lib()
     dev, dt = levels[0][0].device, levels[0][0].dtype
     outs, fused, saved = [], [], []
@@ -225,13 +230,19 @@ def _pyramid_forward(levels, flags, want_saved, want_warped=False):
     stream = _lib.stream_ptr(dev)
     with _lib.on_device(dev):
         arr = _lib.pack_pyramid(levels, outs)
-        key = (tuple(tuple(lv[0].shape) for lv in levels), dt)
+        key = (tuple(tuple(lv[0].shape) for lv in levels), dt, det)
         need = _pyr_ws.get(key)
         if need is None:
-            need = _pyr_ws[key] = int(lib.dcb_bidir_pyramid_workspace_bytes(arr, len(levels)))
-        ws = _lib.workspace(dev, need, "acc", stream)
-        rc = lib.dcb_bidir_pyramid_fwd(arr, len(levels), ws.data_ptr(), ws.numel(), flags | _lib.FLAG_WS_CLEAN, stream)
-    if rc != 0:
+            query = lib.dcb_bidir_pyramid_det_workspace_bytes if det else lib.dcb_bidir_pyramid_workspace_bytes
+            need = _pyr_ws[key] = int(query(arr, len(levels)))
+        if det:
+            ws = _lib.workspace(dev, need, "scratch", stream)
+            flags |= _lib.FLAG_DETERMINISTIC
+        else:
+            ws = _lib.workspace(dev, need, "acc", stream)
+            flags |= _lib.FLAG_WS_CLEAN
+        rc = lib.dcb_bidir_pyramid_fwd(arr, len(levels), ws.data_ptr(), ws.numel(), flags, stream)
+    if rc != 0 and not det:
         _lib.invalidate_acc(dev)
     _lib.check(rc, "dcb_bidir_pyramid_fwd")
     return fused, saved
@@ -301,7 +312,8 @@ def bidirectional_pyramid(levels, holes=True):
     levels = [(first, last, flow_f, flow_b, metric_f | None, metric_b | None), ...] -> [fused, ...]. Two kernel launches
     for the whole pyramid each way, no host sync; gradients reach the features, the flows and the metrics (the occlusion
     masks carry none, as in the reference). ``holes=False``: the fusion without the double-hole fill, as
-    ``Bi_Dir_ResidueExtractor`` (``extractors.py:193-199``)."""
+    ``Bi_Dir_ResidueExtractor`` (``extractors.py:193-199``). Under ``deterministic()`` the forward is bit-reproducible (in
+    fp32 bit-identical to the composition of the deterministic single ops); the backward has no atomics either way."""
     levels = [tuple(lv) for lv in levels]
     if len(levels) > _PYRAMID_MAX_LEVELS:
         return bidirectional_pyramid(levels[:_PYRAMID_MAX_LEVELS], holes) + bidirectional_pyramid(levels[_PYRAMID_MAX_LEVELS:], holes)
@@ -343,7 +355,6 @@ def pyramid_conditioning(img1, img2, flow1, flow2, sizes=(128, 64, 32)):
 
 
 def _block_fusable(first, last, flow_f, flow_b):
-    from .softsplat import is_deterministic
     return first.is_cuda and first.shape == last.shape and first.dtype in (torch.float32, torch.bfloat16, torch.float16) and not is_deterministic()
 
 
@@ -425,8 +436,10 @@ class Bi_Dir_FeatureExtractor(nn.Module):
         last_features = self.last_pre_extractor(local_conditions[:, :3])
         flow_fwd, flow_bwd = flow[:, :2], flow[:, 2:]
         flow_res = (64, 32, 16, 8)                                               # extractors.py:278
-        from .softsplat import is_deterministic
-        whole = first_features.is_cuda and flow.dtype in (torch.float32, torch.bfloat16, torch.float16) and not is_deterministic()
+        # Under deterministic() only fp32 takes the pyramid: the 16-bit composition thresholds masks computed from 16-bit warps,
+        # and the deterministic bits it gives today are kept.
+        fp32 = flow.dtype == torch.float32 and first_features.dtype == torch.float32
+        whole = first_features.is_cuda and flow.dtype in (torch.float32, torch.bfloat16, torch.float16) and (fp32 or not is_deterministic())
         if not whole:                                                            # what the pyramid does not take: scale by scale
             outs = []
             for idx, res in enumerate(flow_res):
@@ -502,8 +515,8 @@ class Bi_Dir_ResidueExtractor(nn.Module):
             flow_f = self.flow_refiners[i](F.interpolate(flow_fwd, size=(res, res), mode="bilinear", align_corners=False) / factor)
             flow_b = self.flow_refiners[i](F.interpolate(flow_bwd, size=(res, res), mode="bilinear", align_corners=False) / factor)
             flows.append((flow_f, flow_b))
-        from .softsplat import is_deterministic
-        if not (prev_frame.is_cuda and flow_fwd.dtype in (torch.float32, torch.bfloat16, torch.float16) and not is_deterministic()):
+        fp32 = flows[0][0].dtype == torch.float32 and prev_feats[0].dtype == torch.float32     # deterministic(): as Bi_Dir_FeatureExtractor
+        if not (prev_frame.is_cuda and flow_fwd.dtype in (torch.float32, torch.bfloat16, torch.float16) and (fp32 or not is_deterministic())):
             outs = []                                                            # what the pyramid does not take: scale by scale
             for i, (flow_f, flow_b) in enumerate(flows):
                 occ_f, occ_b = compute_mask(flow_f, flow_b), compute_mask(flow_b, flow_f)

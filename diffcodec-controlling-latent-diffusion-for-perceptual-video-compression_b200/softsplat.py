@@ -46,7 +46,9 @@ def is_deterministic() -> bool:
 
 @contextlib.contextmanager
 def deterministic(enabled: bool = True):
-    """Within the block, forward splats use the bit-exact sort-then-reduce kernels."""
+    """Within the block, forward splats use the bit-exact sort-then-reduce kernels: ``softsplat``, ``compute_mask``, the
+    warpers, and the conditioning pyramids (``bidirectional_pyramid``, ``pyramid_conditioning``, ``bidirectional_block``, the
+    fp32 extractors), which keep their single library call in its deterministic form. The backward kernels use no atomics."""
     prev = is_deterministic()
     _state.det = bool(enabled)
     try:

@@ -311,6 +311,12 @@ int dcb_bidir_block_bwd(const DcbTensor* grad_fused, const DcbTensor* first, con
  *   n_levels <= 4;  workspace: dcb_bidir_pyramid_workspace_bytes(), DCB_FLAG_WS_CLEAN protocol as dcb_splat_fwd
  *   flags: DCB_PYRAMID_NO_MASKS, or DCB_PYRAMID_NO_HOLES: masks and (1 - mask) as usual, the fusion without the double-hole
  *   fill (Bi_Dir_ResidueExtractor, controlnet/extractors.py:193-199); NO_MASKS | NO_HOLES equals NO_MASKS
+ *   DCB_FLAG_DETERMINISTIC (with or without NO_MASKS / NO_HOLES): bit-reproducible. Every splat of every level is one
+ *   sort-then-reduce (emit, one radix sort, reduce; about 11 launches whatever the number of levels), in the order and with
+ *   the arithmetic of dcb_splat_fwd's deterministic mode; in F32 the outputs equal, bit for bit, the composition of the
+ *   deterministic single ops (soft splats of the flows for the masks, masked soft splats, dcb_bidir_fuse_fwd). The workspace is
+ *   plain scratch of dcb_bidir_pyramid_det_workspace_bytes() bytes (DCB_FLAG_WS_CLEAN with it: DCB_E_MODE); 4 x N*H*W summed
+ *   over levels and both directions must stay below 2^31 (else DCB_E_LIMIT). dcb_bidir_pyramid_bwd takes its saved outputs.
  */
 typedef struct DcbPyramidLevel {
     const DcbTensor *first, *last, *flow_f, *flow_b, *metric_f, *metric_b;
@@ -318,6 +324,8 @@ typedef struct DcbPyramidLevel {
 } DcbPyramidLevel;
 enum { DCB_PYRAMID_NO_MASKS = 4, DCB_PYRAMID_NO_HOLES = 8 /* flags of dcb_bidir_pyramid_fwd (NO_HOLES: also of _bwd) */ };
 int64_t dcb_bidir_pyramid_workspace_bytes(const DcbPyramidLevel* levels, int32_t n_levels);
+/* workspace of dcb_bidir_pyramid_fwd with DCB_FLAG_DETERMINISTIC: keys, sorted keys, the sort's temporary storage, the cells */
+int64_t dcb_bidir_pyramid_det_workspace_bytes(const DcbPyramidLevel* levels, int32_t n_levels);
 int dcb_bidir_pyramid_fwd(const DcbPyramidLevel* levels, int32_t n_levels, void* workspace, int64_t workspace_bytes,
                           int32_t flags, void* stream);
 
