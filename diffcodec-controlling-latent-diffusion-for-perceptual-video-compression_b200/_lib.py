@@ -72,6 +72,7 @@ SYMBOLS = {
     "dcb_occlusion_mask_workspace_bytes": (ctypes.c_int64, [ctypes.c_int64] * 3),
     "dcb_occlusion_mask": (ctypes.c_int, [_P] * 3 + [ctypes.c_void_p, ctypes.c_int64, ctypes.c_int32, ctypes.c_void_p]),
     "dcb_residual_workspace_bytes": (ctypes.c_int64, [ctypes.c_int64] * 4),
+    "dcb_residual_det_workspace_bytes": (ctypes.c_int64, [ctypes.c_int64] * 4),
     "dcb_bidir_fuse_fwd": (ctypes.c_int, [_P] * 7 + [ctypes.c_void_p]),
     "dcb_bidir_fuse_bwd": (ctypes.c_int, [_P] * 11 + [ctypes.c_void_p]),
     "dcb_tile_merge_workspace_bytes": (ctypes.c_int64, [ctypes.c_int64] * 3 + [ctypes.c_int32]),

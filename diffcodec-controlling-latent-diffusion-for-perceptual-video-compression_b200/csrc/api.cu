@@ -48,6 +48,9 @@ int backwarp_bwd_impl(const DcbTensor*, const DcbTensor*, const DcbTensor*, cons
                       void*, long long, cudaStream_t);
 long long mask_workspace(long long N, long long H, long long W);
 long long recipe_workspace(long long N, long long C, long long H, long long W);
+long long recipe_det_workspace(long long N, long long C, long long H, long long W);
+int residual_det_impl(const DcbTensor*, const DcbTensor*, const DcbTensor*, const DcbTensor*, const DcbTensor*, const DcbTensor*,
+                      const DcbTensor*, const DcbTensor*, const DcbTensor*, void*, long long, int, cudaStream_t);
 int occlusion_mask_impl(const DcbTensor*, const DcbTensor*, const DcbTensor*, void*, long long, int, cudaStream_t);
 int residual_fused_impl(const DcbTensor*, const DcbTensor*, const DcbTensor*, const DcbTensor*, const DcbTensor*,
                         const DcbTensor*, const DcbTensor*, const DcbTensor*, void*, long long, int, int, cudaStream_t);
@@ -172,7 +175,7 @@ const char* dcb_build_info(void) {
     return "libdiffcodec_b200 " __DATE__ " nvcc " DCB_STR(__CUDACC_VER_MAJOR__) "." DCB_STR(__CUDACC_VER_MINOR__)
            " target sm_100a; kernels: k_splat_step k_planar_step k_list_count k_list_alloc k_list_fill k_list_gather k_scatter_planar k_normalize k_bwd_target k_bwd_source "
            "k_backwarp_rows k_backwarp_fwd k_backwarp_bwd k_cast_f32_bf16 k_recipe_fuse k_bidir_fuse_fwd k_bidir_fuse_bwd "
-           "k_det_emit k_det_reduce k_tile_merge k_splat_owner k_strip_box k_convert k_flow_ingest k_pyr_scatter k_pyr_fuse k_pyr_det_emit k_pyr_det_reduce k_resample_batch k_splat_cluster";
+           "k_det_emit k_det_reduce k_tile_merge k_splat_owner k_strip_box k_convert k_flow_ingest k_pyr_scatter k_pyr_fuse k_pyr_det_emit k_pyr_det_reduce k_recipe_det_fuse k_resample_batch k_splat_cluster";
 }
 
 int64_t dcb_splat_fwd_workspace_bytes(int64_t N, int64_t C, int64_t H, int64_t W, int32_t dtype, int32_t mode, int32_t flags) {
@@ -368,6 +371,18 @@ int64_t dcb_residual_workspace_bytes(int64_t N, int64_t C, int64_t H, int64_t W)
     return (int64_t)recipe_workspace(N, C, H, W);
 }
 
+int64_t dcb_residual_det_workspace_bytes(int64_t N, int64_t C, int64_t H, int64_t W) {
+    if (N < 0 || C < 0 || H < 0 || W < 0) return 0;
+    return (int64_t)recipe_det_workspace(N, C, H, W);
+}
+
+// DCB_FLAG_DETERMINISTIC takes a scratch workspace: with DCB_FLAG_WS_CLEAN it is refused, as dcb_bidir_pyramid_fwd refuses it
+static int check_det_flags(const char* fn, int flags) {
+    if ((flags & DCB_FLAG_DETERMINISTIC) && (flags & DCB_FLAG_WS_CLEAN))
+        return set_error(DCB_E_MODE, "%s: DCB_FLAG_DETERMINISTIC takes a scratch workspace, not DCB_FLAG_WS_CLEAN", fn);
+    return DCB_OK;
+}
+
 int dcb_residual_fused(const DcbTensor* image1, const DcbTensor* flow1, const DcbTensor* flow2, const DcbTensor* gt,
                        const DcbTensor* fused, const DcbTensor* residual, const DcbTensor* occ_fwd,
                        const DcbTensor* occ_bwd, void* ws, int64_t ws_bytes, int32_t variant, int32_t flags,
@@ -383,6 +398,7 @@ int dcb_residual_fused(const DcbTensor* image1, const DcbTensor* flow1, const Dc
     TRY(check_tensor(fn, "occ_fwd", occ_fwd, false));
     TRY(check_tensor(fn, "occ_bwd", occ_bwd, false));
     if (variant != DCB_RECIPE_DATASET && variant != DCB_RECIPE_WRAPPER) return set_error(DCB_E_MODE, "%s: unknown variant %d", fn, variant);
+    TRY(check_det_flags(fn, flags));
     const long long N = image1->size[0], C = image1->size[1], H = image1->size[2], W = image1->size[3];
     TRY(check_limits(fn, image1));
     if (C < 1 || C > 3) return set_error(DCB_E_LIMIT, "%s: fused recipe handles 1..3 image channels, got %lld", fn, C);
@@ -399,6 +415,9 @@ int dcb_residual_fused(const DcbTensor* image1, const DcbTensor* flow1, const Dc
     TRY(check_out(fn, "residual", residual, dt, elem_size(dt)));
     TRY(check_out(fn, "occ_fwd", occ_fwd, dt, elem_size(dt)));
     TRY(check_out(fn, "occ_bwd", occ_bwd, dt, elem_size(dt)));
+    if (flags & DCB_FLAG_DETERMINISTIC)
+        return residual_det_impl(image1, nullptr, flow1, flow2, gt, fused, residual, occ_fwd, occ_bwd, ws, ws_bytes, variant,
+                                 (cudaStream_t)stream);
     return residual_fused_impl(image1, flow1, flow2, gt, fused, residual, occ_fwd, occ_bwd, ws, ws_bytes, variant, flags,
                                (cudaStream_t)stream);
 }
@@ -417,7 +436,8 @@ int dcb_residual_bidir(const DcbTensor* image1, const DcbTensor* image2, const D
     TRY(check_tensor(fn, "residual", residual, true));
     TRY(check_tensor(fn, "occ_fwd", occ_fwd, false));
     TRY(check_tensor(fn, "occ_bwd", occ_bwd, false));
-    if (flags & ~DCB_FLAG_WS_CLEAN) return set_error(DCB_E_MODE, "%s: unknown flags 0x%x", fn, flags);
+    if (flags & ~(DCB_FLAG_DETERMINISTIC | DCB_FLAG_WS_CLEAN)) return set_error(DCB_E_MODE, "%s: unknown flags 0x%x", fn, flags);
+    TRY(check_det_flags(fn, flags));
     const long long N = image1->size[0], C = image1->size[1], H = image1->size[2], W = image1->size[3];
     TRY(check_limits(fn, image1));
     if (C < 1 || C > 3) return set_error(DCB_E_LIMIT, "%s: fused recipe handles 1..3 image channels, got %lld", fn, C);
@@ -436,6 +456,9 @@ int dcb_residual_bidir(const DcbTensor* image1, const DcbTensor* image2, const D
     TRY(check_out(fn, "residual", residual, dt, elem_size(dt)));
     TRY(check_out(fn, "occ_fwd", occ_fwd, dt, elem_size(dt)));
     TRY(check_out(fn, "occ_bwd", occ_bwd, dt, elem_size(dt)));
+    if (flags & DCB_FLAG_DETERMINISTIC)
+        return residual_det_impl(image1, image2, flow1, flow2, gt, fused, residual, occ_fwd, occ_bwd, ws, ws_bytes, 0,
+                                 (cudaStream_t)stream);
     return residual_bidir_impl(image1, image2, flow1, flow2, gt, fused, residual, occ_fwd, occ_bwd, ws, ws_bytes, flags,
                                (cudaStream_t)stream);
 }

@@ -235,6 +235,19 @@ size_t cub_temp_bytes(long long nkeys, int end_bit);
 int det_sort_keys(void* temp, size_t temp_bytes, const unsigned long long* keys, unsigned long long* sorted, long long nkeys,
                   int end_bit, cudaStream_t st);
 
+// The cells of one pyramid level (pyramid.cu) -- the sums of both footprint fields of the level, by flow_f and by flow_b:
+//   acc_mf / dacc_mf: flow_f splatted by flow_b, [N][HW] float4 (x, y, -, -) and its normaliser   (compute_mask(flow_f, flow_b))
+//   acc_mb / dacc_mb: flow_b splatted by flow_f                                                   (compute_mask(flow_b, flow_f))
+//   acc_f / dacc_f:   `first` splatted by flow_f, [N][Cq][HW] float4 and its normaliser; acc_b / dacc_b: `last` by flow_b
+struct PyrCells {
+    float *acc_mf, *acc_mb, *dacc_mf, *dacc_mb, *dacc_f, *dacc_b, *acc_f, *acc_b;
+};
+// pyramid.cu: DCB_FLAG_DETERMINISTIC, every splat of levels lv[0..n) -- emit, one radix sort, reduce (10 counted launches) --
+// into the cells of each level (cells[l]), inside ws (pyramid_det_workspace(lv, n) bytes of plain scratch). A level whose
+// `last` is NULL has no feature splat on its flow_b field; its normaliser and mask cells are still written.
+int pyramid_det_splats(const DcbPyramidLevel* lv, int n, void* ws, bool masks, PyrCells* cells, cudaStream_t st);
+long long pyramid_det_workspace(const DcbPyramidLevel* lv, int n);
+
 template <class A> __device__ __forceinline__ Foot<A> make_foot(int x, int y, A flow_x, A flow_y) {
     Foot<A> f;
     f.fx = add_rn((A)x, flow_x);

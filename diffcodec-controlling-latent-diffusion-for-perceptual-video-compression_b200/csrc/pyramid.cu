@@ -32,7 +32,8 @@
 //                      arithmetic (det_add), written into the cells launch B reads
 //   k_pyr_fuse<T, 1> : launch B dividing as k_normalize does; nothing is re-zeroed, the workspace is plain scratch.
 // The outputs are then bit-identical, run to run, to the composition of deterministic single ops (compute_mask, the masked
-// soft splat, bidir_fuse) in fp32.
+// soft splat, bidir_fuse) in fp32. The first three steps are pyramid_det_splats(), which the deterministic conditioning
+// recipes (recipe.cu) run too, as one level with its own epilogue.
 #include "splat_planar.cuh"
 
 namespace dcb {
@@ -470,25 +471,91 @@ static PyrDetLayout pyr_det_layout(const DcbPyramidLevel* lv, int n) {
 long long pyramid_det_keys(const DcbPyramidLevel* lv, int n) { return pyr_det_layout(lv, n).nkeys; }
 long long pyramid_det_workspace(const DcbPyramidLevel* lv, int n) { return pyr_det_layout(lv, n).total_bytes; }
 
-template <class T>
-static int launch_pyramid(const PyrScatterArgs& sa, unsigned s_items, const PyrFuseArgs& fa, unsigned f_items, cudaStream_t st) {
-    DCB_CHECK_CUDA(launch_pdl(k_pyr_scatter<T>, dim3(s_items), dim3(32), 0, st, sa));
-    count_launch();
-    DCB_CHECK_CUDA(launch_pdl(k_pyr_fuse<T, false>, dim3(f_items), dim3(32), 0, st, fa));
-    count_launch();
-    return DCB_OK;
+// the cells of every level inside `cells` (the workspace, or its cells part in deterministic mode): first the per-pixel planes
+// of all levels (level_shared_bytes: both mask splats, the four normalisers), then the feature quads (level_feat_bytes)
+static void pyr_cells(const DcbPyramidLevel* lv, int n, char* cells, PyrCells* out) {
+    long long shared_total = 0;
+    for (int l = 0; l < n; ++l) shared_total += level_shared_bytes(lv[l].first->size[0], lv[l].first->size[2], lv[l].first->size[3]);
+    char* shared = cells;
+    char* feat = cells + shared_total;
+    for (int l = 0; l < n; ++l) {
+        const long long N = lv[l].first->size[0], C = lv[l].first->size[1], H = lv[l].first->size[2], W = lv[l].first->size[3];
+        out[l] = PyrCells{};
+        if (N * C * H * W == 0) continue;
+        const long long HW = H * W, Cq = (C + 3) / 4;
+        PyrCells& c = out[l];
+        c.acc_mf = (float*)shared;               c.acc_mb = c.acc_mf + N * HW * 4;
+        c.dacc_mf = c.acc_mb + N * HW * 4;       c.dacc_mb = c.dacc_mf + N * HW;
+        c.dacc_f = c.dacc_mb + N * HW;           c.dacc_b = c.dacc_f + N * HW;
+        c.acc_f = (float*)feat;                  c.acc_b = c.acc_f + N * Cq * HW * 4;
+        shared += level_shared_bytes(N, H, W);
+        feat += level_feat_bytes(N, C, H, W);
+    }
 }
 
 template <class T>
-static int launch_pyramid_det(const PyrDetArgs& da, const PyrDetLayout& D, char* ws, long long r_items, const PyrFuseArgs& fa,
-                              unsigned f_items, cudaStream_t st) {
+static int launch_det_splats(const PyrDetArgs& da, const PyrDetLayout& D, char* ws, long long r_items, cudaStream_t st) {
     DCB_CHECK_CUDA(launch_pdl(k_pyr_det_emit<T>, dim3((unsigned)((D.nsrc + 255) / 256)), dim3(256), 0, st, da));
     count_launch();
     const int rc = det_sort_keys(ws + D.temp_off, D.temp_bytes, da.keys, (unsigned long long*)da.sorted, D.nkeys, D.end_bit, st);
     if (rc != DCB_OK) return rc;
     DCB_CHECK_CUDA(launch_pdl(k_pyr_det_reduce<T>, dim3((unsigned)((r_items + 255) / 256)), dim3(256), 0, st, da));
     count_launch();
-    DCB_CHECK_CUDA(launch_pdl(k_pyr_fuse<T, true>, dim3(f_items), dim3(32), 0, st, fa));
+    return DCB_OK;
+}
+
+// Preconditions (checked by the callers): 1 <= n <= kMaxLevels, all tensors of one dtype (F32 / BF16 / F16), shapes consistent,
+// pyramid_det_keys(lv, n) < 2^31, ws 256-byte aligned and pyramid_det_workspace(lv, n) bytes long.
+int pyramid_det_splats(const DcbPyramidLevel* lv, int n, void* ws, bool masks, PyrCells* cells, cudaStream_t st) {
+    const PyrDetLayout D = pyr_det_layout(lv, n);
+    pyr_cells(lv, n, (char*)ws + D.cells_off, cells);
+    PyrDetArgs da;
+    da.n_fields = 0;
+    da.masks = masks ? 1 : 0; da.s = D.s; da.nkeys = D.nkeys;
+    da.keys = (unsigned long long*)ws;
+    da.sorted = (const unsigned long long*)((char*)ws + D.sorted_off);
+    da.invalid = (unsigned long long)D.nsrc << D.s;
+    unsigned d_src = 0, d_tgt = 0;
+    long long r_items = 0;
+    for (int l = 0; l < n; ++l) {
+        const DcbPyramidLevel& d = lv[l];
+        const long long N = d.first->size[0], C = d.first->size[1], H = d.first->size[2], W = d.first->size[3];
+        if (N * C * H * W == 0) continue;
+        const long long HW = H * W;
+        auto add_field = [&](const DcbTensor* flow, const DcbTensor* in, const DcbTensor* metric, const DcbTensor* mflow, long long Cf,
+                             float* acc, float* dacc, float* acc_m, float* dacc_m) {
+            PyrDetField& F = da.f[da.n_fields++];
+            F.flow = make_view(flow); F.in = make_view(in); F.metric = make_view(metric); F.mflow = make_view(mflow);
+            F.acc = acc; F.dacc = dacc; F.acc_m = acc_m; F.dacc_m = dacc_m;
+            F.C = (int)Cf; F.Cq = Cf > 0 ? (int)((Cf + 3) / 4) : 1;    // C = 0: quad 0 still owns the normaliser and mask cells
+            F.H = (int)H; F.W = (int)W;
+            F.HW = (unsigned)HW; F.NHW = (unsigned)(N * HW);
+            F.src0 = d_src; F.tgt0 = d_tgt; F.item0 = r_items;
+            d_src += F.NHW; d_tgt += F.NHW; r_items += (long long)F.NHW * F.Cq;
+        };
+        const PyrCells& c = cells[l];
+        add_field(d.flow_f, d.first, d.metric_f, d.flow_b, C, c.acc_f, c.dacc_f, c.acc_mb, c.dacc_mb);                  // compute_mask(flow_b, flow_f)
+        add_field(d.flow_b, d.last, d.metric_b, d.flow_f, d.last ? C : 0, c.acc_b, c.dacc_b, c.acc_mf, c.dacc_mf);     // compute_mask(flow_f, flow_b)
+    }
+    if (da.n_fields == 0) return DCB_OK;
+    if ((r_items + 255) / 256 >= (1ll << 31))
+        return set_error(DCB_E_LIMIT, "deterministic splats: %lld (pixel, channel quad) cells exceed the grid", r_items);
+    const int dt = lv[0].first->dtype;
+    switch (dt) {
+        case DCB_F32: return launch_det_splats<float>(da, D, (char*)ws, r_items, st);
+        case DCB_BF16: return launch_det_splats<__nv_bfloat16>(da, D, (char*)ws, r_items, st);
+        case DCB_F16: return launch_det_splats<__half>(da, D, (char*)ws, r_items, st);
+        default: return set_error(DCB_E_DTYPE, "deterministic splats: unsupported dtype %d", dt);
+    }
+}
+
+template <class T>
+static int launch_pyramid(const PyrScatterArgs& sa, unsigned s_items, const PyrFuseArgs& fa, unsigned f_items, bool det, cudaStream_t st) {
+    if (!det) {
+        DCB_CHECK_CUDA(launch_pdl(k_pyr_scatter<T>, dim3(s_items), dim3(32), 0, st, sa));
+        count_launch();
+    }
+    DCB_CHECK_CUDA(launch_pdl(det ? k_pyr_fuse<T, true> : k_pyr_fuse<T, false>, dim3(f_items), dim3(32), 0, st, fa));
     count_launch();
     return DCB_OK;
 }
@@ -497,42 +564,30 @@ static int launch_pyramid_det(const PyrDetArgs& da, const PyrDetLayout& D, char*
 // ws holds pyramid_workspace() bytes, 256-byte aligned, all-zero if DCB_FLAG_WS_CLEAN; with DCB_FLAG_DETERMINISTIC (never with
 // WS_CLEAN) ws is plain scratch of pyramid_det_workspace() bytes and pyramid_det_keys() < 2^31.
 int bidir_pyramid_fwd_impl(const DcbPyramidLevel* lv, int n, void* ws, int flags, cudaStream_t st) {
-    PyrScatterArgs sa; PyrFuseArgs fa; PyrDetArgs da;
-    sa.n_jobs = 0; fa.n_levels = 0; da.n_fields = 0;
+    PyrScatterArgs sa; PyrFuseArgs fa;
+    sa.n_jobs = 0; fa.n_levels = 0;
     fa.masks = (flags & DCB_PYRAMID_NO_MASKS) ? 0 : 1;
     fa.holes = (flags & DCB_PYRAMID_NO_HOLES) ? 0 : 1;
     const bool det = (flags & DCB_FLAG_DETERMINISTIC) != 0;
     long long shared_total = 0;
     for (int l = 0; l < n; ++l) shared_total += level_shared_bytes(lv[l].first->size[0], lv[l].first->size[2], lv[l].first->size[3]);
-    const long long total = pyramid_workspace(lv, n);
-    PyrDetLayout D = {};
-    char* cells = (char*)ws;
+    PyrCells cells[kMaxLevels];
     if (det) {
-        D = pyr_det_layout(lv, n);
-        cells += D.cells_off;
-        da.masks = fa.masks; da.s = D.s; da.nkeys = D.nkeys;
-        da.keys = (unsigned long long*)ws;
-        da.sorted = (const unsigned long long*)((char*)ws + D.sorted_off);
-        da.invalid = (unsigned long long)D.nsrc << D.s;
-    } else if (!(flags & DCB_FLAG_WS_CLEAN)) {
-        DCB_CHECK_CUDA(cudaMemsetAsync(ws, 0, (size_t)total, st));
+        // launch A's place: emit, sort, reduce
+        const int rc = pyramid_det_splats(lv, n, ws, fa.masks != 0, cells, st);
+        if (rc != DCB_OK) return rc;
+    } else {
+        pyr_cells(lv, n, (char*)ws, cells);
+        if (!(flags & DCB_FLAG_WS_CLEAN)) DCB_CHECK_CUDA(cudaMemsetAsync(ws, 0, (size_t)pyramid_workspace(lv, n), st));
     }
-    char* shared = cells;
-    char* feat = cells + shared_total;
-    unsigned s_items = 0, f_items = 0, d_src = 0, d_tgt = 0;
-    long long r_items = 0;
+    unsigned s_items = 0, f_items = 0;
     const int dt = lv[0].first->dtype;
     for (int l = 0; l < n; ++l) {
         const DcbPyramidLevel& d = lv[l];
         const long long N = d.first->size[0], C = d.first->size[1], H = d.first->size[2], W = d.first->size[3];
         if (N * C * H * W == 0) continue;
         const long long HW = H * W, Cq = (C + 3) / 4;
-        float* acc_mf = (float*)shared;              float* acc_mb = acc_mf + N * HW * 4;
-        float* dacc_mf = acc_mb + N * HW * 4;        float* dacc_mb = dacc_mf + N * HW;
-        float* dacc_f = dacc_mb + N * HW;            float* dacc_b = dacc_f + N * HW;
-        float* acc_f = (float*)feat;                 float* acc_b = acc_f + N * Cq * HW * 4;
-        shared += level_shared_bytes(N, H, W);
-        feat += level_feat_bytes(N, C, H, W);
+        const PyrCells& c = cells[l];
         const int tiles_x = (int)((W + 31) / 32), ts = tiles_x * (int)((H + kPRows - 1) / kPRows);
         auto add_job = [&](const DcbTensor* in, const DcbTensor* flow, const DcbTensor* metric, float* acc, float* dacc, long long Cj) {
             PyrJob& b = sa.job[sa.n_jobs++];
@@ -545,32 +600,19 @@ int bidir_pyramid_fwd_impl(const DcbPyramidLevel* lv, int n, void* ws, int flags
             b.item0 = s_items; b.items = (unsigned)(N * ts * b.ncg);
             s_items += b.items;
         };
-        auto add_field = [&](const DcbTensor* flow, const DcbTensor* in, const DcbTensor* metric, const DcbTensor* mflow, float* acc,
-                             float* dacc, float* acc_m, float* dacc_m) {
-            PyrDetField& F = da.f[da.n_fields++];
-            F.flow = make_view(flow); F.in = make_view(in); F.metric = make_view(metric); F.mflow = make_view(mflow);
-            F.acc = acc; F.dacc = dacc; F.acc_m = acc_m; F.dacc_m = dacc_m;
-            F.C = (int)C; F.Cq = (int)Cq; F.H = (int)H; F.W = (int)W;
-            F.HW = (unsigned)HW; F.NHW = (unsigned)(N * HW);
-            F.src0 = d_src; F.tgt0 = d_tgt; F.item0 = r_items;
-            d_src += F.NHW; d_tgt += F.NHW; r_items += (long long)F.NHW * F.Cq;
-        };
-        if (det) {
-            add_field(d.flow_f, d.first, d.metric_f, d.flow_b, acc_f, dacc_f, acc_mb, dacc_mb);   // compute_mask(flow_b, flow_f)
-            add_field(d.flow_b, d.last, d.metric_b, d.flow_f, acc_b, dacc_b, acc_mf, dacc_mf);    // compute_mask(flow_f, flow_b)
-        } else {
+        if (!det) {
             if (fa.masks) {
-                add_job(d.flow_f, d.flow_b, nullptr, acc_mf, dacc_mf, 2);        // compute_mask(flow_f, flow_b)
-                add_job(d.flow_b, d.flow_f, nullptr, acc_mb, dacc_mb, 2);        // compute_mask(flow_b, flow_f)
+                add_job(d.flow_f, d.flow_b, nullptr, c.acc_mf, c.dacc_mf, 2);        // compute_mask(flow_f, flow_b)
+                add_job(d.flow_b, d.flow_f, nullptr, c.acc_mb, c.dacc_mb, 2);        // compute_mask(flow_b, flow_f)
             }
-            add_job(d.first, d.flow_f, d.metric_f, acc_f, dacc_f, C);
-            add_job(d.last, d.flow_b, d.metric_b, acc_b, dacc_b, C);
+            add_job(d.first, d.flow_f, d.metric_f, c.acc_f, c.dacc_f, C);
+            add_job(d.last, d.flow_b, d.metric_b, c.acc_b, c.dacc_b, C);
         }
         PyrLevel& L = fa.lv[fa.n_levels++];
         L.flow_f = make_view(d.flow_f); L.flow_b = make_view(d.flow_b);
         L.metric_f = make_view(d.metric_f); L.metric_b = make_view(d.metric_b);
-        L.acc_mf = acc_mf; L.dacc_mf = dacc_mf; L.acc_mb = acc_mb; L.dacc_mb = dacc_mb;
-        L.acc_f = acc_f; L.dacc_f = dacc_f; L.acc_b = acc_b; L.dacc_b = dacc_b;
+        L.acc_mf = c.acc_mf; L.dacc_mf = c.dacc_mf; L.acc_mb = c.acc_mb; L.dacc_mb = c.dacc_mb;
+        L.acc_f = c.acc_f; L.dacc_f = c.dacc_f; L.acc_b = c.acc_b; L.dacc_b = c.dacc_b;
         L.fused = d.fused; L.warped_f = d.warped_f; L.warped_b = d.warped_b; L.occ_f = d.occ_f; L.occ_b = d.occ_b;
         L.norm_f = (float*)d.norm_f; L.norm_b = (float*)d.norm_b;
         L.C = (int)C; L.Cq = (int)Cq; L.W = (int)W; L.HW = (unsigned)HW;
@@ -581,23 +623,13 @@ int bidir_pyramid_fwd_impl(const DcbPyramidLevel* lv, int n, void* ws, int flags
     }
     if (fa.n_levels == 0) return DCB_OK;
     int rc;
-    if (det) {
-        if ((r_items + 255) / 256 >= (1ll << 31))
-            return set_error(DCB_E_LIMIT, "bidir_pyramid_fwd(deterministic): %lld (pixel, channel quad) cells exceed the grid", r_items);
-        switch (dt) {
-            case DCB_F32: return launch_pyramid_det<float>(da, D, (char*)ws, r_items, fa, f_items, st);
-            case DCB_BF16: return launch_pyramid_det<__nv_bfloat16>(da, D, (char*)ws, r_items, fa, f_items, st);
-            case DCB_F16: return launch_pyramid_det<__half>(da, D, (char*)ws, r_items, fa, f_items, st);
-            default: return set_error(DCB_E_DTYPE, "bidir_pyramid_fwd: unsupported dtype %d", dt);
-        }
-    }
     switch (dt) {
-        case DCB_F32: rc = launch_pyramid<float>(sa, s_items, fa, f_items, st); break;
-        case DCB_BF16: rc = launch_pyramid<__nv_bfloat16>(sa, s_items, fa, f_items, st); break;
-        case DCB_F16: rc = launch_pyramid<__half>(sa, s_items, fa, f_items, st); break;
+        case DCB_F32: rc = launch_pyramid<float>(sa, s_items, fa, f_items, det, st); break;
+        case DCB_BF16: rc = launch_pyramid<__nv_bfloat16>(sa, s_items, fa, f_items, det, st); break;
+        case DCB_F16: rc = launch_pyramid<__half>(sa, s_items, fa, f_items, det, st); break;
         default: return set_error(DCB_E_DTYPE, "bidir_pyramid_fwd: unsupported dtype %d", dt);
     }
-    if (rc != DCB_OK) return rc;
+    if (rc != DCB_OK || det) return rc;
     // the per-pixel planes have several readers (one warp per channel group): re-zeroed behind the kernel
     DCB_CHECK_CUDA(cudaMemsetAsync(ws, 0, (size_t)shared_total, st));
     return DCB_OK;

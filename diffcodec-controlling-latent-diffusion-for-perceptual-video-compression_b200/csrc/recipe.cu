@@ -21,6 +21,10 @@
 // dcb_residual_bidir (residual_bidir_impl) is the two-reference recipe (SURVEY.md App. B-6): image2 splatted by flow2 and
 // image1 by flow1, masks with the pairing of extractors.py:290-295, soft_fuse, residual -- two rider passes of splat_pipe.cu
 // (bidir_pipe_impl), or four single splats and k_recipe_fuse<T, true> for the forwards the pipeline does not cover.
+//
+// DCB_FLAG_DETERMINISTIC (both entries, F32): the recipe is one level of the deterministic pyramid's splats (pyramid_det_splats:
+// emit, one radix sort, reduce) and one epilogue, k_recipe_det_fuse -- 11 launches per frame group, bit-identical to the
+// composition of deterministic single ops (softsplat, compute_mask, the fusion ops, the subtraction).
 #include "dcb_common.cuh"
 
 namespace dcb {
@@ -77,6 +81,17 @@ struct FuseArgs {
     int variant;
 };
 
+// the fusion weights of the one-reference recipe: the torch ops of residual_utils._composed
+__device__ __forceinline__ void recipe_weights(int variant, float of, float ob, float& w0, float& w1) {
+    if (variant == DCB_RECIPE_DATASET) {          // dataset.py:255-259: masks are the confidences
+        const float ws = add_rn(add_rn(of, ob), 0.000001f);
+        w0 = of / ws; w1 = ob / ws;
+    } else {                                      // residual_utils.py:181-185: ones are the confidences
+        const float ws = add_rn(2.f, 0.000001f);
+        w0 = 1.f / ws; w1 = w0;
+    }
+}
+
 // BIDIR: the two-reference recipe (dcb_residual_bidir); warped1 arrives in `residual`, warped2 in `fused`, and the fusion is
 // soft_fuse on the valid masks 1 - occ (bidir_soft_fuse); `variant` is not read
 template <class T, bool BIDIR = false>
@@ -99,13 +114,7 @@ __global__ void __launch_bounds__(256) k_recipe_fuse(const FuseArgs a) {
         return;
     }
     float w0, w1;
-    if (a.variant == DCB_RECIPE_DATASET) {        // dataset.py:255-259: masks are the confidences
-        const float ws = add_rn(add_rn(of, ob), 0.000001f);
-        w0 = of / ws; w1 = ob / ws;
-    } else {                                      // residual_utils.py:181-185: ones are the confidences
-        const float ws = add_rn(2.f, 0.000001f);
-        w0 = 1.f / ws; w1 = w0;
-    }
+    recipe_weights(a.variant, of, ob, w0, w1);
     const bool hole = a.variant == DCB_RECIPE_WRAPPER && add_rn(of, ob) > 1.5f;   // residual_utils.py:190-193
     constexpr int U = 4;                                         // channels in flight: 2 * U loads per thread
     for (int c0 = 0; c0 < a.C; c0 += U) {
@@ -285,6 +294,120 @@ int residual_bidir_impl(const DcbTensor* image1, const DcbTensor* image2, const 
     a.C = (int)C; a.W = (int)W; a.variant = 0;
     if (image1->dtype == DCB_F32) return launch_fuse<float, true>(a, st);
     return launch_fuse<__nv_bfloat16, true>(a, st);
+}
+
+// ---------------------------------------------------------------------------------------------
+// DCB_FLAG_DETERMINISTIC: both recipes as one level of the deterministic pyramid's splats (pyramid.cu) and one epilogue
+// ---------------------------------------------------------------------------------------------
+// The recipe is one pyramid level with flow_f = flow1, flow_b = flow2: field 1 (flow1's footprints) carries image1 and flow2
+// (occ_bwd = compute_mask(flow2, flow1)), field 2 (flow2's footprints) carries flow1 (occ_fwd = compute_mask(flow1, flow2)) and,
+// in the two-reference recipe, image2. pyramid_det_splats writes the cells; k_recipe_det_fuse does the rest per target pixel.
+enum { kRecipeBidir = 2 };   // the third form of k_recipe_det_fuse, next to DCB_RECIPE_DATASET and DCB_RECIPE_WRAPPER
+
+struct RecipeDetArgs {
+    View flow1, flow2, gt;
+    PyrCells cells;          // C <= 3: one channel quad, so every cell of pixel p sits at index p
+    float *fused, *residual, *occ_fwd, *occ_bwd;
+    unsigned total, HW;
+    int C, W;
+};
+
+// Each step is the arithmetic of the composition of deterministic single ops (residual_utils._composed / _composed_bidir):
+// warps divided as k_normalize divides, masks by occlusion() (compute_mask), fusion by the k_recipe_fuse weights or
+// bidir_soft_fuse (bidir_fuse on the valid masks), residual = gt - fused.
+template <int KIND>
+__global__ void __launch_bounds__(256) k_recipe_det_fuse(const RecipeDetArgs a) {
+    pdl_wait();
+    const unsigned p = blockIdx.x * 256 + threadIdx.x;
+    if (p >= a.total) return;
+    const unsigned n = p / a.HW, r = p - n * a.HW;
+    const int y = (int)(r / (unsigned)a.W), x = (int)(r - (unsigned)y * (unsigned)a.W);
+    const PyrCells& c = a.cells;
+    const float* f1 = (const float*)a.flow1.p + n * a.flow1.sN + (long long)y * a.flow1.sH + (long long)x * a.flow1.sW;
+    const float* f2 = (const float*)a.flow2.p + n * a.flow2.sN + (long long)y * a.flow2.sH + (long long)x * a.flow2.sW;
+    const float4 mf = ((const float4*)c.acc_mf)[p], mb = ((const float4*)c.acc_mb)[p];
+    const float of = occlusion(mf.x, mf.y, c.dacc_mf[p], f2[0], f2[a.flow2.sC]);
+    const float ob = occlusion(mb.x, mb.y, c.dacc_mb[p], f1[0], f1[a.flow1.sC]);
+    if (a.occ_fwd) a.occ_fwd[p] = of;
+    if (a.occ_bwd) a.occ_bwd[p] = ob;
+    // normalisers of softsplat.py:256-258 ('soft' = add 1e-7)
+    const float d1 = add_rn(c.dacc_f[p], 0.0000001f);
+    const float4 s1 = ((const float4*)c.acc_f)[p];
+    const float v1[3] = {s1.x, s1.y, s1.z};
+    float v2[3] = {0.f, 0.f, 0.f}, d2 = 1.f;
+    if constexpr (KIND == kRecipeBidir) {
+        const float4 s2 = ((const float4*)c.acc_b)[p];
+        v2[0] = s2.x; v2[1] = s2.y; v2[2] = s2.z;
+        d2 = add_rn(c.dacc_b[p], 0.0000001f);
+    }
+    float w0 = 0.f, w1 = 0.f;
+    bool hole = false;
+    if constexpr (KIND != kRecipeBidir) {
+        recipe_weights(KIND, of, ob, w0, w1);
+        hole = KIND == DCB_RECIPE_WRAPPER && add_rn(of, ob) > 1.5f;
+    }
+    const float* gp = (const float*)a.gt.p + n * a.gt.sN + (long long)y * a.gt.sH + (long long)x * a.gt.sW;
+    float* fo = a.fused + (size_t)n * a.C * a.HW + r;
+    float* ro = a.residual + (size_t)n * a.C * a.HW + r;
+#pragma unroll
+    for (int ch = 0; ch < 3; ++ch) {
+        if (ch >= a.C) break;
+        const float A = v1[ch] / d1;
+        float f;
+        if constexpr (KIND == kRecipeBidir) {
+            f = bidir_soft_fuse(A, v2[ch] / d2, of, ob);
+        } else {
+            f = hole ? mul_rn(0.5f, add_rn(A, A)) : add_rn(mul_rn(w0, A), mul_rn(w1, A));   // warped2 is warped1 (SURVEY.md B-6)
+        }
+        st_stream(fo + (size_t)ch * a.HW, f);
+        st_stream(ro + (size_t)ch * a.HW, sub_rn(ld<float>(gp + (long long)ch * a.gt.sC), f));
+    }
+}
+
+static DcbPyramidLevel recipe_level(const DcbTensor* first) {
+    DcbPyramidLevel lv = {};
+    lv.first = first;
+    return lv;
+}
+
+// sized for the two-reference recipe (C channels on both fields); the one-reference recipe uses the same layout
+long long recipe_det_workspace(long long N, long long C, long long H, long long W) {
+    DcbTensor t = {};
+    t.dtype = DCB_F32;
+    t.size[0] = N; t.size[1] = C; t.size[2] = H; t.size[3] = W;
+    const DcbPyramidLevel lv = recipe_level(&t);
+    return pyramid_det_workspace(&lv, 1);
+}
+
+// image2 NULL: the one-reference recipe (`variant`); else the two-reference recipe. Shapes and dtypes checked by the caller.
+int residual_det_impl(const DcbTensor* image1, const DcbTensor* image2, const DcbTensor* flow1, const DcbTensor* flow2,
+                      const DcbTensor* gt, const DcbTensor* fused, const DcbTensor* residual, const DcbTensor* occ_fwd,
+                      const DcbTensor* occ_bwd, void* ws, long long ws_bytes, int variant, cudaStream_t st) {
+    const long long N = image1->size[0], C = image1->size[1], H = image1->size[2], W = image1->size[3];
+    if (image1->dtype != DCB_F32)
+        return set_error(DCB_E_DTYPE, "residual(deterministic): F32 only, got %d", image1->dtype);
+    if (N * H * W == 0) return DCB_OK;
+    if (8 * N * H * W >= (1ll << 31))
+        return set_error(DCB_E_LIMIT, "residual(deterministic): 8 keys per pixel, 8*N*H*W must stay below 2^31 (got %lld)", 8 * N * H * W);
+    const long long need = recipe_det_workspace(N, C, H, W);
+    if (!ws || ws_bytes < need || ((uintptr_t)ws & 255))
+        return set_error(DCB_E_WORKSPACE, "residual(deterministic): workspace of %lld bytes (256 B aligned) required, got %lld", need, ws_bytes);
+    DcbPyramidLevel lv = recipe_level(image1);
+    lv.last = image2; lv.flow_f = flow1; lv.flow_b = flow2;
+    RecipeDetArgs a;
+    int rc = pyramid_det_splats(&lv, 1, ws, true, &a.cells, st);
+    if (rc != DCB_OK) return rc;
+    a.flow1 = make_view(flow1); a.flow2 = make_view(flow2); a.gt = make_view(gt);
+    a.fused = (float*)fused->ptr; a.residual = (float*)residual->ptr;
+    a.occ_fwd = occ_fwd ? (float*)occ_fwd->ptr : nullptr; a.occ_bwd = occ_bwd ? (float*)occ_bwd->ptr : nullptr;
+    a.HW = (unsigned)(H * W); a.total = (unsigned)(N * H * W);
+    a.C = (int)C; a.W = (int)W;
+    const dim3 grid((a.total + 255) / 256);
+    if (image2) DCB_CHECK_CUDA(launch_pdl(k_recipe_det_fuse<kRecipeBidir>, grid, dim3(256), 0, st, a));
+    else if (variant == DCB_RECIPE_DATASET) DCB_CHECK_CUDA(launch_pdl(k_recipe_det_fuse<DCB_RECIPE_DATASET>, grid, dim3(256), 0, st, a));
+    else DCB_CHECK_CUDA(launch_pdl(k_recipe_det_fuse<DCB_RECIPE_WRAPPER>, grid, dim3(256), 0, st, a));
+    count_launch();
+    return DCB_OK;
 }
 
 }  // namespace dcb

@@ -9,6 +9,10 @@ pipeline passes (dcb_residual_fused: four launches per frame group).
 
 ``residual_conditioning_bidir`` builds the residual the datasets intended (SURVEY.md App. B-6): BOTH decoded
 I-frames warped by their own flows, fused by occlusion, subtracted -- also two pipeline passes (dcb_residual_bidir).
+
+Under ``deterministic()`` both builders keep one library call per frame group in fp32 (DCB_FLAG_DETERMINISTIC: emit, one
+radix sort, reduce, fuse -- 11 launches), bit for bit the composition of deterministic single ops that bf16, fp64 and
+``C > 3`` still run.
 """
 from __future__ import annotations
 
@@ -24,9 +28,65 @@ __all__ = ["residual_conditioning", "residual_conditioning_bidir", "ResidueDatas
 
 _VARIANTS = {"dataset": _lib.RECIPE_DATASET, "wrapper": _lib.RECIPE_WRAPPER}
 
+# Deterministic mode: the workspace of one frame group stays under this many bytes (a group holds one frame at least; a
+# 1080p RGB frame needs about 0.55 GB); its 8 sort keys per pixel stay below the ABI's 2^31.
+DET_GROUP_BYTES = 2 << 30
+_det_groups: dict = {}
+
+
+def _det_group(n, c, h, w):
+    """(frames per group, workspace bytes of one group) of the deterministic recipe for a batch of n frames."""
+    key = (n, c, h, w, DET_GROUP_BYTES)
+    v = _det_groups.get(key)
+    if v is None:
+        need = _lib.lib().dcb_residual_det_workspace_bytes
+        lo, hi = 1, max(1, min(n, ((1 << 31) - 1) // (8 * h * w)))   # the largest group within the cap: need() grows with it
+        while lo < hi:
+            mid = (lo + hi + 1) // 2
+            if need(mid, c, h, w) <= DET_GROUP_BYTES:
+                lo = mid
+            else:
+                hi = mid - 1
+        v = _det_groups[key] = (lo, need(lo, c, h, w))
+    return v
+
+
+def _deterministic_recipe(image1, image2, flow1, flow2, gt, variant):
+    """fp32, 1 <= C <= 3, under deterministic(): dcb_residual_fused (image2 None) or dcb_residual_bidir with
+    DCB_FLAG_DETERMINISTIC, one call per frame group. Frames are independent, so the bits do not depend on the grouping."""
+    lib = _lib.lib()
+    n, c, h, w = image1.shape
+    dev = image1.device
+    fused = torch.empty((n, c, h, w), dtype=torch.float32, device=dev)
+    residual = torch.empty_like(fused)
+    occ_fwd = torch.empty((n, 1, h, w), dtype=torch.float32, device=dev)
+    occ_bwd = torch.empty_like(occ_fwd)
+    g, need = _det_group(n, c, h, w)
+    stream = _lib.stream_ptr(dev)
+    ws = _lib.workspace(dev, need, "scratch", stream)
+    d = _lib.desc
+    with _lib.on_device(dev):
+        for i in range(0, n, g):
+            s = slice(i, i + g)
+            outs = (d(fused[s]), d(residual[s]), d(occ_fwd[s]), d(occ_bwd[s]))
+            if image2 is None:
+                rc = lib.dcb_residual_fused(d(image1[s]), d(flow1[s]), d(flow2[s]), d(gt[s]), *outs, ws.data_ptr(), ws.numel(),
+                                            _VARIANTS[variant], _lib.FLAG_DETERMINISTIC, stream)
+            else:
+                rc = lib.dcb_residual_bidir(d(image1[s]), d(image2[s]), d(flow1[s]), d(flow2[s]), d(gt[s]), *outs, ws.data_ptr(),
+                                            ws.numel(), _lib.FLAG_DETERMINISTIC, stream)
+            _lib.check(rc, "dcb_residual_bidir" if image2 is not None else "dcb_residual_fused")
+    return fused, residual, occ_fwd, occ_bwd
+
+
+def _deterministic_fp32(image1, gt):
+    n, c, h, w = image1.shape
+    return (is_deterministic() and image1.dtype == torch.float32 and gt.dtype == torch.float32 and 1 <= c <= 3
+            and n * h * w > 0)
+
 
 def _composed(image1, flow1, flow2, gt, variant):
-    """General path (any channel count / fp64 / deterministic): same ops, built from the single-op kernels."""
+    """General path (any channel count / fp64 / bf16 deterministic): same ops, built from the single-op kernels."""
     metric = torch.ones_like(flow1[:, :1])
     warped1 = softsplat(tenIn=image1, tenFlow=flow1, tenMetric=metric, strMode="soft")
     warped2 = warped1                                          # the reference recomputes the identical splat
@@ -58,7 +118,10 @@ def residual_conditioning(image1, flow1, flow2, gt, variant: str = "dataset", re
     n, c, h, w = image1.shape
     fusable = (c <= 3 and image1.dtype in (torch.float32, torch.bfloat16) and flow1.dtype == image1.dtype
                and flow2.dtype == image1.dtype and gt.dtype == image1.dtype and not is_deterministic())
-    if not fusable:
+    if _deterministic_fp32(image1, gt):
+        fused, residual, occ_fwd, occ_bwd = _deterministic_recipe(image1, None, flow1.to(image1.dtype), flow2.to(image1.dtype),
+                                                                  gt, variant)
+    elif not fusable:
         fused, residual, occ_fwd, occ_bwd = _composed(image1, flow1.to(image1.dtype), flow2.to(image1.dtype), gt, variant)
     else:
         lib = _lib.lib()
@@ -87,7 +150,7 @@ def residual_conditioning(image1, flow1, flow2, gt, variant: str = "dataset", re
 
 
 def _composed_bidir(image1, image2, flow1, flow2, gt):
-    """General path of the two-reference builder (any channel count / fp64 / deterministic): the single-op kernels."""
+    """General path of the two-reference builder (any channel count / fp64 / bf16 deterministic): the single-op kernels."""
     ones = torch.ones_like(flow1[:, :1])
     warped1 = softsplat(tenIn=image1, tenFlow=flow1, tenMetric=ones, strMode="soft")
     warped2 = softsplat(tenIn=image2, tenFlow=flow2, tenMetric=ones, strMode="soft")
@@ -125,7 +188,10 @@ def residual_conditioning_bidir(image1, image2, flow1, flow2, gt, return_masks: 
     dt_ = image1.dtype
     fusable = (c <= 3 and dt_ in (torch.float32, torch.bfloat16) and all(t.dtype == dt_ for t in (image2, flow1, flow2, gt))
                and not is_deterministic())
-    if not fusable:
+    if _deterministic_fp32(image1, image1):                     # gt is cast to image1's dtype, as the composition casts it
+        fused, residual, occ_fwd, occ_bwd = _deterministic_recipe(image1, image2.to(dt_), flow1.to(dt_), flow2.to(dt_), gt.to(dt_),
+                                                                  "bidir")
+    elif not fusable:
         fused, residual, occ_fwd, occ_bwd = _composed_bidir(image1, image2.to(dt_), flow1.to(dt_), flow2.to(dt_), gt.to(dt_))
     else:
         lib = _lib.lib()

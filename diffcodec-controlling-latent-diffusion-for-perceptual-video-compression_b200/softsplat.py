@@ -48,7 +48,8 @@ def is_deterministic() -> bool:
 def deterministic(enabled: bool = True):
     """Within the block, forward splats use the bit-exact sort-then-reduce kernels: ``softsplat``, ``compute_mask``, the
     warpers, and the conditioning pyramids (``bidirectional_pyramid``, ``pyramid_conditioning``, ``bidirectional_block``, the
-    fp32 extractors), which keep their single library call in its deterministic form. The backward kernels use no atomics."""
+    fp32 extractors) and, in fp32, the conditioning recipes (``residual_conditioning``, ``residual_conditioning_bidir``), which
+    keep their single library call in its deterministic form. The backward kernels use no atomics."""
     prev = is_deterministic()
     _state.det = bool(enabled)
     try:

@@ -218,8 +218,20 @@ int dcb_occlusion_mask(const DcbTensor* flow_a, const DcbTensor* flow_b, const D
  *
  *   image1, gt [N,C,H,W] (1 <= C <= 3; one dtype, F32 or BF16, for every tensor); flow1, flow2 [N,2,H,W]
  *   fused, residual [N,C,H,W] contiguous; occ_fwd / occ_bwd [N,1,H,W] optional outputs
+ *   flags: DCB_FLAG_WS_CLEAN as dcb_splat_fwd; other bits are ignored, except DCB_FLAG_DETERMINISTIC (see below), which
+ *   earlier versions ignored too
+ *
+ * DCB_FLAG_DETERMINISTIC (this entry and dcb_residual_bidir; F32 only, else DCB_E_DTYPE): bit-reproducible, and bit-identical
+ * to the composition of deterministic single ops (dcb_splat_fwd's deterministic mode for the warps and for the flows behind
+ * the masks, the occlusion test, the fusion, the subtraction). The image splat and one mask splat share the footprints of
+ * flow1, the other mask splat (and image2's splat) those of flow2: one key set per flow, 8 x N*H*W keys in all (2^31 or more:
+ * DCB_E_LIMIT), ONE radix sort, one reduce, one epilogue -- 11 launches. The workspace is plain scratch of
+ * dcb_residual_det_workspace_bytes() bytes (DCB_FLAG_WS_CLEAN with it: DCB_E_MODE).
  */
 int64_t dcb_residual_workspace_bytes(int64_t N, int64_t C, int64_t H, int64_t W);
+/* workspace of dcb_residual_fused and dcb_residual_bidir with DCB_FLAG_DETERMINISTIC (one size serves both): keys, sorted
+ * keys, the sort's temporary storage, the cells of both flows' splats */
+int64_t dcb_residual_det_workspace_bytes(int64_t N, int64_t C, int64_t H, int64_t W);
 int dcb_residual_fused(const DcbTensor* image1, const DcbTensor* flow1, const DcbTensor* flow2,
                        const DcbTensor* gt, const DcbTensor* fused, const DcbTensor* residual,
                        const DcbTensor* occ_fwd, const DcbTensor* occ_bwd,
@@ -244,7 +256,7 @@ int dcb_residual_fused(const DcbTensor* image1, const DcbTensor* flow1, const Dc
  *   inputs may have any strides, a stride-0 batch included (one I-frame serving several inter frames)
  *   fused, residual [N,C,H,W] contiguous; occ_fwd / occ_bwd [N,1,H,W] optional outputs
  *   workspace: dcb_residual_workspace_bytes(N, C, H, W) -- the requirement is the same as dcb_residual_fused's;
- *   DCB_FLAG_WS_CLEAN protocol as dcb_residual_fused
+ *   DCB_FLAG_WS_CLEAN protocol as dcb_residual_fused; DCB_FLAG_DETERMINISTIC as dcb_residual_fused (same workspace query)
  */
 int dcb_residual_bidir(const DcbTensor* image1, const DcbTensor* image2, const DcbTensor* flow1, const DcbTensor* flow2,
                        const DcbTensor* gt, const DcbTensor* fused, const DcbTensor* residual,
